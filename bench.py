@@ -2,15 +2,21 @@
 """bench.py -- input Msamples/s through the zoom-FFT PSD path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--workload cfg2|cfg1|cfg3|cfg4] [--frames F]
+                    [--workload cfg2|cfg1|cfg3|cfg4] [--frames F] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of F synthetic frames of
 the workload (default: BASELINE.json configs[1], the RTL-SDR uint8 replay).
-``value`` is measured with the batch already resident in HBM; ``e2e`` goes
+``value`` is measured over exactly K steps with the batch already resident in
+HBM and no profiling events between the kernels; ``e2e`` goes
 through the public host API (pinned host buffers, H2D + D2H inside the timed
 region).  For N > 1 launch with torch.distributed.run: one rank per GPU, every
 rank processes its own F frames (weak scaling, no data-path collective) and
 the finished rows are gathered to rank 0 over NCCL inside the timed region.
+
+``--dump-outputs DIR`` writes the rows the last timed step returned (gathered
+on rank 0 for N > 1) to DIR/rows.npy as float32.  The frames are generated
+from fixed seeds, so two builds run with the same arguments can be compared
+row for row.
 
 ``--impl reference`` times the reference's own CPU arithmetic (the oracle
 port: the same scipy.signal.decimate / welch calls, oracle/zoompsd_oracle.py)
@@ -249,6 +255,19 @@ def ncu_traffic(workload, kernel, frames_per_launch):
         return None
 
 
+DUMP_MAX_BYTES = 60 * 10**6          # rows.npy stays under 64 MB, header included
+
+
+def dump_rows(path, rows):
+    """``path``/rows.npy: float32 rows, or -- past DUMP_MAX_BYTES -- a fixed, seeded sample of
+    whole rows kept in their order (the same rows for the same arguments)."""
+    if rows.nbytes > DUMP_MAX_BYTES:
+        keep = DUMP_MAX_BYTES // rows[0].nbytes
+        rows = rows[np.sort(np.random.default_rng(0).choice(len(rows), keep, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "rows.npy"), np.ascontiguousarray(rows, dtype=np.float32))
+
+
 # --------------------------------------------------------------------------
 # GPU arm
 # --------------------------------------------------------------------------
@@ -441,14 +460,12 @@ def run_b200(args, w):
     sampler = ClockSampler(uuid, local_rank)
     sampler.start()
 
-    # ---------------- device-resident throughput ----------------
+    # ---------------- device-resident throughput: the K timed steps ----------------
     for _ in range(args.warmup):
         step_device()
     join_device()
     barrier()
     k0 = eng.counters()["kernels"]
-    eng.profile()
-    eng.set_profiling(True)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.time()
     ev0.record(stream)
@@ -461,10 +478,22 @@ def run_b200(args, w):
     barrier()
     t1 = time.time()
     ms = ev0.elapsed_time(ev1)
-    eng.set_profiling(False)
-    prof = eng.profile()
     launches = eng.counters()["kernels"] - k0
     clocks = sampler.summary(t0 - 0.06, t1 + 0.06)     # K steps take milliseconds: the samples around them
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = (d_rows2[(step_no[0] - 1) & 1] if world == 1 else torch.cat(gather_list)).cpu().numpy()
+
+    # ---------------- per-kernel times: K more steps with events around every kernel ----------------
+    # (a pass of its own: the events are recorded between the kernels, so they stay out of the timed steps)
+    eng.profile()
+    eng.set_profiling(True)
+    for _ in range(args.steps):
+        step_device()
+    join_device()
+    barrier()
+    eng.set_profiling(False)
+    prof = eng.profile()
 
     # ---------------- end to end (host buffers) ----------------
     for _ in range(max(1, min(args.warmup, 3))):
@@ -602,15 +631,9 @@ def run_b200(args, w):
     value = samples_step * args.steps / (ms * 1e-3) / 1e6
     e2e_value = samples_step * e2e_steps / (ms_e2e * 1e-3) / 1e6
     copy_value = samples_step * e2e_steps / (ms_copy * 1e-3) / 1e6
-    burst_value, value_source, steps_counted, ms_counted = value, "timed K steps", args.steps, ms
     if sustained:
         sus_value = samples_step * sustained["steps"] / (ms_sus * 1e-3) / 1e6
-        sustained.update(value=sus_value, unit=UNIT, seconds=ms_sus * 1e-3,
-                         ratio_to_burst=sus_value / burst_value)
-        if abs(sus_value / burst_value - 1.0) > 0.03:
-            # a burst of K steps at boost clocks is not what a long job sees: report the long run
-            value, value_source = sus_value, "sustained leg (differs from the K-step burst by > 3 %)"
-            steps_counted, ms_counted = sustained["steps"], ms_sus
+        sustained.update(value=sus_value, unit=UNIT, seconds=ms_sus * 1e-3, ratio_to_value=sus_value / value)
 
     if rank == 0:
         peak, peak_src = measured_hbm_peak()
@@ -637,7 +660,7 @@ def run_b200(args, w):
             algo_launch = F * w.frame_len * w.bytes_per_sample / max(1, top_n // args.steps)
         avg_launch_ms = top_ms / max(1, top_n)
         achieved = algo_launch / (avg_launch_ms * 1e-3) / 1e9
-        step_ms = ms_counted / steps_counted
+        step_ms = ms / args.steps
         roofline = {
             "bound": "hbm", "kernel": names.get(top, top), "achieved": achieved, "peak": peak, "unit": "GB/s",
             "frac": achieved / peak,
@@ -676,14 +699,17 @@ def run_b200(args, w):
                                                     "overlapped, after the timed legs of this run")
         # the binding roofline: fp32 FMA pipe (SURVEY 8d "report both")
         flops_sample, flop_parts = algorithmic_flops(w, eng, nch)
-        sm_mhz = ((sustained["clocks"]["sm_mhz"] if sustained else None) or clocks["sm_mhz"] or
-                  clocks.get("sm_max_mhz") or 1965.0)
+        if clocks["sm_mhz"]:
+            sm_mhz, mhz_src = clocks["sm_mhz"], "SM clock sampled around the timed steps"
+        else:
+            sm_mhz = clocks.get("sm_max_mhz") or 1965.0
+            mhz_src = "maximum SM clock: no clock sample fell around the timed steps"
         sms = torch.cuda.get_device_properties(local_rank).multi_processor_count
         peak_tf = sms * 128 * 2 * sm_mhz * 1e6 / 1e12
         ach_tf = flops_sample * (F * w.frame_len) / (step_ms * 1e-3) / 1e12
         roofline_fp32 = {
             "bound": "fp32", "achieved": ach_tf, "peak": peak_tf, "unit": "TFLOP/s", "frac": ach_tf / peak_tf,
-            "peak_source": "%d SMs x 128 lanes x 2 FLOP x %.0f MHz (SM clock sampled during the run)" % (sms, sm_mhz),
+            "peak_source": "%d SMs x 128 lanes x 2 FLOP x %.0f MHz (%s)" % (sms, sm_mhz, mhz_src),
             "algorithmic_flop_per_input_sample": flops_sample,
             "flop_parts_per_input_sample%s" % ("_per_channel" if nch > 1 else ""): {k: round(v, 3) for k, v in flop_parts.items()},
             "scope": "whole step, one GPU",
@@ -707,15 +733,11 @@ def run_b200(args, w):
         h2d_step = in_bytes if bcast_feed else world * in_bytes
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
-            "warmup": args.warmup, "ms_per_step": ms_counted / steps_counted, "higher_is_better": True,
+            "warmup": args.warmup, "ms_per_step": ms / args.steps, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
-            "config": cfg, "rows_per_s": world * nch * F * steps_counted / (ms_counted * 1e-3),
-            "value_source": value_source,
-            "burst": {"value": burst_value, "unit": UNIT, "steps": args.steps, "ms_per_step": ms / args.steps,
-                      "clocks": clocks},
+            "config": cfg, "rows_per_s": world * nch * F * args.steps / (ms * 1e-3),
             "sustained": sustained,
-            # the long leg holds >= 50 samples; the K-step burst lasts milliseconds (see burst.clocks)
-            "clocks": sustained["clocks"] if (sustained and sustained["clocks"].get("samples", 0) > clocks.get("samples", 0)) else clocks,
+            "clocks": clocks,
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d_step,
                     "d2h_bytes_per_step": world * nch * F * W * 4, "steps": e2e_steps,
                     "ms_per_step": ms_e2e / e2e_steps,
@@ -735,6 +757,8 @@ def run_b200(args, w):
             line["multi_gpu_check"] = verify
         if cpu_baseline is not None:
             line["cpu_baseline"] = cpu_baseline
+        if dumped is not None:
+            dump_rows(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     eng.close()
     if world > 1:
@@ -768,14 +792,21 @@ def main():
     ap.add_argument("--set", action="append", dest="sets", metavar="OPTION=VALUE", help="tuning: zfb_set_option")
     ap.add_argument("--lib", default=None, help="tuning: path of an alternative sm_100a build")
     ap.add_argument("--e2e-steps", type=int, default=20)
-    ap.add_argument("--sustain-s", type=float, default=3.0,
-                    help="seconds of back-to-back steps for the sustained leg (0 = skip)")
+    ap.add_argument("--sustain-s", type=float, default=0.0,
+                    help="seconds of back-to-back steps for a sustained leg reported beside the value "
+                         "(default 0: none)")
     ap.add_argument("--cfg4-feed", default="allgather", choices=["allgather", "broadcast", "replicate"],
                     help="cfg4, N > 1: H2D on rank 0 + NCCL broadcast over NVLink, or H2D on every rank")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true",
                     help="N > 1: do not bind each rank to the CPUs of its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rows of the last timed step to DIR/rows.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.warmup < 3:
         args.warmup = 3
     w = synth.WORKLOADS[args.workload]

@@ -13,9 +13,9 @@ objects:
 * ``Data.new_complex/add/get_data_start/get_data_end`` (T:1400-1483)
 * ``Waterfall.init_image/image_update``           (S:1625-1664)
 
-It only works where ``/root/reference`` exists (the build container); it is
-used by ``oracle/make_golden.py`` to record ``tests/golden/*.npz`` and by
-tests that are skipped when the reference tree is absent (the GPU box).
+It only works where the reference's source tree is present
+(``PYPAN_REFERENCE_DIR``); ``oracle/make_golden.py`` uses it to record
+``tests/golden/*.npz``, which the tests compare against.
 No reference source is copied: the files are read where they lie.
 """
 from __future__ import annotations

@@ -363,148 +363,6 @@ def scipy_shaped_calls(engine):
         zsig.decimate(x[:27], 2, engine=engine)          # scipy: padlen
 
 
-def dropin_on_reference_modules(engine):
-    """dropin.install on the UNMODIFIED reference modules (build container
-    only): their own update()/PSD.update() call sequences now produce the
-    golden rows through the engine."""
-    import types
-    from oracle import ref_harness as rh
-    from pypanadapter_b200 import dropin
-    if not rh.available():
-        import pytest
-        pytest.skip("reference tree not present")
-    # ---- spectrum variant: ApplicationDisplay.update(chunk) ----
-    mod = rh.load("spectrum")
-    saved = dropin.install(mod, engine=engine)
-    try:
-        for name in ("cfg1_S1024", "cfg1_S256", "defaults_S"):
-            case = gc.case_by_name(name)
-            x = gc.make_input(case)
-            rh._set_state(mod, case["fs"], case["N"], case["R"], len(x) // case["N"], case["window"])
-            got = {}
-            fake = types.SimpleNamespace(N_WIN=case["n_win"], win=rh._Anything(), spectrum_plot=rh._Anything(),
-                                         waterfall=types.SimpleNamespace(
-                                             image_update=lambda psd: got.__setitem__("psd", psd.copy())))
-            mod.ApplicationDisplay.update(fake, x)
-            floor = parity.floor_db20(case["fs"], case["window"], case["N"], case["R"] > 1)
-            parity.assert_row_parity(got["psd"], parity.golden_rows()[name], floor, "dropin " + name)
-        # raw RTL bytes (rtl_tcp byte callback): converted and flipped on the device == the
-        # reference's update on what RTLSDRstream.read_callback would have emitted (S:459-460)
-        case = gc.case_by_name("cfg1_S256")
-        raw = synth.quantise_u8(0.8 * gc.make_input(case))
-        rh._set_state(mod, case["fs"], case["N"], case["R"], len(raw) // 2 // case["N"], case["window"])
-        got = {}
-        fake = types.SimpleNamespace(N_WIN=case["n_win"], win=rh._Anything(), spectrum_plot=rh._Anything(),
-                                     waterfall=types.SimpleNamespace(
-                                         image_update=lambda psd: got.__setitem__("psd", psd.copy())))
-        mod.ApplicationDisplay.update(fake, raw)
-        want = zo.zoom_psd(raw, case["fs"], case["N"], case["R"], case["window"], crop=case["n_win"], flip=True)
-        parity.assert_row_parity(got["psd"], want, parity.floor_db20(case["fs"], case["window"], case["N"], True),
-                                 "dropin raw u8")
-        case = gc.ZOOMFFT_CASES[0]
-        x = gc.make_input(case)
-        rh._set_state(mod, case["fs"], case["N"], case["R"], len(x) // case["N"], "hamming")
-        z = mod.ApplicationDisplay.zoomfft(types.SimpleNamespace(), x, case["R"])
-        ref = np.load(os.path.join(parity.GOLDEN_DIR, "zoomfft.npz"))[case["name"]]
-        assert np.abs(z - ref).max() < 2e-5 * np.abs(ref).max()
-        # ---- Waterfall: the reference's own class, its methods on the device ring ----
-        g = np.load(os.path.join(parity.GOLDEN_DIR, "waterfall.npz"))
-        engine.configure(2.4e6, 2048, 8, 2048 * 10, "hamming", crop="thread")      # row_width 256
-        for scroll, tag in ((1, "pos"), (-1, "neg")):
-            mod.AppState.scroll = scroll
-            wf = mod.Waterfall.__new__(mod.Waterfall)
-            wf.fftwidth, wf.minlev, wf.maxlev = 0, -220, -120                      # S:1590-1593
-            shown = {}
-            wf.scale = lambda *a, **k: None
-            wf.setImage = lambda img, **k: shown.update(img=np.array(img), kw=k)
-            ref = None
-            for r in gc.waterfall_rows_noise():
-                psd = r.copy()
-                wf.image_update(psd)
-                assert psd[0] == 0 and psd[128] == 0 and psd[255] == 0             # S:1647-1648
-                ref = zo.waterfall_update(ref, r.copy(), scroll)
-            assert shown["kw"]["levels"] == [0, 256] and shown["kw"]["autoLevels"] is False
-            assert np.array_equal(shown["img"], zo.waterfall_indices(ref, -220, -120).T)
-            assert np.abs(wf.img_array - ref).max() < 1e-4
-            assert wf.autolevel() == (-220, -120)
-            gold = g["auto_noise_" + tag]
-            assert (wf.minlevel, wf.maxlevel) == (gold[0], gold[1])                # the reference's own autolevel
-            assert wf.newlevel(-180.0, -100.0) == (-180.0, -100.0)
-            last = gc.waterfall_rows_noise()[-1].copy()
-            wf.image_update(last)
-            ref = zo.waterfall_update(ref, gc.waterfall_rows_noise()[-1].copy(), scroll)
-            assert np.array_equal(shown["img"], zo.waterfall_indices(ref, -180.0, -100.0).T)
-        mod.AppState.scroll = 1
-        # ---- update(chunk) -> image_update(psd): each row enters the ring once, in order ----
-        case = gc.case_by_name("cfg1_S256")
-        wf = mod.Waterfall.__new__(mod.Waterfall)
-        wf.fftwidth, wf.minlev, wf.maxlev = 0, -220, -120
-        wf.scale = lambda *a, **k: None
-        wf.setImage = lambda img, **k: None
-        fake = types.SimpleNamespace(N_WIN=256, win=rh._Anything(), spectrum_plot=rh._Anything(), waterfall=wf)
-        rows = []
-        for i in range(4):
-            x = synth.make_frame(synth.CFG1, i)
-            rh._set_state(mod, case["fs"], case["N"], case["R"], len(x) // case["N"], case["window"])
-            mod.ApplicationDisplay.update(fake, x)
-            rows.append(engine.read_rows(1)[0].astype(np.float64))
-        img = wf.img_array
-        for j, r in enumerate(reversed(rows)):
-            r = r.copy()
-            r[[0, 128, 255]] = 0
-            assert np.array_equal(img[64 - 2 - j], r), j
-    finally:
-        dropin.uninstall(mod, saved)
-    assert mod.ApplicationDisplay.update is saved["ApplicationDisplay.update"]
-    assert "img_array" not in mod.Waterfall.__dict__
-    # ---- thread variant: Data + PSD.update ----
-    mod = rh.load("thread")
-    saved = dropin.install(mod, engine=engine)
-    try:
-        case = gc.case_by_name("cfg1_T")
-        x = gc.make_input(case)
-        rh._set_state(mod, case["fs"], case["N"], case["R"], 1, case["window"])
-        d = mod.Data()
-        assert isinstance(d, buffers_Data())
-        d.NR = types.SimpleNamespace(next=lambda y: 0.0, target=0)
-        d.new_complex()
-        d.delay_time = 0.
-        for i in range(0, len(x), d.chunk_size):
-            d.add(x[i:i + d.chunk_size])
-            d.delay_time = 0.
-        psd = types.SimpleNamespace(dataclass=d, lock=rh._Mutex(), psd=None)
-        mod.PSD.update(psd)
-        floor = parity.floor_db20(case["fs"], case["window"], case["N"], True)
-        parity.assert_row_parity(psd.psd, parity.golden_rows()["cfg1_T"], floor, "dropin PSD.update")
-        d.target = 100000
-        assert d.target == 100000
-        d.target = 10             # below fft_size: ignored (T:1476)
-        assert d.target == 100000
-        # GUI timer side (T:2140-2148): only the rows it displays enter the ring
-        before = engine.rows_written
-        for i in range(0, len(x), d.chunk_size):
-            d.add(x[i:i + d.chunk_size])
-            d.delay_time = 0.
-        mod.PSD.update(psd)                                   # a second row nobody displays
-        assert engine.rows_written == before
-        wf = mod.Waterfall.__new__(mod.Waterfall)
-        wf.fftwidth, wf.minlev, wf.maxlev = 0, -220, -120
-        wf.scale = lambda *a, **k: None
-        shown = {}
-        wf.setImage = lambda img, **k: shown.update(img=np.array(img))
-        row = np.array(psd.psd, copy=True)
-        wf.image_update(row)
-        assert engine.rows_written == 1 and shown["img"].shape == (256, 64)
-        ref = zo.waterfall_update(None, np.array(psd.psd, dtype=np.float32).astype(np.float64), 1)
-        assert np.array_equal(shown["img"], zo.waterfall_indices(ref, -220, -120).T)
-    finally:
-        dropin.uninstall(mod, saved)
-    engine.configure(2.4e6, 2048, 8, 2048 * 10, "hamming", crop="thread")
-    n0 = engine.rows_written
-    engine.process(synth.make_frame(synth.CFG1, 0, 2048 * 10))
-    assert engine.rows_written == n0 + 1                      # uninstall restored ring_append
-
-
 def dropin_on_standin_modules(engine):
     """dropin.install on stand-in modules with the reference's class / method
     names and EMPTY hot-path bodies (tests/standin_pan.py) -- runs wherever the
@@ -534,18 +392,59 @@ def dropin_on_standin_modules(engine):
         z = mod.ApplicationDisplay(256).zoomfft(x, case["R"])
         ref = np.load(os.path.join(parity.GOLDEN_DIR, "zoomfft.npz"))[case["name"]]
         assert np.abs(z - ref).max() < 2e-5 * np.abs(ref).max()
-        # update(chunk) -> Waterfall.image_update: the image the reference would hold
+        # raw RTL bytes (rtl_tcp byte callback): converted and flipped on the device == the
+        # reference's update on what RTLSDRstream.read_callback would have emitted (S:459-460)
+        case = gc.case_by_name("cfg1_S256")
+        raw = synth.quantise_u8(0.8 * gc.make_input(case))
+        sp.set_state(mod, case["fs"], case["N"], case["R"], len(raw) // 2 // case["N"], case["window"])
+        app = mod.ApplicationDisplay(case["n_win"])
+        got = {}
+        app.waterfall = types.SimpleNamespace(image_update=lambda psd: got.__setitem__("psd", psd.copy()))
+        app.update(raw)
+        want = zo.zoom_psd(raw, case["fs"], case["N"], case["R"], case["window"], crop=case["n_win"], flip=True)
+        parity.assert_row_parity(got["psd"], want, parity.floor_db20(case["fs"], case["window"], case["N"], True),
+                                 "stand-in dropin raw u8")
+        # ---- Waterfall in both scroll directions: its methods on the device ring ----
+        g = np.load(os.path.join(parity.GOLDEN_DIR, "waterfall.npz"))
+        engine.configure(2.4e6, 2048, 8, 2048 * 10, "hamming", crop="thread")      # row_width 256
+        for scroll, tag in ((1, "pos"), (-1, "neg")):
+            mod.AppState.scroll = scroll
+            wf = mod.Waterfall()
+            ref = None
+            for r in gc.waterfall_rows_noise():
+                psd = r.copy()
+                wf.image_update(psd)
+                assert psd[0] == 0 and psd[128] == 0 and psd[255] == 0             # S:1647-1648
+                ref = zo.waterfall_update(ref, r.copy(), scroll)
+            assert wf.shown["kw"]["levels"] == [0, 256] and wf.shown["kw"]["autoLevels"] is False
+            assert np.array_equal(wf.shown["img"], zo.waterfall_indices(ref, -220, -120).T)
+            assert np.abs(wf.img_array - ref).max() < 1e-4
+            assert wf.autolevel() == (-220, -120)
+            gold = g["auto_noise_" + tag]
+            assert (wf.minlevel, wf.maxlevel) == (gold[0], gold[1])                # the reference's own autolevel
+            assert wf.newlevel(-180.0, -100.0) == (-180.0, -100.0)
+            wf.image_update(gc.waterfall_rows_noise()[-1].copy())
+            ref = zo.waterfall_update(ref, gc.waterfall_rows_noise()[-1].copy(), scroll)
+            assert np.array_equal(wf.shown["img"], zo.waterfall_indices(ref, -180.0, -100.0).T)
+        mod.AppState.scroll = 1
+        # update(chunk) -> Waterfall.image_update: the image the reference would hold, each row
+        # entering the ring once, in order
         case = gc.case_by_name("cfg1_S256")
         app = mod.ApplicationDisplay(256)
         ref_img = None
-        for i in range(3):
+        rows = []
+        for i in range(4):
             x = synth.make_frame(synth.CFG1, i)
             sp.set_state(mod, case["fs"], case["N"], case["R"], len(x) // case["N"], case["window"])
             app.update(x)
-            row = engine.read_rows(1)[0].astype(np.float64)
-            ref_img = zo.waterfall_update(ref_img, row.copy(), 1)
+            rows.append(engine.read_rows(1)[0].astype(np.float64))
+            ref_img = zo.waterfall_update(ref_img, rows[-1].copy(), 1)
         assert np.array_equal(app.waterfall.img_array, ref_img)
         assert np.array_equal(app.waterfall.shown["img"], zo.waterfall_indices(ref_img, -220, -120).T)
+        for j, r in enumerate(reversed(rows)):
+            r = r.copy()
+            r[[0, 128, 255]] = 0
+            assert np.array_equal(app.waterfall.img_array[64 - 2 - j], r), j
         # ---- the taper dialog's ShowCurve (S:1354-1379) ----
         import scipy.signal
         for tname, p0, p1, spec in (("hamming", 0, 0, "hamming"), ("kaiser", 9.5, 0, ("kaiser", 9.5)),
@@ -565,6 +464,9 @@ def dropin_on_standin_modules(engine):
             assert len(dlg.plot0.items) == 1 and len(dlg.plot1.items) == 1
     finally:
         dropin.uninstall(mod, saved)
+    assert mod.ApplicationDisplay.update is saved["ApplicationDisplay.update"]
+    assert mod.Waterfall.__dict__["image_update"] is saved["Waterfall.image_update"]
+    assert "img_array" not in mod.Waterfall.__dict__                    # added by install: removed again
     # ---- thread variant: Data, PSD.update, and the GUI timer (T:2140-2157) ----
     mod = sp.make("thread")
     saved = dropin.install(mod, engine=engine)
@@ -593,8 +495,13 @@ def dropin_on_standin_modules(engine):
         app.update()                                          # new width: the image starts over (S:1641-1643)
         W = 2 * int(.5 * case["N"] / case["R"])
         assert app.waterfall.fftwidth == W and app.waterfall.shown["img"].shape == (W, W // 4)
+        assert engine.rows_written == 1
         img = zo.waterfall_update(None, np.array(psd.psd, dtype=np.float32).astype(np.float64), 1)
         assert np.array_equal(app.waterfall.img_array, img)
+        # a row PSD.update computes but the timer never shows stays out of the ring (T:2140-2148)
+        feed()
+        psd.update()
+        assert engine.rows_written == 1
         # a zoom click (S:2079-2086 makes fft_ratio a float): PSD.update has re-planned for the new
         # width while the timer still shows the row of the old one -- then the new row arrives
         st.fft_ratio = case["R"] * 2.0
@@ -622,8 +529,18 @@ def dropin_on_standin_modules(engine):
         psd2 = mod.PSD(d2)
         psd2.update()
         parity.assert_row_parity(psd2.psd, parity.golden_rows()["cfg1_T"], floor, "stand-in PSD.update (2nd Data)")
+        d2.target = 100000
+        assert d2.target == 100000
+        d2.target = 10                                        # below fft_size: ignored (T:1476)
+        assert d2.target == 100000
     finally:
         dropin.uninstall(mod, saved)
+    assert mod.Data is saved["Data"] and mod.PSD.update is saved["PSD.update"]
+    engine.configure(2.4e6, 2048, 16, 2048 * 10, "hamming", crop="thread")
+    assert engine.row_width == engine.ring_width == W // 2    # the ring keeps rows of its own width only
+    n0 = engine.rows_written
+    engine.process(synth.make_frame(synth.CFG1, 0, 2048 * 10))
+    assert engine.rows_written == n0 + 1                      # uninstall restored ring_append
 
 
 def fast_mode_state_survives_frame_len(engine):

@@ -1,8 +1,7 @@
 """TEST INFRASTRUCTURE: minimal stand-ins for the two reference programs.
 
-The GPU box has no /root/reference, so `dropin.install` cannot be exercised
-there on the real modules (tests/buffers_suite.dropin_on_reference_modules does
-that in the build container).  `make("spectrum")` / `make("thread")` build
+The reference programs are not part of this repository, so `dropin.install` is
+exercised on stand-ins.  `make("spectrum")` / `make("thread")` build
 modules with the SAME class, method and attribute names the drop-in touches --
 `AppState`, `ApplicationDisplay.zoomfft/update`, `PSD`, `Data`, `Waterfall`
 (pypanadapter_spectrum.py:1577-1686, 2088-2130; pypanadapter_thread.py:1400-1549,

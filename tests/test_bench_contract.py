@@ -8,6 +8,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -52,6 +54,54 @@ def test_gpu_arm_has_no_cpu_fallback():
         pytest.skip("a CUDA device is present")
     r = _run(["--steps", "1", "--warmup", "3", "--no-cpu-baseline"])
     assert r.returncode != 0 and "no CPU fallback" in (r.stdout + r.stderr)
+
+
+def test_dump_outputs_is_refused_by_the_reference_arm(tmp_path):
+    r = _run(["--impl", "reference", "--steps", "1", "--dump-outputs", str(tmp_path / "out")])
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+    assert not (tmp_path / "out").exists()
+
+
+@pytest.mark.gpu
+def test_gpu_arm_times_k_steps_and_dumps_their_rows(tmp_path):
+    """--steps K times K steps (the kernel launches of the timed region double with K), and
+    --dump-outputs writes the rows of the last timed step: float32, one row per frame, the same
+    rows from run to run with the same arguments, and the rows the engine returns for the
+    (3 + K)-th batch of the same frames -- cfg2 carries its EMA from row to row, and over so few
+    rows the rows of the step before still differ."""
+    import numpy as np
+    import torch
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    from pypanadapter_b200 import synth
+    from pypanadapter_b200.engine import ZoomPSD
+    w = synth.CFG2
+    d_in = torch.from_numpy(synth.make_frames(w, 4)).cuda()
+    want = {}
+    with ZoomPSD(0) as eng:
+        eng.configure(w.fs, w.fft_size, w.fft_ratio, w.frame_len, w.window, dtype=w.dtype, flip=w.flip,
+                      f_demod=w.f_demod, crop=w.crop, ema_alpha=w.ema_alpha, mode="fast")
+        d_rows = torch.empty((4, eng.row_width), dtype=torch.float32, device="cuda")
+        torch.cuda.synchronize()
+        for batch in range(1, 3 + 4 + 1):
+            eng.process_device(d_in.data_ptr(), 4, d_rows.data_ptr())
+            eng.synchronize()
+            want[batch] = d_rows.cpu().numpy()
+    assert not np.array_equal(want[4], want[5])
+    lines, rows = [], []
+    for i, steps in enumerate((2, 2, 4)):
+        out = tmp_path / str(i)
+        r = _run(["--frames", "4", "--steps", str(steps), "--warmup", "3", "--no-cpu-baseline",
+                  "--dump-outputs", str(out)])
+        assert r.returncode == 0, r.stderr[-3000:]
+        lines.append(json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1]))
+        rows.append(np.load(out / "rows.npy"))
+    assert [ln["steps"] for ln in lines] == [2, 2, 4]
+    assert lines[2]["gpu_launches"] == 2 * lines[0]["gpu_launches"] > 0
+    assert rows[0].dtype == np.float32 and rows[0].shape == (4, lines[0]["config"]["row_width"])
+    assert np.isfinite(rows[0]).all()
+    assert np.array_equal(rows[0], rows[1])
+    assert np.array_equal(rows[0], want[3 + 2]) and np.array_equal(rows[2], want[3 + 4])
 
 
 def test_committed_gpu_arm_line_carries_the_contract():

@@ -139,10 +139,6 @@ def test_scipy_shaped_calls(emu_engine):
     bs.scipy_shaped_calls(emu_engine)
 
 
-def test_dropin_on_reference_modules(emu_engine):
-    bs.dropin_on_reference_modules(emu_engine)
-
-
 # ---- ZFB_MODE_FAST ------------------------------------------------------------------
 @pytest.mark.parametrize("name", es.FAST_CASES)
 def test_fast_golden_case(emu_engine, name):

@@ -289,19 +289,6 @@ def test_scipy_shaped_calls(gpu_engine):
     bs.scipy_shaped_calls(gpu_engine)
 
 
-def _reference_tree_present():
-    from oracle import ref_harness as rh
-    return rh.available()
-
-
-if _reference_tree_present():
-    # only collected where /root/reference exists (the build container, which has no GPU: the
-    # emulator runs the same routine in test_emu_engine.py); on the GPU box the same install is
-    # exercised by test_dropin_on_standin_modules below
-    def test_dropin_on_reference_modules(gpu_engine):
-        bs.dropin_on_reference_modules(gpu_engine)
-
-
 # ---- ZFB_MODE_FAST ------------------------------------------------------------------
 @pytest.mark.parametrize("name", es.FAST_CASES)
 def test_fast_golden_case(gpu_engine, name):
