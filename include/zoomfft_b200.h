@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ZFB_ABI_VERSION 2
+#define ZFB_ABI_VERSION 3
 
 /* status codes */
 #define ZFB_OK            0
@@ -249,6 +249,57 @@ int  zfb_read_rows(zfb_engine *e, int age, int nrows, float *h_out);
  * that was computed elsewhere, S:1638-1652). */
 int  zfb_ring_push_rows(zfb_engine *e, const float *h_rows, int nrows);
 
+/* ---- max-hold, min-hold and average traces, peak markers (DESIGN 3.8) -----
+ * The reference plots each row as it arrives (spectrum_plot.setData(psd),
+ * S:2130) and keeps nothing across rows.  A trace set extends that plot with the
+ * standard traces of a spectrum analyser, kept on the device over EVERY row the
+ * engine computes -- also rows that never reach the ring (ring_append = 0, the
+ * threaded GUI's skipped rows, T:2140-2148) -- in the rows' own units (dB20, or
+ * linear power with ZFB_FLAG_LINEAR):
+ *   ZFB_TRACE_LAST  the newest row
+ *   ZFB_TRACE_MAX   running maximum per column (NaN ignored, fmaxf)
+ *   ZFB_TRACE_MIN   running minimum per column (fminf)
+ *   ZFB_TRACE_AVG   mean linear power (the row, or 10^(v/20) of a dB20 row), summed
+ *                   in fp64 in frame order; read out as sum/count, in dB20 as
+ *                   20 log10(sum/count), rounded to float
+ * Rows of zfb_process_device, zfb_process_host and zfb_samples_process feed it on
+ * every path (slabs, pipelined batches, fp64 rows), with EMA applied as the
+ * caller gets them; rows of zfb_ring_push_rows do not.  LAST, MAX, MIN and the
+ * fp64 sum are bit-identical however the same frames are split into calls,
+ * groups, slabs or batches.  The set is off by default: then nothing is
+ * allocated or launched and rows, ring and counters are as without it.  It
+ * starts empty on zfb_traces_enable, zfb_traces_reset and a zfb_configure that
+ * changes fs, fft_size, fft_ratio, row_width, f_demod or flags; it keeps
+ * counting over a change of frame_len (PSD.update hands over chunks of varying
+ * length, T:1516-1520), window, ema_alpha, dtype, flip or mode.  While it is on,
+ * zfb_process_channels_* return ZFB_EINVAL (one trace set per engine). */
+#define ZFB_TRACE_LAST 0
+#define ZFB_TRACE_MAX  1
+#define ZFB_TRACE_MIN  2
+#define ZFB_TRACE_AVG  3
+int  zfb_traces_enable(zfb_engine *e, int on);
+int  zfb_traces_reset(zfb_engine *e);
+/* rows in the traces since they last started empty (0 while off) */
+int64_t zfb_traces_count(const zfb_engine *e);
+/* row_width floats of trace `kind` to h_out; joins pending work, blocks.
+ * ZFB_ESTATE when the traces are off or hold no row. */
+int  zfb_trace_read(zfb_engine *e, int kind, float *h_out);
+/* Peak markers of trace `kind`: scipy.signal.find_peaks(trace, height=height,
+ * distance=distance) -- local maxima, a plateau's midpoint, never the first or
+ * last column, NaN never a peak; height filter first, then scipy's greedy
+ * distance selection -- and of those the k highest in descending order (ties to
+ * the lower column).  Per marker: its column, the trace value there and the
+ * parabolic offset 0.5(a-c)/(a-2b+c) in fp64 from the three values around it
+ * (0 on a plateau or next to a non-finite value).  1 <= k <= 64, distance >= 1,
+ * height NaN = none.  *npeaks = markers written.  Only the markers are copied
+ * back.  Errors as zfb_trace_read. */
+int  zfb_trace_peaks(zfb_engine *e, int kind, int k, int distance, double height, int32_t *cols, float *values,
+                     double *offsets, int *npeaks);
+/* the same on any device vector of n float32 (1 <= n <= 262144), e.g. a row of
+ * zfb_process_device; ordered on the engine's stream, blocks. */
+int  zfb_find_peaks_device(zfb_engine *e, const float *d_x, int n, int k, int distance, double height,
+                           int32_t *cols, float *values, double *offsets, int *npeaks);
+
 /* ---- waterfall image and autolevel on the device (SURVEY 8f.1) -----------
  * Replaces Waterfall.init_image / image_update's img_array bookkeeping
  * (S:1625-1662: -500 fill, grid columns, np.roll of the whole image per row,
@@ -334,7 +385,7 @@ int  zfb_get_counters(const zfb_engine *e, uint64_t out5[5]);
 /* kernel classes: 0..15 = decimate-by-2 stage s (replaces scipy.signal.
  * decimate call s of the loop at S:2097-2098), 16 = Welch kernel / four-step
  * column pass, 17 = four-step row pass (both: scipy.signal.welch, S:2111),
- * 18 = row finalisation (S:2114-2119 + EMA), 19 = waterfall image
+ * 18 = row finalisation (S:2114-2119 + EMA, trace update), 19 = waterfall image
  * (S:1625-1664), 20 = autolevel selection sweep (S:1676). */
 #define ZFB_PROF_CLASSES 21
 /* on != 0: bracket every kernel launch with CUDA events on the engine's

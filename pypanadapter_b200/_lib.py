@@ -32,11 +32,15 @@ ZFB_FLAG_NO_LO = 1
 ZFB_FLAG_LINEAR = 2
 ZFB_FLAG_ONESIDED = 4
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 PROF_CLASSES = 21
 ZFB_IMAGE_F32 = 0
 ZFB_IMAGE_U8 = 1
 ZFB_IMAGE_RGBA = 2
+ZFB_TRACE_LAST = 0
+ZFB_TRACE_MAX = 1
+ZFB_TRACE_MIN = 2
+ZFB_TRACE_AVG = 3
 
 
 class ZfbConfig(C.Structure):
@@ -100,6 +104,14 @@ SYMBOLS = {
     "zfb_ring_rows_written": (C.c_int64, [_P]),
     "zfb_read_rows": (C.c_int, [_P, C.c_int, C.c_int, _P]),
     "zfb_ring_push_rows": (C.c_int, [_P, _P, C.c_int]),
+    "zfb_traces_enable": (C.c_int, [_P, C.c_int]),
+    "zfb_traces_reset": (C.c_int, [_P]),
+    "zfb_traces_count": (C.c_int64, [_P]),
+    "zfb_trace_read": (C.c_int, [_P, C.c_int, C.POINTER(C.c_float)]),
+    "zfb_trace_peaks": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_int32),
+                                  C.POINTER(C.c_float), C.POINTER(C.c_double), C.POINTER(C.c_int)]),
+    "zfb_find_peaks_device": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_int32),
+                                        C.POINTER(C.c_float), C.POINTER(C.c_double), C.POINTER(C.c_int)]),
     "zfb_ring_image": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_double, C.c_double, _P, _P, C.c_int]),
     "zfb_ring_quantiles": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, C.POINTER(C.c_double), C.c_int,
                                      C.POINTER(C.c_double), C.POINTER(C.c_int64)]),

@@ -29,6 +29,7 @@
 #include "zfb_image.cuh"
 #include "zfb_taper.cuh"
 #include "zfb_precise.cuh"
+#include "zfb_trace.cuh"
 
 using namespace zfb;
 
@@ -160,6 +161,13 @@ struct zfb_engine {
     bool thr_valid = false;            // img_thr holds the level thresholds of thr_levels
     double thr_levels[2] = {0.0, 0.0};
     bool ema_have = false;             // the EMA state holds a row (host side; launch order = stream order)
+    // trace set (zfb_traces_enable; zfb_trace.cuh): nothing is allocated or launched while it is off
+    bool traces_on = false;
+    int64_t trace_count = 0;           // rows in the traces (host side; launch order = stream order)
+    double trace_key[6] = {0, 0, 0, 0, 0, 0};   // fs, N, R, row_width, f_demod, flags of the last configure
+    DevBuf trace;                      // [W] fp64 sums, then LAST, MAX, MIN, AVG read-out [4][W] float
+    DevBuf trace_rows;                 // [group][W] rows of a launch group the caller did not ask for
+    DevBuf peaks;                      // PeakOut, then one flag byte per element
 
     // ZFB_MODE_FAST
     struct FastPlan {
@@ -1296,6 +1304,34 @@ cudaError_t run_decimation_fast(zfb_engine *e, const void *d_in, int gf, int *ou
     return cudaSuccess;
 }
 
+// traces on: the rows of a launch group go to the caller's buffer or, without one, to this scratch
+float *trace_rows_or(zfb_engine *e, float *d_rows) {
+    return (d_rows || !e->traces_on || e->cur_nch > 0) ? d_rows : (float *)e->trace_rows.p;
+}
+
+// fold `nf` finished rows into the trace set, on the stream that finished them (after them)
+int trace_update(zfb_engine *e, const float *rows, int nf, cudaStream_t st) {
+    if (!e->traces_on || e->cur_nch > 0 || nf < 1) return ZFB_OK;
+    const int W = e->W;
+    TraceParams tp{};
+    tp.rows = rows;
+    tp.nframes = nf;
+    tp.W = W;
+    tp.linear = (e->cfg.flags & ZFB_FLAG_LINEAR) ? 1 : 0;
+    tp.have = e->trace_count > 0 ? 1 : 0;
+    tp.sum = (double *)e->trace.p;
+    tp.last = (float *)(tp.sum + W);
+    tp.mx = tp.last + W;
+    tp.mn = tp.mx + W;
+    const int pr = prof_begin(e, 18, st);
+    ZFB_LAUNCH(trace_update_kernel, dim3((unsigned)((W + TR_COLS - 1) / TR_COLS)), dim3(TR_NT), 0, st, tp);
+    prof_end(e, pr, st);
+    e->counters[2] += 1;
+    e->trace_count += nf;
+    CK(e, cudaGetLastError());
+    return ZFB_OK;
+}
+
 // fp64 path (zfb_precise.cuh): rows of few Welch segments, `gf` frames resident on the device
 int run_group_precise(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
     const zfb_config &c = e->cfg;
@@ -1380,7 +1416,7 @@ int run_group_precise(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
         rp.linear = (c.flags & ZFB_FLAG_LINEAR) ? 1 : 0;
         rp.ema_state = (float *)e->ema.p;
         rp.ema_have = e->ema_have ? 1 : 0;
-        rp.rows = d_rows ? d_rows + (size_t)g0 * e->W : nullptr;
+        rp.rows = trace_rows_or(e, d_rows ? d_rows + (size_t)g0 * e->W : nullptr);
         const bool to_ring = e->ring_append && e->ring.p && e->ring_W == e->W && e->cur_nch == 0;
         rp.ring = to_ring ? (float *)e->ring.p : nullptr;
         rp.ring_pos = (long long)(e->ring_written % e->ring_rows);
@@ -1393,6 +1429,8 @@ int run_group_precise(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
         e->counters[2] += 2;
         if (rp.alpha >= 0.0) e->ema_have = true;
         if (to_ring) e->ring_written += nf;
+        const int rc = trace_update(e, rp.rows, nf, st);
+        if (rc) return rc;
     }
     CK(e, cudaGetLastError());
     e->last_group_frames = gf;
@@ -1705,7 +1743,7 @@ int finish_rows(zfb_engine *e, zfb_engine *from, int gf, int nsplit, float *d_ro
     f.linear = (c.flags & ZFB_FLAG_LINEAR) ? 1 : 0;
     f.ema_state = (float *)e->ema.p;
     f.ema_have = e->ema_have ? 1 : 0;
-    f.rows = d_rows;
+    f.rows = trace_rows_or(e, d_rows);
     // rows enter the ring when it has their width; channel-batched launches (rows of different
     // receivers) never do
     const bool to_ring = e->ring_append && e->ring.p && e->ring_W == e->W && e->cur_nch == 0;
@@ -1725,6 +1763,8 @@ int finish_rows(zfb_engine *e, zfb_engine *from, int gf, int nsplit, float *d_ro
     e->counters[2] += 1;
     prof_end(e, prf, st);
     CK(e, cudaGetLastError());
+    const int rc = trace_update(e, f.rows, gf, st);
+    if (rc) return rc;
     if (to_ring) e->ring_written += gf;
     e->last_group_frames = gf;
     e->last_front = from;
@@ -2044,7 +2084,8 @@ void zfb_destroy(zfb_engine *e) {
     if (e->aux_stream) cudaStreamSynchronize(e->aux_stream);
     if (e->aux_stream_hi) cudaStreamSynchronize(e->aux_stream_hi);
     DevBuf *bufs[] = {&e->window, &e->winfft, &e->winfft16, &e->wf_sparse, &e->twiddle, &e->twiddle_sub, &e->pow16, &e->mid[0], &e->mid[1], &e->pow, &e->rows_tmp, &e->ema,
-                      &e->img_out, &e->img_lut, &e->img_thr, &e->sel_hist, &e->ring, &e->stage_in[0], &e->stage_in[1], &e->big};
+                      &e->img_out, &e->img_lut, &e->img_thr, &e->sel_hist, &e->ring, &e->stage_in[0], &e->stage_in[1], &e->big,
+                      &e->trace, &e->trace_rows, &e->peaks};
     for (DevBuf *b : bufs) release(*b);
     for (int i = 0; i < 2; ++i) {
         if (e->h_stage[i]) cudaFreeHost(e->h_stage[i]);
@@ -2098,6 +2139,14 @@ int zfb_plan_geometry(int frame_len, int fft_size, int fft_ratio, int out5[5]) {
 
 static int configure_impl(zfb_engine *e, const zfb_config *cfg);
 static void setup_lanes(zfb_engine *e);
+
+// trace state and the scratch for rows of launch groups without a caller's row buffer
+static int trace_buffers(zfb_engine *e) {
+    const size_t W = (size_t)e->W;
+    int rc = ensure(e, e->trace, W * (sizeof(double) + 4 * sizeof(float)));
+    if (rc) return rc;
+    return ensure(e, e->trace_rows, (size_t)e->group * W * sizeof(float));     // fp64 passes: px_group <= group
+}
 
 int zfb_configure(zfb_engine *e, const zfb_config *cfg) {
     if (!e) return ZFB_EINVAL;
@@ -2364,6 +2413,16 @@ static int configure_impl(zfb_engine *e, const zfb_config *cfg) {
         }
         CK(e, cudaMemcpyAsync(e->px_win.p, cfg->window, (size_t)g.nperseg * sizeof(double), cudaMemcpyHostToDevice, e->stream));
         CK(e, cudaStreamSynchronize(e->stream));       // the caller's window table may go away
+    }
+    // the traces keep counting over a change of frame_len, window, EMA, wire format, flip or mode;
+    // anything that changes what a column means or its units starts them afresh
+    const double key[6] = {cfg->fs, (double)N, (double)cfg->fft_ratio, (double)cfg->row_width, cfg->f_demod,
+                           (double)cfg->flags};
+    if (memcmp(key, e->trace_key, sizeof key) != 0) e->trace_count = 0;
+    memcpy(e->trace_key, key, sizeof key);
+    if (e->traces_on) {
+        rc = trace_buffers(e);
+        if (rc) return rc;
     }
     memcpy(e->geom, geom_now, sizeof geom_now);
     e->geom_valid = true;
@@ -2727,6 +2786,136 @@ int zfb_reset_ema(zfb_engine *e) {
     return ZFB_OK;
 }
 
+// ---- max-hold / min-hold / average traces and peak markers (zfb_trace.cuh) ----------------------
+int zfb_traces_enable(zfb_engine *e, int on) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    e->trace_count = 0;
+    if (!on) {
+        // rows still being folded in read these buffers
+        CK(e, cudaStreamSynchronize(e->stream));
+        e->traces_on = false;
+        for (DevBuf *b : {&e->trace, &e->trace_rows, &e->peaks}) release(*b);
+        return ZFB_OK;
+    }
+    e->traces_on = true;
+    if (e->configured) {
+        const int rc = trace_buffers(e);
+        if (rc) {
+            e->traces_on = false;
+            return rc;
+        }
+    }
+    return ZFB_OK;
+}
+
+int zfb_traces_reset(zfb_engine *e) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    e->trace_count = 0;      // launch order is stream order: the next update starts afresh
+    return ZFB_OK;
+}
+
+int64_t zfb_traces_count(const zfb_engine *e) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    return e->traces_on ? e->trace_count : 0;
+}
+
+// device address of a trace in row units (AVG: read out into its slot first, on e->stream)
+static int trace_vector(zfb_engine *e, int kind, const float **out) {
+    if (kind < ZFB_TRACE_LAST || kind > ZFB_TRACE_AVG) return fail(e, ZFB_EINVAL, "trace kind %d: must be 0..3", kind);
+    if (!e->traces_on) return fail(e, ZFB_ESTATE, "traces are off (zfb_traces_enable)");
+    if (!e->configured || e->trace_count < 1) return fail(e, ZFB_ESTATE, "the traces hold no row yet");
+    const int W = e->W;
+    const double *sum = (const double *)e->trace.p;
+    float *f = (float *)(sum + W);             // LAST, MAX, MIN, AVG
+    if (kind == ZFB_TRACE_AVG) {
+        ZFB_LAUNCH(trace_avg_kernel, dim3((unsigned)((W + 255) / 256)), dim3(256), 0, e->stream, sum,
+                   (long long)e->trace_count, W, (e->cfg.flags & ZFB_FLAG_LINEAR) ? 1 : 0, f + 3 * (size_t)W);
+        CK(e, cudaGetLastError());
+        e->counters[2] += 1;
+    }
+    *out = f + (size_t)kind * W;
+    return ZFB_OK;
+}
+
+int zfb_trace_read(zfb_engine *e, int kind, float *h_out) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    join_pending_work(e);
+    if (!h_out) return fail(e, ZFB_EINVAL, "trace_read: h_out is NULL");
+    CK(e, cudaSetDevice(e->device));
+    const float *src = nullptr;
+    const int rc = trace_vector(e, kind, &src);
+    if (rc) return rc;
+    const size_t bytes = (size_t)e->W * sizeof(float);
+    CK(e, cudaMemcpyAsync(h_out, src, bytes, cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->counters[4] += bytes;
+    return ZFB_OK;
+}
+
+// one peak query on e->stream over n floats at d_x; copies back the <= k markers only
+static int find_peaks(zfb_engine *e, const float *d_x, int n, int k, int distance, double height, int32_t *cols,
+                      float *values, double *offsets, int *npeaks) {
+    if (!d_x || !cols || !values || !offsets || !npeaks) return fail(e, ZFB_EINVAL, "find_peaks: NULL argument");
+    if (n < 1 || n > PK_MAX_N) return fail(e, ZFB_EINVAL, "find_peaks: n = %d must be in [1, %d]", n, PK_MAX_N);
+    if (k < 1 || k > PK_MAX) return fail(e, ZFB_EINVAL, "find_peaks: k = %d must be in [1, %d]", k, PK_MAX);
+    if (distance < 1) return fail(e, ZFB_EINVAL, "find_peaks: distance = %d must be >= 1", distance);
+    int rc = ensure(e, e->peaks, sizeof(PeakOut) + (size_t)n);
+    if (rc) return rc;
+    PeakParams pp{};
+    pp.x = d_x;
+    pp.n = n;
+    pp.k = k;
+    pp.distance = distance;
+    pp.use_height = height == height ? 1 : 0;
+    // x >= height on float values == x >= the smallest float not below height
+    float h = (float)height;
+    if (pp.use_height && (double)h < height) h = nextafterf(h, INFINITY);
+    pp.height = h;
+    pp.out = (PeakOut *)e->peaks.p;
+    pp.flag = (unsigned char *)e->peaks.p + sizeof(PeakOut);
+    ZFB_LAUNCH(trace_peaks_kernel, dim3(1), dim3(PK_NT), 0, e->stream, pp);
+    CK(e, cudaGetLastError());
+    e->counters[2] += 1;
+    PeakOut out;
+    CK(e, cudaMemcpyAsync(&out, e->peaks.p, sizeof out, cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->counters[4] += sizeof out;
+    *npeaks = out.count;
+    for (int i = 0; i < out.count; ++i) {
+        cols[i] = out.column[i];
+        values[i] = out.value[i];
+        offsets[i] = out.offset[i];
+    }
+    return ZFB_OK;
+}
+
+int zfb_trace_peaks(zfb_engine *e, int kind, int k, int distance, double height, int32_t *cols, float *values,
+                    double *offsets, int *npeaks) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    const float *src = nullptr;
+    const int rc = trace_vector(e, kind, &src);
+    if (rc) return rc;
+    return find_peaks(e, src, e->W, k, distance, height, cols, values, offsets, npeaks);
+}
+
+int zfb_find_peaks_device(zfb_engine *e, const float *d_x, int n, int k, int distance, double height, int32_t *cols,
+                          float *values, double *offsets, int *npeaks) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    return find_peaks(e, d_x, n, k, distance, height, cols, values, offsets, npeaks);
+}
+
 // channel-batched launches exist for the FAST path with one register-blocked
 // chain and fused strips (fft_ratio 4, 8, 16 on raw input); everything else
 // loops over the channels
@@ -2818,6 +3007,8 @@ static int check_channels(zfb_engine *e, const double *f_demod, int nch) {
     if (nch < 0 || (nch > 0 && !f_demod)) return fail(e, ZFB_EINVAL, "channels: bad arguments");
     if (nch > 0 && e->cfg.ema_alpha >= 0.0)
         return fail(e, ZFB_EINVAL, "channels: EMA state is per engine; configure with ema_alpha < 0");
+    if (nch > 0 && e->traces_on)
+        return fail(e, ZFB_EINVAL, "channels: the trace set is per engine; zfb_traces_enable(e, 0) first");
     if (nch > 0 && e->nstages == 0)
         return fail(e, ZFB_EINVAL, "channels: fft_ratio 1 has no software LO");
     return ZFB_OK;

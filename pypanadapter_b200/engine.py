@@ -188,6 +188,8 @@ class ZoomPSD:
         self._key = None               # a failed zfb_configure leaves the engine unconfigured
         self._check(self._lib.zfb_configure(self._h, C.byref(cfg)), "zfb_configure")
         self._key = key
+        self._axis = (float(fs), int(fft_size), fft_ratio_i, int(W), bool(onesided),
+                      float(f_demod) if fft_ratio_i > 1 and not no_lo else 0.0)
         self.row_width = int(W) // 2 + 1 if onesided else int(W)
         self.frame_len = int(frame_len)
         self.dtype = dtype
@@ -351,6 +353,78 @@ class ZoomPSD:
                     "zfb_read_rows")
         return out
 
+    # -- max-hold / min-hold / average traces and peak markers (DESIGN 3.8) --------
+    def traces_enable(self, on: bool = True):
+        """Keep the LAST / MAX / MIN / AVG traces on the device over every row the engine
+        computes from now on (starts them empty); ``False`` drops them."""
+        self._check(self._lib.zfb_traces_enable(self._h, 1 if on else 0), "zfb_traces_enable")
+
+    def traces_reset(self):
+        self._check(self._lib.zfb_traces_reset(self._h), "zfb_traces_reset")
+
+    @property
+    def trace_count(self) -> int:
+        """rows in the traces since they last started empty"""
+        return int(self._lib.zfb_traces_count(self._h))
+
+    def read_trace(self, kind: str) -> np.ndarray:
+        """Trace ``"last" | "max" | "min" | "avg"`` in the rows' units, float32 (row_width,)."""
+        out = np.empty(self.row_width, dtype=np.float32)
+        self._check(self._lib.zfb_trace_read(self._h, _trace_kind(kind), out.ctypes.data_as(C.POINTER(C.c_float))),
+                    "zfb_trace_read")
+        return out
+
+    def trace_peaks(self, kind: str, k: int = 8, distance: int = 1, height=None) -> np.ndarray:
+        """The ``k`` highest markers of ``scipy.signal.find_peaks(trace, height=height,
+        distance=distance)`` on trace ``kind``, highest first: a structured array of
+        ``column``, ``value``, ``offset`` (parabolic, in columns) and ``freq_hz``."""
+        kind_i = _trace_kind(kind)
+        return self._peaks(lambda *a: self._lib.zfb_trace_peaks(self._h, kind_i, *a), "zfb_trace_peaks",
+                           k, distance, height, self.row_width)
+
+    def find_peaks_device(self, ptr: int, n: int, k: int = 8, distance: int = 1, height=None) -> np.ndarray:
+        """The same markers for ``n`` float32 at device address ``ptr`` (e.g. a row of
+        ``process_device``); ``freq_hz`` is filled when ``n`` is the row width."""
+        return self._peaks(lambda *a: self._lib.zfb_find_peaks_device(self._h, C.c_void_p(ptr), int(n), *a),
+                           "zfb_find_peaks_device", k, distance, height, int(n))
+
+    def _peaks(self, call, what, k, distance, height, n):
+        k = int(k)
+        cols = np.zeros(max(k, 1), dtype=np.int32)
+        vals = np.zeros(max(k, 1), dtype=np.float32)
+        offs = np.zeros(max(k, 1), dtype=np.float64)
+        got = C.c_int(0)
+        self._check(call(k, int(distance), float("nan") if height is None else float(height),
+                         cols.ctypes.data_as(C.POINTER(C.c_int32)), vals.ctypes.data_as(C.POINTER(C.c_float)),
+                         offs.ctypes.data_as(C.POINTER(C.c_double)), C.byref(got)), what)
+        m = got.value
+        out = np.zeros(m, dtype=PEAK_DTYPE)
+        out["column"], out["value"], out["offset"] = cols[:m], vals[:m], offs[:m]
+        if self._key is not None and n == self.row_width:
+            out["freq_hz"] = self.row_frequencies()[cols[:m]] + offs[:m] * self._bin_hz()
+        else:
+            out["freq_hz"] = np.nan
+        return out
+
+    def _bin_hz(self) -> float:
+        fs, N, R, _W, _os, _f = self._axis
+        return fs / (R * N)
+
+    def row_frequencies(self) -> np.ndarray:
+        """Frequency of each row column in Hz (float64), by the column -> bin map of the
+        finalisation: (j - N/2) fs/(R N) for fftshifted bin j = column + N/2 - W/2, or
+        k fs/N for one-sided rows; plus f_demod where the chain mixes (R > 1, not no_lo)."""
+        if self._key is None:
+            raise ZoomFFTError(_lib.ZFB_ESTATE, "row_frequencies: engine is not configured")
+        fs, N, R, W, onesided, f_lo = self._axis
+        c = np.arange(self.row_width, dtype=np.int64)
+        os_lo = N // 2 - W // 2
+        if onesided:
+            M = N // 2 + 1
+            k = (c + os_lo + (M + 1) // 2) % M
+            return k * (fs / N)
+        return (c + os_lo - N // 2) * (fs / (R * N)) + f_lo
+
     def set_profiling(self, on: bool):
         self._check(self._lib.zfb_set_profiling(self._h, 1 if on else 0), "zfb_set_profiling")
 
@@ -449,6 +523,19 @@ class ZoomPSD:
         self._check(self._lib.zfb_get_counters(self._h, c), "zfb_get_counters")
         return dict(frames=int(c[0]), samples=int(c[1]), kernels=int(c[2]),
                     h2d_bytes=int(c[3]), d2h_bytes=int(c[4]))
+
+
+PEAK_DTYPE = np.dtype([("column", np.int32), ("value", np.float32), ("offset", np.float64),
+                       ("freq_hz", np.float64)])
+
+_TRACE_KINDS = {"last": _lib.ZFB_TRACE_LAST, "max": _lib.ZFB_TRACE_MAX, "min": _lib.ZFB_TRACE_MIN,
+                "avg": _lib.ZFB_TRACE_AVG}
+
+
+def _trace_kind(kind: str) -> int:
+    if kind not in _TRACE_KINDS:
+        raise ValueError("trace kind must be one of %s, got %r" % (", ".join(map(repr, _TRACE_KINDS)), kind))
+    return _TRACE_KINDS[kind]
 
 
 def _prof_name(c: int) -> str:
