@@ -153,27 +153,20 @@ int  zfb_reset_ema(zfb_engine *e);
  * "precise" = -1 (default: rows of <= 6 Welch segments take the fp64 path),
  * 0 never, 1 always.
  * Measurement knobs of mode FAST (defaults are the measured best; rows do not
- * depend on them beyond 1e-3 dB): "strips_async" 0 | 1 | 2 | 3 (edge strips on
- * the main stream | side stream, submitted first | after the FIR chain | beside
- * the last stage only), "strips_priority" 0 | 1, "strip_split", "strip_decay",
- * "strip_decay_early", "fir_threads" 128 | 256, "fir_generic", "iir_stream" 0 | 1
+ * depend on them beyond 1e-3 dB): "strips_async" 0 | 1 (edge strips on the
+ * main stream | side stream, submitted before the FIR chain), "strip_split",
+ * "strip_decay", "strip_decay_early", "fir_generic", "iir_stream" 0 | 1
  * (streaming last stage), "iir_stream_len", "iir_stream_warm", "iir_l2_keep",
- * "iir_depth" 0 | 1 | 2, "welch_prune" 0 | 1 | 2.
- * "slabs" = 2 (default 1: measured no faster): zfb_process_device batches of
- * >= "slab_min" (64) frames in mode FAST are cut into slabs that run through
- * two lane engines (own workspaces and streams) at the same time, the rows
- * finished in frame order on the engine's stream -- bit-identical to one lane.
+ * "welch_prune" 0 | 1 | 2.
+ * "slabs" = 0 | 1: accepted for existing callers and changes nothing (a batch
+ * always runs through one lane unless it is pipelined).
  * "pipeline": see zfb_join.
  * "host_taper" = 1 (default): zfb_process_host cuts a batch into sub-groups
  * that halve towards its end (copies overlap compute; only the last, smallest
  * sub-group's kernels are left after the last copy); 0: four equal sub-groups.
- * "big_cluster" = 0 (default) | 1 | 2: N = 65536 in one pass over clusters of
- * 16 CTAs exchanging the radix-16 blocks through distributed shared memory
- * (2: split-phase cluster barrier with the next segment prefetched); rows are
- * bit-identical to the default two-kernel path, which measured faster.
  * Unknown names: ZFB_EINVAL. */
 int  zfb_set_option(zfb_engine *e, const char *name, long long value);
-/* Lanes the last zfb_process_device batch ran through: 2 (slabs, pipeline) or 1. */
+/* Lanes the last zfb_process_device batch ran through: 2 (pipeline) or 1. */
 int  zfb_slab_lanes(const zfb_engine *e);
 /* Pipelined batches, zfb_set_option("pipeline", 1) (default 0; mode FAST, rows
  * on the fp32 path): zfb_process_device hands whole batches to the two lane

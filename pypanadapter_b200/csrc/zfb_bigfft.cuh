@@ -292,155 +292,6 @@ __global__ void __launch_bounds__(256) big_r16_kernel(const BigR16Params p) {
     for (int r = 1; r < 16; ++r) out[r * rstride] = cmul(v[r], w[r]);
 }
 
-// ---- N = 65536 in ONE pass: a cluster of 16 CTAs per (frame, split) -------------------------------
-// big_r16_kernel + scratch + welch_kernel<12,16>(prepared) without the scratch round trip: CTA c of
-// the cluster runs the front pass on columns n = 256 c .. 256 c + 255 of a segment (16 strided
-// loads, DC estimate, window, DFT16, W_N^(rn)) and stores output r straight into CTA r's shared
-// memory (DSMEM) at position n; after a cluster barrier CTA r holds block Z_r whole and runs the
-// 4096-point FFT on it, removes the rest of the segment mean (the 16 per-CTA sums travel the same
-// way) and accumulates |X|^2 over its segments.  The receive buffers alternate between segments, so
-// there is one cluster barrier per segment.  Same arithmetic, operation for operation, as the
-// two-kernel path: pow16 is bit-identical.
-struct BigClusterParams {
-    BigR16Params  r;               // front-pass operands (scratch / partial / means unused)
-    const float2 *twiddle_sub;     // S entries exp(-2 pi i k / S)
-    float        *pow16;           // [frames * 16][nsplit][S]
-    int           seg_per_split, nsplit;
-    const float2 *wf16;            // dense FFT(window) per residue, or
-    int           wf_n;            // ... its few non-zero bins
-    const int    *wf_bin;
-    const float2 *wf_val;
-};
-
-constexpr int BIGC_LOG2S = 12, BIGC_S = 1 << BIGC_LOG2S, BIGC_NT = 256, BIGC_CX = 16;
-constexpr int BIGC_FFT_SM = BIGC_S + (BIGC_S >> 4) + 1;            // fft_block's exchange area (float2)
-constexpr size_t BIGC_SMEM = (size_t)(2 * BIGC_S + BIGC_FFT_SM + 40 + 2 * BIGC_CX) * sizeof(float2);
-
-// PREFETCH: split-phase cluster barrier -- the 16 global loads of the NEXT segment are issued between
-// arrive and wait and stay in flight through the barrier and this segment's FFT (32 more registers:
-// the W_N^(rn) powers are then rebuilt per segment from 4 table lookups instead of being kept)
-template <int KIND, bool PREFETCH>
-__global__ void __launch_bounds__(BIGC_NT, 2) big_cluster_kernel(const BigClusterParams p) {
-    constexpr int S = BIGC_S, NT = BIGC_NT, PPT = 16;
-    ZFB_DYN_SMEM(smem_raw);
-    float2 *recv = reinterpret_cast<float2 *>(smem_raw);           // [2][S] block Z_rank of a segment
-    float2 *sm = recv + 2 * S;                                     // FFT exchange area
-    float2 *red = sm + BIGC_FFT_SM;                                // block_sum scratch (33)
-    float2 *part = red + 40;                                       // [2][16] the 16 CTAs' sample sums
-    const int tid = threadIdx.x;
-    const unsigned rank = cluster_rank();                          // == blockIdx.x: residue r of this CTA's block
-    const int split = blockIdx.y, frame = blockIdx.z;
-    const int N = S << 4;
-    const size_t esz = (KIND == KIND_U8_RAW) ? 2 : 8;
-    const char *frame_in = (const char *)p.r.in + (size_t)frame * (size_t)p.r.in_stride * esz;
-    const int n = (int)rank * NT + tid;                            // front-pass column of this thread
-    const float2 dc = __ldg(p.r.dc + frame);
-    const float inv_n = 1.0f / (float)N;
-
-    // the one thread of this CTA that owns a listed bin of a sparse FFT(window)
-    int sparse_m = -1;
-    if (p.wf_n > 0) {
-        for (int j = 0; j < p.wf_n; ++j) {
-            const int b = __ldg(p.wf_bin + j);
-            if ((b & 15) == (int)rank && ((b >> 4) & (NT - 1)) == tid) sparse_m = (b >> 4) / NT + PPT * j;
-        }
-    }
-
-    float acc[PPT];
-#pragma unroll
-    for (int m = 0; m < PPT; ++m) acc[m] = 0.f;
-    const int s_begin = split * p.seg_per_split;
-    const int s_end = min(p.r.nseg, s_begin + p.seg_per_split);
-
-    float2 x[16];                                                  // raw samples of the segment in front
-    if (PREFETCH && s_begin < s_end) {
-#pragma unroll
-        for (int q = 0; q < 16; ++q) x[q] = welch_fetch<KIND>(frame_in, s_begin * p.r.hop + n + S * q, p.r.len, p.r.flip);
-    }
-    cluster_sync();                                                // every CTA of the cluster is running
-    for (int s = s_begin; s < s_end; ++s) {
-        const int buf = (s - s_begin) & 1;
-        const int base = s * p.r.hop;
-        float2 v[16];
-        float2 raw_sum = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int q = 0; q < 16; ++q) {
-            const int idx = n + S * q;
-            float2 xv = PREFETCH ? x[q] : welch_fetch<KIND>(frame_in, base + idx, p.r.len, p.r.flip);
-            const float wn = __ldg(p.r.window + idx);
-            xv = make_float2(xv.x - dc.x, xv.y - dc.y);
-            raw_sum = cadd(raw_sum, xv);
-            v[q] = make_float2(xv.x * wn, xv.y * wn);
-        }
-        raw_sum = block_sum<NT>(raw_sum, tid, red);
-        if (tid < BIGC_CX) cluster_map(part + buf * BIGC_CX, (unsigned)tid)[rank] = raw_sum;
-        dft16(v);
-        {
-            // W_N^(r n), r = 1..15 (as big_r16_kernel)
-            float2 w[16];
-            w[1] = __ldg(p.r.twiddle + n);
-            w[2] = __ldg(p.r.twiddle + ((2 * n) & (N - 1)));
-            w[4] = __ldg(p.r.twiddle + ((4 * n) & (N - 1)));
-            w[8] = __ldg(p.r.twiddle + ((8 * n) & (N - 1)));
-            w[3] = cmul(w[1], w[2]);
-            w[5] = cmul(w[1], w[4]);
-            w[6] = cmul(w[2], w[4]);
-            w[7] = cmul(w[3], w[4]);
-#pragma unroll
-            for (int r = 9; r < 16; ++r) w[r] = cmul(w[r - 8], w[8]);
-            cluster_map(recv + buf * S, 0u)[n] = v[0];
-#pragma unroll
-            for (int r = 1; r < 16; ++r) cluster_map(recv + buf * S, (unsigned)r)[n] = cmul(v[r], w[r]);
-        }
-        if (PREFETCH) {
-            cluster_arrive();
-            if (s + 1 < s_end) {
-#pragma unroll
-                for (int q = 0; q < 16; ++q) x[q] = welch_fetch<KIND>(frame_in, base + p.r.hop + n + S * q, p.r.len, p.r.flip);
-            }
-            cluster_wait();
-        } else {
-            cluster_sync();                                        // block Z_rank and the 16 sums have arrived
-        }
-
-        float2 msum = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int t = 0; t < BIGC_CX; ++t) msum = cadd(msum, part[buf * BIGC_CX + t]);
-        const float2 mean = make_float2(msum.x * inv_n, msum.y * inv_n);
-#pragma unroll
-        for (int m = 0; m < PPT; ++m) v[m] = recv[buf * S + tid + m * NT];
-        fft_block<BIGC_LOG2S, PPT>(v, tid, p.twiddle_sub, sm);
-        if (p.wf_n > 0) {
-            if (sparse_m >= 0) {
-                const float2 c = cmul(make_float2(-mean.x, -mean.y), __ldg(p.wf_val + sparse_m / PPT));
-                const int own = sparse_m % PPT;
-#pragma unroll
-                for (int m = 0; m < PPT; ++m) {
-                    const float f = (m == own) ? 1.f : 0.f;
-                    v[m].x = fmaf(f, c.x, v[m].x);
-                    v[m].y = fmaf(f, c.y, v[m].y);
-                }
-            }
-        } else {
-            const float2 nm = make_float2(-mean.x, -mean.y);
-            const float2 *wf = p.wf16 + (size_t)rank * S + tid;
-#pragma unroll
-            for (int m = 0; m < PPT; ++m) v[m] = cadd(v[m], cmul(nm, __ldg(wf + m * NT)));
-        }
-#pragma unroll
-        for (int m = 0; m < PPT; ++m) acc[m] = fmaf(v[m].x, v[m].x, fmaf(v[m].y, v[m].y, acc[m]));
-    }
-    // no CTA may leave while another can still store into its shared memory: the last stores
-    // precede the last barrier, which every CTA has passed by now -- nothing more to wait for
-
-    float *row = p.pow16 + (((size_t)frame * 16 + rank) * p.nsplit + split) * S;
-#pragma unroll
-    for (int m = 0; m < PPT; ++m) {
-        const int k = tid + m * NT;
-        row[(k + S / 2) & (S - 1)] = acc[m];
-    }
-}
-
 // pow16 [frames*16][nsplit][S] (fftshifted sub-spectra) -> pow [frames][1][W]
 struct BigGatherParams {
     const float *pow16;

@@ -55,29 +55,24 @@ struct DevBuf {
 struct zfb_engine {
     int device = 0;
     int sm_count = 148;
-    // Slab pipelining (zfb_set_option("slabs") = 2): a large zfb_process_device batch is cut into
-    // slabs that alternate between two LANE engines (same plan and options, own workspaces, own
-    // streams).  A lane runs a slab up to the Welch power sums; this engine turns the sums into rows
-    // on its own stream, slab after slab (EMA strictly in frame order, dB20, ring) with the one-lane
-    // path's kernel on the same operands: rows are bit-identical.  What it buys: the FIR interior
-    // of one slab runs beside the latency-bound last stage / strips / Welch of the other.
-    int slabs = 1;                               // measured: no faster than one lane (profiles/r02aa, r02ab)
-    int slab_min = 64;                           // zfb_set_option("slab_min"): smallest batch cut into slabs
+    // Pipelined batches (zfb_set_option("pipeline") = 1): whole zfb_process_device batches alternate
+    // between two LANE engines (same plan and options, own workspaces, own streams).  A lane runs a
+    // batch up to the Welch power sums; this engine turns the sums into rows on fin_stream, in call
+    // order (EMA strictly in frame order, dB20, ring) with the one-lane path's kernel on the same
+    // operands: rows are bit-identical (virtual receivers: the lane finishes its rows itself).
+    // e->stream is NOT made to wait for them until zfb_join / zfb_synchronize (or any other call on
+    // the engine): the FIR interior of batch k + 1 runs beside the last stage / strips / Welch of batch k.
     bool is_lane = false, lanes_ready = false, lanes_stale = true;
     std::vector<double> window_host;             // the configured window (the caller's table may go away)
     zfb_engine *lane[2] = {nullptr, nullptr};
-    // Pipelined batches (zfb_set_option("pipeline") = 1): whole zfb_process_device batches alternate
-    // between the lanes and the rows are finished on fin_stream; e->stream is NOT made to wait for
-    // them until zfb_join / zfb_synchronize (or any other call on the engine): the FIR interior of
-    // batch k + 1 runs beside the last stage / strips / Welch of batch k.
     int pipeline = 0;
     int next_lane = 0;
     cudaStream_t fin_stream = nullptr;
     cudaEvent_t ev_done = nullptr;               // everything issued so far is finished (on fin_stream)
     bool join_pending = false;
-    int last_lanes = 1;                          // zfb_slab_lanes
+    int last_lanes = 1;                          // zfb_slab_lanes: 2 after a pipelined batch, else 1
     zfb_engine *last_front = nullptr;            // whose mid[] holds the last decimated chunks (debug read)
-    cudaEvent_t ev_slab_in = nullptr;            // the batch's input is ready (recorded on `stream`)
+    cudaEvent_t ev_batch_in = nullptr;           // the batch's input is ready (recorded on `stream`)
     cudaEvent_t ev_lane[2] = {nullptr, nullptr}; // a lane's power sums are ready
     cudaEvent_t ev_fin[2] = {nullptr, nullptr};  // ... and consumed: the lane may overwrite them
     bool ev_fin_used[2] = {false, false};
@@ -86,10 +81,8 @@ struct zfb_engine {
 
     cudaStream_t own_stream = nullptr, stream = nullptr, copy_stream = nullptr;
     cudaStream_t aux_stream = nullptr;           // edge strips of mode fast run beside the FIR interior
-    cudaStream_t aux_stream_hi = nullptr;        // the same at the highest stream priority (option strips_priority)
-    int strips_priority = 0;                     // 1: strip CTAs are dispatched ahead of pending interior CTAs
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    int strips_async = 1;                        // zfb_set_option("strips_async")
+    int strips_async = 1;                        // zfb_set_option("strips_async"): 0 = strips on the main stream
     int strip_split = 1;                         // zfb_set_option("strip_split"): narrower regions for the late strip stages
     int strip_decay = 192;                       // zfb_set_option("strip_decay"): samples between the last stage's cut and its outputs
     int strip_decay_early = 64;                  // zfb_set_option("strip_decay_early"): the same for the stages before it
@@ -97,7 +90,6 @@ struct zfb_engine {
     int late_mix = 1;                            // zfb_set_option("late_mix"): FIR chain may mix at its output
     int iir_stream = 1;                          // zfb_set_option("iir_stream"): streaming last stage of mode fast
     int iir_S = 640, iir_Wm = 256;               // zfb_set_option("iir_stream_len" (target) / "iir_stream_warm")
-    int iir_depth = 0;                           // zfb_set_option("iir_depth"): 0 = 3+3 tiles in flight per warp, 1 = 4+4, 2 = 5+4
     int iir_l2_keep = 70;                        // zfb_set_option("iir_l2_keep"): % of a stream's blocks kept in L2
     // plan of the streaming last stage (zfb_iirstream.cuh), valid while iis.active
     struct IirStreamPlan {
@@ -132,11 +124,7 @@ struct zfb_engine {
     float2 wf_sparse_val[WF_SPARSE_MAX] = {};
     int welch_prune = 2;               // 0: all bins accumulated; 1: only keepable ones; 2: + 3 CTAs/SM where it fits
     int host_taper = 1;                // zfb_set_option("host_taper"): host batches end in ever smaller sub-groups
-    int big_cluster = 0;               // zfb_set_option("big_cluster"): N = 65536 in one pass over a 16-CTA cluster (DSMEM)
-    int big_cluster_ok = -1;           // -1: not probed yet; 0: the device cannot hold such a cluster; 1: it can
     int fir_generic = 0;               // 1: never use the register-blocked FIR kernel (tests)
-    int fir_smem_pad = 0;              // zfb_set_option("fir_smem_pad"): bytes (measurement)
-    int fir_threads = 128;             // zfb_set_option("fir_threads"): 256 or 128 threads per CTA of fir_run_kernel
     int nperseg = 0, hop = 0, nseg = 0, W = 0, log2N = 0;
     int Wp = 0;                        // width of a pow row: W, or N for one-sided rows
     bool onesided = false;             // ZFB_FLAG_ONESIDED
@@ -650,13 +638,6 @@ template <int KIND> int fir_run_setup_kind(zfb_engine *e);
 int fir_run_setup_cs16(zfb_engine *e);
 constexpr int kIirNS = 3, kIirNO = 3;      // x pieces / output rows in flight per lane (zfb_iirstream.cuh)
 
-cudaError_t create_high_priority_stream(cudaStream_t *st) {
-    int lo = 0, hi = 0;                                  // numerically lower = higher priority
-    cudaError_t err = cudaDeviceGetStreamPriorityRange(&lo, &hi);
-    if (err != cudaSuccess) return err;
-    return cudaStreamCreateWithPriority(st, cudaStreamNonBlocking, hi);
-}
-
 int setup_device_once(zfb_engine *e) {
     DecimConst dc;
     build_decim_const(dc);
@@ -672,21 +653,6 @@ int setup_device_once(zfb_engine *e) {
             pc.zi[k][1] = z2;
         }
         CK(e, cudaMemcpyToSymbol(c_px, &pc, sizeof pc));
-    }
-    // the single-pass 65536-point kernel: > 48 KB of dynamic shared memory, clusters of 16 CTAs
-    // (above the portable 8); failures here only switch that path off
-    {
-        bool ok = true;
-        const void *fns[6] = {(const void *)big_cluster_kernel<KIND_U8_RAW, false>, (const void *)big_cluster_kernel<KIND_C64_RAW, false>,
-                              (const void *)big_cluster_kernel<KIND_C64_MID, false>, (const void *)big_cluster_kernel<KIND_U8_RAW, true>,
-                              (const void *)big_cluster_kernel<KIND_C64_RAW, true>, (const void *)big_cluster_kernel<KIND_C64_MID, true>};
-        for (const void *fn : fns) {
-            ok &= cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BIGC_SMEM) == cudaSuccess;
-            ok &= cudaFuncSetAttribute(fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
-        }
-        if (ok) ok = cluster_max_active(fns[1], dim3(BIGC_CX, 1, 1), dim3(BIGC_NT), BIGC_CX, BIGC_SMEM) >= 1;
-        cudaGetLastError();
-        e->big_cluster_ok = ok ? 1 : 0;
     }
     for (int kind = 0; kind < 3; ++kind)
         for (int nt : {NTHR_BIG, NTHR_SMALL})
@@ -728,10 +694,6 @@ int setup_device_once(zfb_engine *e) {
         CK(e, cudaFuncSetAttribute(chain_lookup_fn(kind), cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
     CK(e, cudaFuncSetAttribute((iir_stream_kernel<kIirNS, kIirNO>), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                (int)IirStreamShape<kIirNS, kIirNO>::SMEM));
-    CK(e, cudaFuncSetAttribute((iir_stream_kernel<4, 4>), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)IirStreamShape<4, 4>::SMEM));
-    CK(e, cudaFuncSetAttribute((iir_stream_kernel<5, 4>), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)IirStreamShape<5, 4>::SMEM));
     int rc = fir_run_setup_kind<KIND_C64_RAW>(e);
     if (rc == ZFB_OK) rc = fir_run_setup_kind<KIND_U8_RAW>(e);
     if (rc == ZFB_OK) rc = fir_run_setup_kind<KIND_C64_MID>(e);
@@ -902,22 +864,19 @@ void prof_end(zfb_engine *e, int idx, cudaStream_t on = nullptr) {
     X(5, KIND, 2, 3, 3, 0, -1)   \
     X(6, KIND, 3, 3, 3, 3, -1)
 
-// measurement knob (zfb_set_option("fir_smem_pad")): extra dynamic shared memory per CTA of the FIR run
-// kernel, i.e. fewer of them per SM -- leaves registers for other kernels' CTAs beside it
-static thread_local size_t g_fir_smem_pad = 0;
-
-template <int KIND, int NT>
+// 128-thread CTAs: 256 were slower (0.292 against 0.273 ms per 512 cfg2 frames, DESIGN §3.0)
+template <int KIND>
 void launch_fir_run_kind(int variant, const FirRunParams &rp, int L_out, int gf, cudaStream_t st) {
 #define ZFB_X(ID, K, NS, A, B, C, D)                                                              \
     if (variant == ID) {                                                                          \
-        using SH = FirRunShape<NS, A, B, C, D, NT>;                                               \
+        using SH = FirRunShape<NS, A, B, C, D, 128>;                                              \
         const int per_tile = SH::SPAN >> NS;                                                      \
         const unsigned tiles = (unsigned)((L_out + per_tile - 1) / per_tile);                     \
         if (K != KIND_C64_MID && rp.chan) {                                                       \
-            ZFB_LAUNCH((fir_run_kernel<K, NS, A, B, C, D, (K != KIND_C64_MID), NT>), dim3(tiles, (unsigned)gf), \
-                       dim3(NT), SH::SMEM + g_fir_smem_pad, st, rp);                              \
+            ZFB_LAUNCH((fir_run_kernel<K, NS, A, B, C, D, (K != KIND_C64_MID), 128>), dim3(tiles, (unsigned)gf), \
+                       dim3(128), SH::SMEM, st, rp);                                              \
         } else {                                                                                  \
-            ZFB_LAUNCH((fir_run_kernel<K, NS, A, B, C, D, false, NT>), dim3(tiles, (unsigned)gf), dim3(NT), SH::SMEM + g_fir_smem_pad, st, rp); \
+            ZFB_LAUNCH((fir_run_kernel<K, NS, A, B, C, D, false, 128>), dim3(tiles, (unsigned)gf), dim3(128), SH::SMEM, st, rp); \
         }                                                                                         \
         return;                                                                                   \
     }
@@ -940,20 +899,11 @@ void launch_fir_run_cs16(int variant, const FirRunParams &rp, int L_out, int gf,
 #undef ZFB_X
 }
 
-void launch_fir_run(int variant, int kind, const FirRunParams &rp, int L_out, int gf, cudaStream_t st, int nt) {
-    if (kind == KIND_CS16_RAW) {
-        launch_fir_run_cs16(variant, rp, L_out, gf, st);
-        return;
-    }
-    if (nt == 128) {
-        if (kind == KIND_U8_RAW) launch_fir_run_kind<KIND_U8_RAW, 128>(variant, rp, L_out, gf, st);
-        else if (kind == KIND_C64_RAW) launch_fir_run_kind<KIND_C64_RAW, 128>(variant, rp, L_out, gf, st);
-        else launch_fir_run_kind<KIND_C64_MID, 128>(variant, rp, L_out, gf, st);
-        return;
-    }
-    if (kind == KIND_U8_RAW) launch_fir_run_kind<KIND_U8_RAW, FIR_NT>(variant, rp, L_out, gf, st);
-    else if (kind == KIND_C64_RAW) launch_fir_run_kind<KIND_C64_RAW, FIR_NT>(variant, rp, L_out, gf, st);
-    else launch_fir_run_kind<KIND_C64_MID, FIR_NT>(variant, rp, L_out, gf, st);
+void launch_fir_run(int variant, int kind, const FirRunParams &rp, int L_out, int gf, cudaStream_t st) {
+    if (kind == KIND_CS16_RAW) launch_fir_run_cs16(variant, rp, L_out, gf, st);
+    else if (kind == KIND_U8_RAW) launch_fir_run_kind<KIND_U8_RAW>(variant, rp, L_out, gf, st);
+    else if (kind == KIND_C64_RAW) launch_fir_run_kind<KIND_C64_RAW>(variant, rp, L_out, gf, st);
+    else launch_fir_run_kind<KIND_C64_MID>(variant, rp, L_out, gf, st);
 }
 
 // which specialised variant (0 = none) handles this chain
@@ -972,13 +922,9 @@ int fir_run_variant(const FirChainParams &p) {
 template <int KIND>
 int fir_run_setup_kind(zfb_engine *e) {
 #define ZFB_X(ID, K, NS, A, B, C, D)                                                              \
-    CK(e, cudaFuncSetAttribute((fir_run_kernel<K, NS, A, B, C, D>), cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                               (int)FirRunShape<NS, A, B, C, D>::SMEM));                          \
     CK(e, cudaFuncSetAttribute((fir_run_kernel<K, NS, A, B, C, D, false, 128>), cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                               (int)FirRunShape<NS, A, B, C, D, 128>::SMEM + 64 * 1024));         \
+                               (int)FirRunShape<NS, A, B, C, D, 128>::SMEM));                     \
     if (K != KIND_C64_MID) {                                                                      \
-        CK(e, cudaFuncSetAttribute((fir_run_kernel<K, NS, A, B, C, D, (K != KIND_C64_MID)>),      \
-                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FirRunShape<NS, A, B, C, D>::SMEM)); \
         CK(e, cudaFuncSetAttribute((fir_run_kernel<K, NS, A, B, C, D, (K != KIND_C64_MID), 128>), \
                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FirRunShape<NS, A, B, C, D, 128>::SMEM)); \
     }
@@ -1009,14 +955,8 @@ ChainFn chain_lookup(int kind) {
 void launch_iir_stream(zfb_engine *e, int gf, cudaStream_t st) {
     const zfb_engine::IirStreamPlan &pl = e->iis;
     const unsigned ctas = (unsigned)(gf * pl.q.groups);
-    // tiles in flight per warp (option iir_depth): 3 + 3 (default), 4 + 4, 5 + 4
-    if (e->iir_depth == 1)
-        ZFB_LAUNCH((iir_stream_kernel<4, 4>), dim3(ctas), dim3(32), (IirStreamShape<4, 4>::SMEM), st, pl.tm_in, pl.tm_out, pl.q);
-    else if (e->iir_depth == 2)
-        ZFB_LAUNCH((iir_stream_kernel<5, 4>), dim3(ctas), dim3(32), (IirStreamShape<5, 4>::SMEM), st, pl.tm_in, pl.tm_out, pl.q);
-    else
-        ZFB_LAUNCH((iir_stream_kernel<kIirNS, kIirNO>), dim3(ctas), dim3(32), (IirStreamShape<kIirNS, kIirNO>::SMEM), st,
-                   pl.tm_in, pl.tm_out, pl.q);
+    ZFB_LAUNCH((iir_stream_kernel<kIirNS, kIirNO>), dim3(ctas), dim3(32), (IirStreamShape<kIirNS, kIirNO>::SMEM), st,
+               pl.tm_in, pl.tm_out, pl.q);
 }
 
 // the K samples at either end of every decimated chunk, computed by the exact edge strips into
@@ -1154,20 +1094,15 @@ cudaError_t run_decimation_fast(zfb_engine *e, const void *d_in, int gf, int *ou
     const int K = e->fplan.K;
     // Strips read only the raw input and own the first / last K decimated samples; the
     // interior owns the rest, so the two need no order between them: with k <= 4 the
-    // strips go to a side stream and fill the SMs beside the FIR interior.
+    // strips go to a side stream and fill the SMs beside the FIR interior.  They are submitted
+    // before the FIR chain, so their CTAs are dispatched first.
     const bool async_strips = e->strips_async && s0 == 0;
-    cudaStream_t aux = e->strips_priority ? e->aux_stream_hi : e->aux_stream;
     cudaError_t err = cudaSuccess;
-    // strips_async 1: strips are submitted before the FIR chain (their CTAs are dispatched
-    // first), 2: after it (they fill its tail and run beside the exact last stage)
-    const bool strips_first = e->strips_async == 1;
     if (async_strips) {
         if ((err = cudaEventRecord(e->ev_fork, st)) != cudaSuccess) return err;      // input ready, buffers free
-        if ((err = cudaStreamWaitEvent(aux, e->ev_fork, 0)) != cudaSuccess) return err;
-        if (strips_first) {
-            launch_fused_strips(e, d_in, gf, final_out, aux);
-            if ((err = cudaEventRecord(e->ev_join, aux)) != cudaSuccess) return err;
-        }
+        if ((err = cudaStreamWaitEvent(e->aux_stream, e->ev_fork, 0)) != cudaSuccess) return err;
+        launch_fused_strips(e, d_in, gf, final_out, e->aux_stream);
+        if ((err = cudaEventRecord(e->ev_join, e->aux_stream)) != cudaSuccess) return err;
     }
     const void *src = d_in_cs16 ? d_in_cs16 : d_in;
     long long src_stride = c.frame_len;
@@ -1191,9 +1126,7 @@ cudaError_t run_decimation_fast(zfb_engine *e, const void *d_in, int gf, int *ou
                 rp.chan = (const ChannelLo *)e->chan_dev.p;
                 rp.chan_frames = e->cur_chan_frames;
             }
-            g_fir_smem_pad = (size_t)e->fir_smem_pad;
-            launch_fir_run(e->chain_run[j], kind, rp, e->len[lvl], gf, st, e->fir_threads);
-            g_fir_smem_pad = 0;
+            launch_fir_run(e->chain_run[j], kind, rp, e->len[lvl], gf, st);
         } else {
             const unsigned tiles = (unsigned)((e->len[lvl] + p.TO - 1) / p.TO);
             ZFB_LAUNCH(chain_lookup(kind), dim3(tiles, (unsigned)gf), dim3(FIR_NT), e->chain_smem[j], st, p);
@@ -1204,17 +1137,6 @@ cudaError_t run_decimation_fast(zfb_engine *e, const void *d_in, int gf, int *ou
         src_stride = p.out_stride;
         kind = KIND_C64_MID;
         b ^= 1;
-    }
-    if (async_strips && !strips_first) {
-        if (e->strips_async == 3) {
-            // strips beside the last stage only: they wait for the FIR interior (which leaves no
-            // registers for them on an SM anyway) and share the SMs with the streaming last stage,
-            // one warp per CTA and DRAM-latency-bound
-            if ((err = cudaEventRecord(e->ev_fork, st)) != cudaSuccess) return err;
-            if ((err = cudaStreamWaitEvent(aux, e->ev_fork, 0)) != cudaSuccess) return err;
-        }
-        launch_fused_strips(e, d_in, gf, final_out, aux);
-        if ((err = cudaEventRecord(e->ev_join, aux)) != cudaSuccess) return err;
     }
     const int v = (e->decim_threads == NTHR_BIG) ? 0 : 1;
     {   // the last decimate call, exact, over the whole (FIR-filtered) chunk; it leaves the
@@ -1443,7 +1365,7 @@ int run_group_precise(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
 // int16 IQ converted by the first FIR chain's own loads (no widening pass over the chunk)?
 bool fir_cs16_fused(const zfb_engine *e) {
     return e->cs16_fused && e->fast_active && !e->precise_active && e->nchains >= 1 && e->chain_run[0] != 0 &&
-           e->fir_threads == 128 && e->cur_nch == 0;
+           e->cur_nch == 0;
 }
 
 // one group of frames, all resident on the device, through the whole chain
@@ -1591,48 +1513,6 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
         r.partial = r.scratch + ((size_t)e->group * (size_t)e->nseg << e->log2N);
         r.means = r.partial + (size_t)e->group * (size_t)e->nseg * (size_t)(S / 256);
         r.dc = r.means + (size_t)e->group * (size_t)e->nseg;
-        if (e->big_cluster && e->big_cluster_ok == 1 && e->log2N == 16) {
-            // one pass: clusters of 16 CTAs exchange the radix-16 blocks through shared memory
-            BigClusterParams cp{};
-            cp.r = r;
-            cp.twiddle_sub = (const float2 *)e->twiddle_sub.p;
-            cp.pow16 = (float *)e->pow16.p;
-            cp.seg_per_split = per;
-            cp.nsplit = ns16;
-            cp.wf16 = (const float2 *)e->winfft16.p;
-            cp.wf_n = e->wf_sparse_n;
-            cp.wf_bin = (const int *)e->wf_sparse.p;
-            cp.wf_val = (const float2 *)((const char *)e->wf_sparse.p + WF_SPARSE_MAX * sizeof(int));
-            const int prc = prof_begin(e, 16);
-            const dim3 gc((unsigned)BIGC_CX, (unsigned)ns16, (unsigned)gf);
-            if (kind == KIND_C64_RAW) {
-                ZFB_LAUNCH(big_dc_kernel<KIND_C64_RAW>, dim3((unsigned)gf), dim3(1024), 0, st, r);
-                if (e->big_cluster == 2) CK(e, ZFB_LAUNCH_CLUSTER((big_cluster_kernel<KIND_C64_RAW, true>), gc, dim3(BIGC_NT), BIGC_CX, BIGC_SMEM, st, cp));
-                else CK(e, ZFB_LAUNCH_CLUSTER((big_cluster_kernel<KIND_C64_RAW, false>), gc, dim3(BIGC_NT), BIGC_CX, BIGC_SMEM, st, cp));
-            } else if (kind == KIND_U8_RAW) {
-                ZFB_LAUNCH(big_dc_kernel<KIND_U8_RAW>, dim3((unsigned)gf), dim3(1024), 0, st, r);
-                if (e->big_cluster == 2) CK(e, ZFB_LAUNCH_CLUSTER((big_cluster_kernel<KIND_U8_RAW, true>), gc, dim3(BIGC_NT), BIGC_CX, BIGC_SMEM, st, cp));
-                else CK(e, ZFB_LAUNCH_CLUSTER((big_cluster_kernel<KIND_U8_RAW, false>), gc, dim3(BIGC_NT), BIGC_CX, BIGC_SMEM, st, cp));
-            } else {
-                ZFB_LAUNCH(big_dc_kernel<KIND_C64_MID>, dim3((unsigned)gf), dim3(1024), 0, st, r);
-                if (e->big_cluster == 2) CK(e, ZFB_LAUNCH_CLUSTER((big_cluster_kernel<KIND_C64_MID, true>), gc, dim3(BIGC_NT), BIGC_CX, BIGC_SMEM, st, cp));
-                else CK(e, ZFB_LAUNCH_CLUSTER((big_cluster_kernel<KIND_C64_MID, false>), gc, dim3(BIGC_NT), BIGC_CX, BIGC_SMEM, st, cp));
-            }
-            prof_end(e, prc);
-            const int prg = prof_begin(e, 17);
-            BigGatherParams g{};
-            g.pow16 = (const float *)e->pow16.p;
-            g.pow_out = (float *)e->pow.p;
-            g.log2N = e->log2N;
-            g.nsplit = ns16;
-            g.W = e->W;
-            g.frames = gf;
-            const long long cellsg = (long long)gf * e->W;
-            ZFB_LAUNCH(big_gather_kernel, dim3((unsigned)((cellsg + 255) / 256)), dim3(256), 0, st, g);
-            prof_end(e, prg);
-            e->counters[2] += 3;
-            nsplit = 1;
-        } else {
         const int pr = prof_begin(e, 16);
         const dim3 gr((unsigned)(S / 256), (unsigned)e->nseg, (unsigned)gf);
         if (kind == KIND_C64_RAW) {
@@ -1684,7 +1564,6 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
         prof_end(e, pr2);
         e->counters[2] += 5;
         nsplit = 1;
-        }
     } else {
         int want = e->welch_splits > 0 ? e->welch_splits : 4;
         if (want > e->nseg) want = e->nseg;
@@ -1725,7 +1604,7 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
     return ZFB_OK;
 }
 
-// rows of one launch group from the power sums in from->pow (this engine's, or a slab lane's): scale,
+// rows of one launch group from the power sums in from->pow (this engine's, or a lane's): scale,
 // EMA in frame order, dB20, ring -- on stream st (e->stream, or fin_stream for pipelined batches)
 int finish_rows(zfb_engine *e, zfb_engine *from, int gf, int nsplit, float *d_rows, cudaStream_t st) {
     const zfb_config &c = e->cfg;
@@ -2037,7 +1916,6 @@ int zfb_create(int device, zfb_engine **out) {
         if (cudaStreamCreateWithFlags(&e->own_stream, cudaStreamNonBlocking) != cudaSuccess ||
             cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking) != cudaSuccess ||
             cudaStreamCreateWithFlags(&e->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
-            create_high_priority_stream(&e->aux_stream_hi) != cudaSuccess ||
             cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
             cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming) != cudaSuccess) {
             rc = fail(nullptr, ZFB_ECUDA, "stream creation failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -2073,7 +1951,7 @@ void zfb_destroy(zfb_engine *e) {
         if (e->ev_lane[i]) cudaEventDestroy(e->ev_lane[i]);
         if (e->ev_fin[i]) cudaEventDestroy(e->ev_fin[i]);
     }
-    if (e->ev_slab_in) cudaEventDestroy(e->ev_slab_in);
+    if (e->ev_batch_in) cudaEventDestroy(e->ev_batch_in);
     if (e->fin_stream) {
         cudaStreamSynchronize(e->fin_stream);
         cudaStreamDestroy(e->fin_stream);
@@ -2082,7 +1960,6 @@ void zfb_destroy(zfb_engine *e) {
     if (e->own_stream) cudaStreamSynchronize(e->own_stream);
     if (e->copy_stream) cudaStreamSynchronize(e->copy_stream);
     if (e->aux_stream) cudaStreamSynchronize(e->aux_stream);
-    if (e->aux_stream_hi) cudaStreamSynchronize(e->aux_stream_hi);
     DevBuf *bufs[] = {&e->window, &e->winfft, &e->winfft16, &e->wf_sparse, &e->twiddle, &e->twiddle_sub, &e->pow16, &e->mid[0], &e->mid[1], &e->pow, &e->rows_tmp, &e->ema,
                       &e->img_out, &e->img_lut, &e->img_thr, &e->sel_hist, &e->ring, &e->stage_in[0], &e->stage_in[1], &e->big,
                       &e->trace, &e->trace_rows, &e->peaks};
@@ -2110,7 +1987,6 @@ void zfb_destroy(zfb_engine *e) {
     if (e->own_stream) cudaStreamDestroy(e->own_stream);
     if (e->copy_stream) cudaStreamDestroy(e->copy_stream);
     if (e->aux_stream) cudaStreamDestroy(e->aux_stream);
-    if (e->aux_stream_hi) cudaStreamDestroy(e->aux_stream_hi);
     if (e->ev_fork) cudaEventDestroy(e->ev_fork);
     if (e->ev_join) cudaEventDestroy(e->ev_join);
     delete e;
@@ -2430,12 +2306,12 @@ static int configure_impl(zfb_engine *e, const zfb_config *cfg) {
     return ZFB_OK;
 }
 
-// lanes of the slab pipeline: two engines on the same device with this engine's plan and options
+// lanes of the pipelined batches: two engines on the same device with this engine's plan and options
 // (best effort: any failure leaves the one-lane path in charge)
 static void setup_lanes(zfb_engine *e) {          // e->mu is held by the caller
     e->lanes_ready = false;
     e->lanes_stale = false;
-    if (e->is_lane || (e->slabs < 2 && !e->pipeline) || !e->configured || !e->fast_active || e->precise_active ||
+    if (e->is_lane || !e->pipeline || !e->configured || !e->fast_active || e->precise_active ||
         e->window_host.empty())
         return;
     // re-planning a lane may free workspaces that rows of earlier batches are still read from
@@ -2445,7 +2321,7 @@ static void setup_lanes(zfb_engine *e) {          // e->mu is held by the caller
     zfb_config c2 = e->cfg;
     c2.window = e->window_host.data();
     c2.ema_alpha = -1.0;                          // rows are finished by this engine: no EMA state in a lane
-    if (!e->ev_slab_in && cudaEventCreateWithFlags(&e->ev_slab_in, cudaEventDisableTiming) != cudaSuccess) return;
+    if (!e->ev_batch_in && cudaEventCreateWithFlags(&e->ev_batch_in, cudaEventDisableTiming) != cudaSuccess) return;
     for (int i = 0; i < 2; ++i) {
         if (!e->lane[i]) {
             if (zfb_create(e->device, &e->lane[i]) != ZFB_OK) { e->lane[i] = nullptr; return; }
@@ -2454,13 +2330,12 @@ static void setup_lanes(zfb_engine *e) {          // e->mu is held by the caller
         zfb_engine *l = e->lane[i];
         {
             std::lock_guard<std::mutex> lk2(l->mu);
-            l->strips_priority = e->strips_priority; l->strips_async = e->strips_async; l->strip_split = e->strip_split;
+            l->strips_async = e->strips_async; l->strip_split = e->strip_split;
             l->strip_decay = e->strip_decay; l->strip_decay_early = e->strip_decay_early; l->ring_append = 0;
             l->late_mix = e->late_mix; l->iir_stream = e->iir_stream; l->iir_S = e->iir_S; l->iir_Wm = e->iir_Wm;
-            l->iir_depth = e->iir_depth; l->iir_l2_keep = e->iir_l2_keep; l->precise = e->precise;
+            l->iir_l2_keep = e->iir_l2_keep; l->precise = e->precise;
             l->decim_threads = e->decim_threads; l->welch_splits = e->welch_splits; l->cs16_fused = e->cs16_fused;
-            l->welch_prune = e->welch_prune; l->fir_generic = e->fir_generic; l->fir_smem_pad = e->fir_smem_pad;
-            l->fir_threads = e->fir_threads; l->group_user = e->group_user;
+            l->welch_prune = e->welch_prune; l->fir_generic = e->fir_generic; l->group_user = e->group_user;
             l->fplan = e->fplan;
             l->configured = false;
         }
@@ -2475,49 +2350,6 @@ static void setup_lanes(zfb_engine *e) {          // e->mu is held by the caller
     e->lanes_ready = true;
 }
 
-// a batch in slabs: lane k & 1 runs slab k up to its power sums, this engine finishes the rows in order
-static int process_slabs(zfb_engine *e, const void *d_in, int nframes, float *d_rows) {
-    const size_t fbytes = (size_t)e->cfg.frame_len * sample_bytes(e->cfg);
-    // an even number of equal slabs, none above a launch group
-    const int nsl = 2 * ((nframes + 2 * e->group - 1) / (2 * e->group));
-    const int per = (nframes + nsl - 1) / nsl;
-    CK(e, cudaEventRecord(e->ev_slab_in, e->stream));
-    for (int i = 0; i < 2; ++i) {
-        zfb_engine *l = e->lane[i];
-        CK(e, cudaStreamWaitEvent(l->stream, e->ev_slab_in, 0));
-        l->profiling = e->profiling;
-    }
-    int rc = ZFB_OK;
-    for (int k = 0; k * per < nframes && rc == ZFB_OK; ++k) {
-        const int i = k & 1;
-        zfb_engine *l = e->lane[i];
-        const int f0 = k * per;
-        const int gf = (nframes - f0 < per) ? nframes - f0 : per;
-        if (e->ev_fin_used[i]) CK(e, cudaStreamWaitEvent(l->stream, e->ev_fin[i], 0));
-        int nsplit = 1;
-        bool done = false;
-        const uint64_t launches0 = l->counters[2];
-        rc = run_group_front(l, (const char *)d_in + (size_t)f0 * fbytes, gf, nullptr, &nsplit, &done);
-        e->counters[2] += l->counters[2] - launches0;
-        if (rc != ZFB_OK) {
-            e->err = l->err;
-            break;
-        }
-        CK(e, cudaEventRecord(e->ev_lane[i], l->stream));
-        CK(e, cudaStreamWaitEvent(e->stream, e->ev_lane[i], 0));
-        rc = finish_rows(e, l, gf, nsplit, d_rows ? d_rows + (size_t)f0 * e->W : nullptr, e->stream);
-        if (rc != ZFB_OK) break;
-        CK(e, cudaEventRecord(e->ev_fin[i], e->stream));
-        e->ev_fin_used[i] = true;
-    }
-    if (rc != ZFB_OK) {
-        // nothing of the lanes may still be running when the caller sees the error
-        for (int i = 0; i < 2; ++i) cudaStreamSynchronize(e->lane[i]->stream);
-        cudaGetLastError();
-    }
-    return rc;
-}
-
 // a whole batch on the next lane, its rows finished on fin_stream; e->stream joins later (zfb_join)
 static int process_pipelined(zfb_engine *e, const void *d_in, int nframes, float *d_rows) {
     const size_t fbytes = (size_t)e->cfg.frame_len * sample_bytes(e->cfg);
@@ -2525,9 +2357,9 @@ static int process_pipelined(zfb_engine *e, const void *d_in, int nframes, float
     e->next_lane ^= 1;
     zfb_engine *l = e->lane[i];
     // the input, and whatever the caller's stream did to the EMA state / ring before this call
-    CK(e, cudaEventRecord(e->ev_slab_in, e->stream));
-    CK(e, cudaStreamWaitEvent(l->stream, e->ev_slab_in, 0));
-    CK(e, cudaStreamWaitEvent(e->fin_stream, e->ev_slab_in, 0));
+    CK(e, cudaEventRecord(e->ev_batch_in, e->stream));
+    CK(e, cudaStreamWaitEvent(l->stream, e->ev_batch_in, 0));
+    CK(e, cudaStreamWaitEvent(e->fin_stream, e->ev_batch_in, 0));
     l->profiling = e->profiling;
     int rc = ZFB_OK;
     for (int g0 = 0; g0 < nframes && rc == ZFB_OK; g0 += e->group) {
@@ -2647,20 +2479,14 @@ int zfb_set_group(zfb_engine *e, int frames_per_group) {
 int zfb_set_option(zfb_engine *e, const char *name, long long value) {
     if (!e || !name) return ZFB_EINVAL;
     std::lock_guard<std::mutex> lk(e->mu);
-    e->lanes_stale = true;                       // the slab lanes take this engine's options when next used
-    if (strcmp(name, "slabs") == 0) {
-        if (value < 0 || value > 2) return fail(e, ZFB_EINVAL, "slabs must be 0, 1 (one lane) or 2");
-        e->slabs = (int)value;
+    e->lanes_stale = true;                       // the lanes take this engine's options when next used
+    if (strcmp(name, "slabs") == 0) {            // kept for callers that set it: 0 and 1 both mean one lane per batch
+        if (value < 0 || value > 1) return fail(e, ZFB_EINVAL, "slabs must be 0 or 1 (one lane)");
         return ZFB_OK;
     }
     if (strcmp(name, "pipeline") == 0) {
         join_pending_work(e);
         e->pipeline = value ? 1 : 0;
-        return ZFB_OK;
-    }
-    if (strcmp(name, "slab_min") == 0) {
-        if (value < 2 || value > (1 << 20)) return fail(e, ZFB_EINVAL, "slab_min (frames) must be in [2, 2^20]");
-        e->slab_min = (int)value;
         return ZFB_OK;
     }
     if (strcmp(name, "decim_threads") == 0) {
@@ -2684,11 +2510,8 @@ int zfb_set_option(zfb_engine *e, const char *name, long long value) {
         return ZFB_OK;
     }
     if (strcmp(name, "strips_async") == 0) {
-        e->strips_async = (value == 2 || value == 3) ? (int)value : (value ? 1 : 0);
-        return ZFB_OK;
-    }
-    if (strcmp(name, "strips_priority") == 0) {
-        e->strips_priority = value ? 1 : 0;
+        if (value < 0 || value > 1) return fail(e, ZFB_EINVAL, "strips_async must be 0 (main stream) or 1 (side stream)");
+        e->strips_async = (int)value;
         return ZFB_OK;
     }
     if (strcmp(name, "strip_decay") == 0) {
@@ -2730,11 +2553,6 @@ int zfb_set_option(zfb_engine *e, const char *name, long long value) {
         e->configured = false;
         return ZFB_OK;
     }
-    if (strcmp(name, "iir_depth") == 0) {
-        if (value < 0 || value > 2) return fail(e, ZFB_EINVAL, "iir_depth must be 0, 1 or 2");
-        e->iir_depth = (int)value;
-        return ZFB_OK;
-    }
     if (strcmp(name, "iir_l2_keep") == 0) {
         if (value < 0 || value > 100) return fail(e, ZFB_EINVAL, "iir_l2_keep is a percentage");
         e->iir_l2_keep = (int)value;
@@ -2752,23 +2570,8 @@ int zfb_set_option(zfb_engine *e, const char *name, long long value) {
         e->ring_append = value ? 1 : 0;
         return ZFB_OK;
     }
-    if (strcmp(name, "fir_smem_pad") == 0) {
-        if (value < 0 || value > 64 * 1024) return fail(e, ZFB_EINVAL, "fir_smem_pad must be in [0, 65536]");
-        e->fir_smem_pad = (int)value;
-        return ZFB_OK;
-    }
-    if (strcmp(name, "fir_threads") == 0) {
-        if (value != 128 && value != FIR_NT) return fail(e, ZFB_EINVAL, "fir_threads must be 128 or %d", FIR_NT);
-        e->fir_threads = (int)value;
-        return ZFB_OK;
-    }
     if (strcmp(name, "host_taper") == 0) {
         e->host_taper = value ? 1 : 0;
-        return ZFB_OK;
-    }
-    if (strcmp(name, "big_cluster") == 0) {
-        if (value < 0 || value > 2) return fail(e, ZFB_EINVAL, "big_cluster must be 0, 1 or 2 (split-phase barrier with prefetch)");
-        e->big_cluster = (int)value;
         return ZFB_OK;
     }
     if (strcmp(name, "fir_generic") == 0) {
@@ -3051,13 +2854,6 @@ static int process_device_impl(zfb_engine *e, const void *d_in, int nframes, con
         }
     }
     join_pending_work(e);
-    if (!e->is_lane && e->slabs >= 2 && nframes >= e->slab_min && nframes >= 2 && e->fast_active && !e->precise_active) {
-        if (e->lanes_stale) setup_lanes(e);
-        if (e->lanes_ready) {
-            e->last_lanes = 2;
-            return process_slabs(e, d_in, nframes, d_rows);
-        }
-    }
     e->last_lanes = 1;
     for (int g0 = 0; g0 < nframes; g0 += e->group) {
         const int gf = (nframes - g0 < e->group) ? nframes - g0 : e->group;
@@ -3075,8 +2871,8 @@ static int process_pipelined_channels(zfb_engine *e, const void *d_in, int nfram
     const int i = e->next_lane;
     e->next_lane ^= 1;
     zfb_engine *l = e->lane[i];
-    CK(e, cudaEventRecord(e->ev_slab_in, e->stream));
-    CK(e, cudaStreamWaitEvent(l->stream, e->ev_slab_in, 0));
+    CK(e, cudaEventRecord(e->ev_batch_in, e->stream));
+    CK(e, cudaStreamWaitEvent(l->stream, e->ev_batch_in, 0));
     l->profiling = e->profiling;
     uint64_t c0[5];
     memcpy(c0, l->counters, sizeof c0);
@@ -3245,7 +3041,7 @@ int zfb_debug_read_decimated(zfb_engine *e, float *h_out_iq, int max_samples) {
     int n = e->len[e->nstages];
     if (n > max_samples) n = max_samples;
     CK(e, cudaStreamSynchronize(e->stream));
-    const zfb_engine *src = e->last_front ? e->last_front : e;     // a slab lane, after a batch in slabs
+    const zfb_engine *src = e->last_front ? e->last_front : e;     // a lane, after a pipelined batch
     CK(e, cudaMemcpy(h_out_iq, src->mid[src->final_buf].p, (size_t)n * sizeof(float2), cudaMemcpyDeviceToHost));
     e->counters[4] += (size_t)n * sizeof(float2);
     return n;
@@ -3778,7 +3574,7 @@ int zfb_get_profile(zfb_engine *e, double ms_out[ZFB_PROF_CLASSES], uint64_t lau
     CK(e, cudaSetDevice(e->device));
     CK(e, cudaStreamSynchronize(e->stream));
     for (int c = 0; c < ZFB_PROF_CLASSES; ++c) { ms_out[c] = 0.0; launches_out[c] = 0; }
-    // the slab lanes' kernels belong to this engine's profile (e->stream has waited for all of them)
+    // the lanes' kernels belong to this engine's profile (e->stream has waited for all of them)
     for (zfb_engine *x : {e, e->lane[0], e->lane[1]}) {
         if (!x) continue;
         if (x != e) cudaStreamSynchronize(x->stream);

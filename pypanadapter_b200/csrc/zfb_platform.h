@@ -9,73 +9,10 @@
     ::cuemu::launch(kernel, grid, block, smem, __VA_ARGS__)
 #define ZFB_DYN_SMEM(name) unsigned char *name = ::cuemu::dyn_smem()
 #define ZFB_BUILD_KIND "emulated"
-// thread-block clusters of (cx, 1, 1) CTAs with distributed shared memory
-#define ZFB_LAUNCH_CLUSTER(kernel, grid, block, cx, smem, stream, ...) \
-    (::cuemu::launch_cluster(kernel, grid, block, cx, smem, __VA_ARGS__), cudaSuccess)
-namespace zfb {
-inline unsigned cluster_rank() { return ::cuemu::cluster_rank(); }
-inline void cluster_sync() { ::cuemu::cluster_sync(); }
-inline void cluster_arrive() {}
-inline void cluster_wait() { ::cuemu::cluster_sync(); }
-template <typename T> inline T *cluster_map(T *p, unsigned rank) { return ::cuemu::cluster_map(p, rank); }
-inline int cluster_max_active(const void *, dim3, dim3, unsigned, size_t) { return 1; }
-}  // namespace zfb
 #else
 #include <cuda_runtime.h>
 #define ZFB_LAUNCH(kernel, grid, block, smem, stream, ...) \
     kernel<<<grid, block, smem, stream>>>(__VA_ARGS__)
 #define ZFB_DYN_SMEM(name) extern __shared__ __align__(16) unsigned char name[]
 #define ZFB_BUILD_KIND "sm_100a"
-#include <cooperative_groups.h>
-// thread-block clusters of (cx, 1, 1) CTAs with distributed shared memory (cudaLaunchKernelEx)
-template <typename... KArgs, typename... Args>
-inline cudaError_t zfb_launch_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, unsigned cx, size_t smem,
-                                      cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = cx;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-#define ZFB_LAUNCH_CLUSTER(kernel, grid, block, cx, smem, stream, ...) \
-    zfb_launch_cluster(kernel, grid, block, cx, smem, stream, __VA_ARGS__)
-namespace zfb {
-__device__ __forceinline__ unsigned cluster_rank() { return cooperative_groups::this_cluster().block_rank(); }
-__device__ __forceinline__ void cluster_sync() { cooperative_groups::this_cluster().sync(); }
-// split-phase: stores before arrive are visible to every CTA after its wait
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
-template <typename T>
-__device__ __forceinline__ T *cluster_map(T *p, unsigned rank) {
-    return cooperative_groups::this_cluster().map_shared_rank(p, rank);
-}
-// clusters of this shape the device can hold at once (0: the launch would fail)
-inline int cluster_max_active(const void *kernel, dim3 grid, dim3 block, unsigned cx, size_t smem) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = cx;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, kernel, &cfg) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    return n;
-}
-}  // namespace zfb
 #endif

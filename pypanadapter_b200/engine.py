@@ -223,7 +223,7 @@ class ZoomPSD:
 
     @property
     def slab_lanes(self) -> int:
-        """lanes the last ``process_device`` batch ran through (2: cut into slabs)"""
+        """lanes the last ``process_device`` batch ran through (2: pipelined, else 1)"""
         return int(self._lib.zfb_slab_lanes(self._h))
 
     def join(self, cuda_stream_ptr: int | None = None):

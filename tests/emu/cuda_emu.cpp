@@ -71,115 +71,6 @@ static void run_cta(Cta &c, Idx bidx, dim3 block, dim3 grid) {
     }
 }
 
-thread_local Cluster *t_cluster = nullptr;
-
-// one cluster: the fibers of all its CTAs round-robin on this OS thread (static __shared__ storage
-// is per OS thread here, so cluster kernels may only use dynamic shared memory)
-static void run_cluster(Cluster &cl, Idx first, dim3 block, dim3 grid) {
-    t_cluster = &cl;
-    cl.arrived = 0;
-    const int nt = cl.ctas[0].nthreads;
-    cl.nfibers = (long)nt * (long)cl.ctas.size();
-    t_blockDim = Idx{block.x, block.y, block.z};
-    t_gridDim = Idx{grid.x, grid.y, grid.z};
-    long live = 0;
-    for (size_t r = 0; r < cl.ctas.size(); ++r) {
-        Cta &c = cl.ctas[r];
-        t_cta = &c;
-        c.bar_arrived = 0;
-        for (auto &g : c.bar_gen) g = 0;
-        for (auto &w : c.warps) { w.arrived = 0; memset(w.gen, 0, sizeof(w.gen)); }
-        c.live = c.nthreads;
-        live += c.live;
-        for (int t = 0; t < c.nthreads; ++t) {
-            Fiber &f = c.fib[t];
-            f.done = false;
-            f.wait_counter = nullptr;
-            f.cluster_gen = 0;
-            getcontext(&f.ctx);
-            f.ctx.uc_stack.ss_sp = f.stack;
-            f.ctx.uc_stack.ss_size = kStack;
-            f.ctx.uc_link = nullptr;
-            makecontext(&f.ctx, (void (*)())fiber_entry, 0);
-        }
-    }
-    while (live > 0) {
-        bool progressed = false;
-        live = 0;
-        for (size_t r = 0; r < cl.ctas.size(); ++r) {
-            Cta &c = cl.ctas[r];
-            for (int t = 0; t < c.nthreads; ++t) {
-                Fiber &f = c.fib[t];
-                if (f.done) continue;
-                if (f.wait_counter) {
-                    if (*f.wait_counter < f.wait_target) continue;
-                    f.wait_counter = nullptr;
-                }
-                t_cta = &c;
-                c.cur = t;
-                t_blockIdx = Idx{first.x + (unsigned)r, first.y, first.z};
-                t_threadIdx = Idx{(unsigned)t % block.x, ((unsigned)t / block.x) % block.y,
-                                  (unsigned)t / (block.x * block.y)};
-                swapcontext(&c.sched, &f.ctx);
-                progressed = true;
-            }
-            live += c.live;
-        }
-        if (!progressed && live > 0) {
-            fprintf(stderr, "cuda_emu: deadlock in cluster at CTA (%u,%u,%u): %ld fibers blocked\n", first.x,
-                    first.y, first.z, live);
-            abort();
-        }
-    }
-    t_cluster = nullptr;
-}
-
-void run_grid_cluster(const std::function<void()> &body, dim3 grid, dim3 block, unsigned cx, size_t smem) {
-    const int nthreads = (int)(block.x * block.y * block.z);
-    if (nthreads <= 0 || cx == 0 || grid.x % cx != 0) { fprintf(stderr, "cuda_emu: bad cluster launch\n"); abort(); }
-    const long nclusters = (long)(grid.x / cx) * grid.y * grid.z;
-    if (nclusters <= 0) return;
-    int nworkers = (int)std::thread::hardware_concurrency();
-    if (nworkers < 1) nworkers = 1;
-    if (nworkers > 16) nworkers = 16;
-    if (nworkers > nclusters) nworkers = (int)nclusters;
-    std::atomic<long> next{0};
-    auto worker = [&]() {
-        Cluster cl;
-        cl.ctas.resize(cx);
-        const size_t per_cta = kStack * (size_t)nthreads;
-        char *stacks = (char *)mmap(nullptr, per_cta * cx, PROT_READ | PROT_WRITE,
-                                    MAP_PRIVATE | MAP_ANONYMOUS | MAP_NORESERVE, -1, 0);
-        if (stacks == (char *)MAP_FAILED) { perror("cuda_emu mmap"); abort(); }
-        for (unsigned r = 0; r < cx; ++r) {
-            Cta &c = cl.ctas[r];
-            c.nthreads = nthreads;
-            c.fib.resize(nthreads);
-            c.bar_gen.assign(nthreads, 0);
-            c.warps.resize((nthreads + 31) / 32);
-            c.body = &body;
-            for (int t = 0; t < nthreads; ++t) c.fib[t].stack = stacks + per_cta * r + kStack * (size_t)t;
-            c.smem = (unsigned char *)aligned_alloc(128, ((smem + 127) / 128 + 1) * 128);
-        }
-        for (;;) {
-            const long b = next.fetch_add(1);
-            if (b >= nclusters) break;
-            const long ncx = grid.x / cx;
-            Idx first{(unsigned)(b % ncx) * cx, (unsigned)((b / ncx) % grid.y), (unsigned)(b / (ncx * grid.y))};
-            run_cluster(cl, first, block, grid);
-        }
-        for (auto &c : cl.ctas) free(c.smem);
-        munmap(stacks, per_cta * cx);
-    };
-    if (nworkers == 1) {
-        worker();
-    } else {
-        std::vector<std::thread> pool;
-        for (int i = 0; i < nworkers; ++i) pool.emplace_back(worker);
-        for (auto &th : pool) th.join();
-    }
-}
-
 void run_grid(const std::function<void()> &body, dim3 grid, dim3 block, size_t smem) {
     const int nthreads = (int)(block.x * block.y * block.z);
     const long nblocks = (long)grid.x * grid.y * grid.z;

@@ -63,7 +63,6 @@ struct Fiber {
     // wait descriptor: runnable when *counter >= target (counter == nullptr: runnable)
     const long *wait_counter = nullptr;
     long wait_target = 0;
-    long cluster_gen = 0;             // cluster barriers this fiber has arrived at
 };
 
 struct Warp {
@@ -89,36 +88,8 @@ struct Idx { unsigned int x, y, z; };
 extern thread_local Idx t_threadIdx, t_blockIdx, t_blockDim, t_gridDim;
 extern thread_local Cta *t_cta;
 
-// thread-block cluster (cluster dims (cx, 1, 1)): its CTAs run interleaved on ONE OS thread
-struct Cluster {
-    std::vector<Cta> ctas;
-    long arrived = 0;                 // cluster-barrier arrivals of all fibers
-    long nfibers = 0;
-};
-extern thread_local Cluster *t_cluster;
-
 void run_grid(const std::function<void()> &body, dim3 grid, dim3 block, size_t smem);
-void run_grid_cluster(const std::function<void()> &body, dim3 grid, dim3 block, unsigned cx, size_t smem);
 void yield_until(const long *counter, long target);
-
-inline unsigned cluster_rank() {
-    Cluster *cl = t_cluster;
-    return cl ? (unsigned)(t_cta - cl->ctas.data()) : 0u;
-}
-// barrier over all threads of the cluster (barrier.cluster.arrive.release + wait.acquire)
-inline void cluster_sync() {
-    Cluster *cl = t_cluster;
-    Fiber &f = t_cta->fib[t_cta->cur];
-    cl->arrived += 1;
-    f.cluster_gen += 1;
-    yield_until(&cl->arrived, f.cluster_gen * cl->nfibers);
-}
-// the address of `p` (in this CTA's dynamic shared memory) in the CTA of rank `rank` (mapa)
-template <typename T>
-inline T *cluster_map(T *p, unsigned rank) {
-    Cluster *cl = t_cluster;
-    return reinterpret_cast<T *>(cl->ctas[rank].smem + (reinterpret_cast<unsigned char *>(p) - t_cta->smem));
-}
 
 inline unsigned char *dyn_smem() { return t_cta->smem; }
 
@@ -126,12 +97,6 @@ template <typename... KArgs, typename... Args>
 inline void launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, Args... args) {
     std::function<void()> body = [=]() { kernel(args...); };
     run_grid(body, grid, block, smem);
-}
-
-template <typename... KArgs, typename... Args>
-inline void launch_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, unsigned cx, size_t smem, Args... args) {
-    std::function<void()> body = [=]() { kernel(args...); };
-    run_grid_cluster(body, grid, block, cx, smem);
 }
 
 }  // namespace cuemu
@@ -260,8 +225,7 @@ enum { cudaSuccess = 0, cudaErrorMemoryAllocation = 2, cudaErrorInvalidValue = 1
 enum cudaMemcpyKind { cudaMemcpyHostToDevice, cudaMemcpyDeviceToHost, cudaMemcpyDeviceToDevice,
                       cudaMemcpyHostToHost, cudaMemcpyDefault };
 enum { cudaStreamNonBlocking = 1, cudaEventDisableTiming = 2, cudaHostAllocDefault = 0 };
-enum cudaFuncAttribute { cudaFuncAttributeMaxDynamicSharedMemorySize = 8, cudaFuncAttributePreferredSharedMemoryCarveout = 9,
-                         cudaFuncAttributeNonPortableClusterSizeAllowed = 12 };
+enum cudaFuncAttribute { cudaFuncAttributeMaxDynamicSharedMemorySize = 8, cudaFuncAttributePreferredSharedMemoryCarveout = 9 };
 struct cudaDeviceProp { int multiProcessorCount; size_t sharedMemPerBlockOptin; int major, minor; int l2CacheSize; };
 struct cudaPointerAttributes { int type; };
 enum { cudaMemoryTypeUnregistered = 0, cudaMemoryTypeHost = 1, cudaMemoryTypeDevice = 2 };
@@ -296,8 +260,6 @@ static inline cudaError_t cudaMemset2DAsync(void *d, size_t pitch, int v, size_t
     return cudaSuccess;
 }
 static inline cudaError_t cudaStreamCreateWithFlags(cudaStream_t *s, unsigned) { *s = (void *)1; return cudaSuccess; }
-static inline cudaError_t cudaDeviceGetStreamPriorityRange(int *lo, int *hi) { *lo = 0; *hi = -5; return cudaSuccess; }
-static inline cudaError_t cudaStreamCreateWithPriority(cudaStream_t *s, unsigned, int) { *s = (void *)1; return cudaSuccess; }
 static inline cudaError_t cudaStreamDestroy(cudaStream_t) { return cudaSuccess; }
 static inline cudaError_t cudaStreamSynchronize(cudaStream_t) { return cudaSuccess; }
 static inline cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }

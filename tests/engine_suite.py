@@ -91,58 +91,6 @@ class TorchDevice:
         return obj.cpu().numpy()
 
 
-def slabs_equal_one_lane(engine, dev, nframes=7, w=None, n=None):
-    """zfb_process_device cuts large batches into slabs that run through two lane engines at the
-    same time (option ``slabs``); the rows -- EMA carried across slabs, groups and calls, ring
-    content, counters -- must equal the one-lane path's bit for bit (frames are independent:
-    S:2092, S:2098, S:2111)."""
-    w = w or synth.CFG2
-    n = n or 4096 * 16 * 4 + 1234           # 7 Welch segments: the fp32 path
-    frames = synth.make_frames(w, nframes, n=n)
-    p_in, keep = dev.put(frames)
-
-    def run(slabs, group, calls):
-        engine.set_option("slabs", slabs)
-        engine.set_option("slab_min", 2)
-        engine.set_group(group)
-        engine.ring_configure(4)
-        engine.configure(w.fs, w.fft_size, w.fft_ratio, n, w.window, dtype="u8", flip=True, crop="thread",
-                         ema_alpha=0.3)
-        assert engine.fast_active
-        engine.reset_ema()
-        k0 = engine.counters()
-        p_rows, rows = dev.empty((nframes, engine.row_width))
-        f0 = 0
-        fbytes = frames[0].nbytes
-        for cnt in calls:
-            engine.process_device(p_in + f0 * fbytes, cnt, p_rows + f0 * engine.row_width * 4)
-            f0 += cnt
-        engine.synchronize()
-        assert engine.slab_lanes == slabs
-        k1 = engine.counters()
-        return dev.get(rows), engine.read_rows(4), engine.read_decimated().shape, \
-            {k: k1[k] - k0[k] for k in ("frames", "samples")}
-
-    try:
-        want = run(1, 0, [nframes])
-        for group, calls in ((0, [nframes]), (2, [nframes]), (0, [3, nframes - 3]), (3, [nframes - 2, 2])):
-            got = run(2, group, calls)
-            assert np.array_equal(got[0], want[0]), (group, calls)
-            assert np.array_equal(got[1], want[1]), (group, calls)
-            assert got[2] == want[2] and got[3] == want[3]
-        # one engine option changed between batches reaches the lanes
-        engine.set_option("slabs", 2)
-        engine.set_option("strips_async", 0)
-        got = run(2, 0, [nframes])
-        assert np.array_equal(got[0], want[0])
-    finally:
-        engine.set_option("strips_async", 1)
-        engine.set_option("slabs", 1)
-        engine.set_option("slab_min", 64)
-        engine.set_group(0)
-        engine.ring_configure(256)
-
-
 def ema_batch_independent(engine):
     """EMA rows do not depend on where a launch group or a call ends -- on the fp64 path of
     few-segment rows too (its state between launches is fp32 like the fp32 path's)."""
@@ -168,7 +116,9 @@ def ema_batch_independent(engine):
 def pipeline_equals_one_lane(engine, dev, nframes=9, w=None, n=None):
     """``pipeline`` = 1: whole batches alternate between the lane engines, rows are finished on a
     stream of the engine's own and the caller's stream joins later (zfb_join).  Rows, EMA across
-    batches, ring, counters: bit-identical to the plain path; other calls join implicitly."""
+    batches, ring, counters: bit-identical to the plain path; other calls join implicitly.  An
+    option changed between batches reaches the lanes, and the decimated chunk is read from the
+    lane that ran the last batch."""
     w = w or synth.CFG2
     n = n or 4096 * 16 * 4 + 1234           # 7 Welch segments: the fp32 path
     frames = synth.make_frames(w, nframes, n=n)
@@ -197,7 +147,8 @@ def pipeline_equals_one_lane(engine, dev, nframes=9, w=None, n=None):
             engine.join()
         engine.synchronize()
         k1 = engine.counters()
-        return dev.get(rows)[:f0], engine.read_rows(4), tail, {k: k1[k] - k0[k] for k in ("frames", "samples")}
+        return dev.get(rows)[:f0], engine.read_rows(4), tail, {k: k1[k] - k0[k] for k in ("frames", "samples")}, \
+            engine.read_decimated().shape
 
     try:
         for host_tail in (0, 2):
@@ -208,8 +159,15 @@ def pipeline_equals_one_lane(engine, dev, nframes=9, w=None, n=None):
                 assert np.array_equal(got[0], want[0]), (group, calls)
                 assert np.array_equal(got[1], want[1]), (group, calls)
                 assert (got[2] is None and want[2] is None) or np.array_equal(got[2], want[2])
-                assert got[3] == want[3]
+                assert got[3] == want[3] and got[4] == want[4]
+        # one engine option changed between batches reaches the lanes (want: the last host_tail's)
+        engine.set_option("strips_async", 0)
+        got = run(1, 0, [3, nframes - host_tail - 3], host_tail)
+        assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1])
+        assert (got[2] is None and want[2] is None) or np.array_equal(got[2], want[2])
+        assert got[3] == want[3] and got[4] == want[4]
     finally:
+        engine.set_option("strips_async", 1)
         engine.set_option("pipeline", 0)
         engine.set_group(0)
         engine.ring_configure(256)
@@ -291,7 +249,9 @@ def error_paths(engine):
         engine.ring_quantiles(16, 1, 1, [1.5])                       # quantile outside [0, 1]
     with pytest.raises(ZoomFFTError):
         engine.set_option("no_such_knob", 1)
-    for name, bad in (("slabs", 3), ("slab_min", 1), ("big_cluster", 3), ("welch_splits", 17)):
+    for name, bad in (("slabs", 3), ("slab_min", 1), ("big_cluster", 3), ("welch_splits", 17), ("slabs", 2),
+                      ("strips_async", 2), ("iir_depth", 0), ("strips_priority", 0), ("fir_smem_pad", 0),
+                      ("fir_threads", 128)):
         with pytest.raises(ZoomFFTError):
             engine.set_option(name, bad)
     # pipelined batches fall back to the plain path where there are no lanes (mode exact, fft_ratio 2):
@@ -666,11 +626,10 @@ def pipeline_random_ops(engine, dev, seed=0, nops=40):
         engine.ring_configure(256)
 
 
-def big_cluster_equals_scratch(engine, nframes=3):
-    """N = 65536 in one pass over a 16-CTA cluster (option ``big_cluster``; blocks of the radix-16
-    front pass exchanged through distributed shared memory) == the two-kernel path through the
-    scratch buffer, bit for bit (same arithmetic, only the data movement differs); and parity against
-    the oracle.  Sparse (hann) and dense (kaiser) FFT(window) tables, uint8 + flip and complex64."""
+def big_r16_parity(engine, nframes=3):
+    """N = 65536 on the radix-16 path (front pass into the scratch buffer, then the one-CTA FFT of
+    every block of N/16) against the oracle: a DC offset, sparse (hann) and dense (kaiser)
+    FFT(window) tables, complex64; uint8 + flip gives finite rows."""
     fs, N = 2.4e6, 65536
     for window, dtype, nsegs in (("hann", "c64", 7), (("kaiser", 8.6), "c64", 3), ("hamming", "u8", 4)):
         n = N * (nsegs + 1) // 2 + 321
@@ -680,22 +639,17 @@ def big_cluster_equals_scratch(engine, nframes=3):
             xs.append((x + np.complex64(0.2 - 0.1j)).astype(np.complex64) * np.complex64(0.6))
         x = np.stack(xs)
         wire = np.stack([synth.quantise_u8(f) for f in x]) if dtype == "u8" else x
-        rows = {}
         try:
             engine.set_option("precise", 0)                  # keep few-segment rows on the fp32 path
-            for on in (0, 1, 2):                             # 2: split-phase barrier, next segment prefetched
-                engine.set_option("big_cluster", on)
-                engine.configure(fs, N, 1, n, window, dtype=dtype, flip=(dtype == "u8"), crop=None)
-                rows[on] = engine.process(wire)
+            engine.configure(fs, N, 1, n, window, dtype=dtype, flip=(dtype == "u8"), crop=None)
+            rows = engine.process(wire)
         finally:
-            engine.set_option("big_cluster", 0)
             engine.set_option("precise", -1)
-        assert np.array_equal(rows[0], rows[1]), (window, dtype)
-        assert np.array_equal(rows[0], rows[2]), (window, dtype)
+        assert rows.shape[0] == nframes and np.all(np.isfinite(rows)), (window, dtype)
         if dtype == "c64":
             want = zo.zoom_psd(x[0], fs, N, 1, window, crop=None)
-            parity.assert_row_parity(rows[1][0].astype(np.float64), want, parity.floor_db20(fs, window, N, False) + 30.0,
-                                     "big cluster %s" % (window,))
+            parity.assert_row_parity(rows[0].astype(np.float64), want, parity.floor_db20(fs, window, N, False) + 30.0,
+                                     "radix-16 %s" % (window,))
 
 
 def random_configs(engine, seed, count):

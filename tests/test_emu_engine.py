@@ -23,10 +23,6 @@ def test_batch_equals_single(emu_engine, emu_lib):
     es.batch_equals_single(emu_engine, emu_lib)
 
 
-def test_slabs_equal_one_lane(emu_engine):
-    es.slabs_equal_one_lane(emu_engine, es.HostAsDevice())
-
-
 def test_pipeline_equals_one_lane(emu_engine):
     es.pipeline_equals_one_lane(emu_engine, es.HostAsDevice())
 
@@ -47,8 +43,8 @@ def test_pipeline_random_ops(emu_engine, seed):
     es.pipeline_random_ops(emu_engine, es.HostAsDevice(), seed=seed, nops=30)
 
 
-def test_big_cluster_equals_scratch(emu_engine):
-    es.big_cluster_equals_scratch(emu_engine, nframes=2)
+def test_big_r16_parity(emu_engine):
+    es.big_r16_parity(emu_engine, nframes=2)
 
 
 def test_ema_batch_independent(emu_engine):

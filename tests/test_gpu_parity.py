@@ -33,36 +33,6 @@ def test_ema_batch_independent(gpu_engine):
     es.ema_batch_independent(gpu_engine)
 
 
-def test_slabs_equal_one_lane(gpu_engine):
-    es.slabs_equal_one_lane(gpu_engine, es.TorchDevice())
-
-
-def test_slabs_equal_one_lane_full_size(gpu_engine):
-    """cfg2 at its full frame length, 160 frames in slabs of 40 across both lanes (several slabs per
-    lane: the lanes' power sums are reused while the rows of earlier slabs are being finished)."""
-    import torch
-    w = synth.CFG2
-    frames = synth.make_frames(w, 160, distinct=160)
-    d_in = torch.from_numpy(frames).cuda()
-    rows = {}
-    for slabs in (1, 2):
-        gpu_engine.set_option("slabs", slabs)
-        gpu_engine.set_group(40)
-        gpu_engine.configure(w.fs, w.fft_size, w.fft_ratio, w.frame_len, w.window, dtype="u8", flip=True,
-                             crop="thread", ema_alpha=w.ema_alpha)
-        gpu_engine.reset_ema()
-        d_rows = torch.zeros((160, gpu_engine.row_width), dtype=torch.float32, device="cuda")
-        torch.cuda.synchronize()
-        for _ in range(3):                      # back-to-back batches: the EMA runs on across them
-            gpu_engine.process_device(d_in.data_ptr(), 160, d_rows.data_ptr())
-        gpu_engine.synchronize()
-        assert gpu_engine.slab_lanes == slabs
-        rows[slabs] = d_rows.cpu().numpy()
-    gpu_engine.set_group(0)
-    assert np.array_equal(rows[1], rows[2])
-    assert np.isfinite(rows[2]).all()
-
-
 def test_pipeline_equals_one_lane(gpu_engine):
     es.pipeline_equals_one_lane(gpu_engine, es.TorchDevice())
 
@@ -115,8 +85,8 @@ def test_pipeline_full_size_and_join_stream(gpu_engine):
     assert np.isfinite(out[1]).all()
 
 
-def test_big_cluster_equals_scratch(gpu_engine):
-    es.big_cluster_equals_scratch(gpu_engine, nframes=5)
+def test_big_r16_parity(gpu_engine):
+    es.big_r16_parity(gpu_engine, nframes=5)
 
 
 def test_batch_equals_single(gpu_engine, gpu_lib):

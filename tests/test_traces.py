@@ -15,7 +15,7 @@ def test_exact_against_numpy(emu_engine):
     ts.exact_against_numpy(emu_engine)
 
 
-def test_batch_independence(emu_engine):
+def test_traces_independent_of_batching(emu_engine):
     ts.batch_independence(emu_engine, es.HostAsDevice())
 
 
@@ -46,7 +46,7 @@ def test_exact_against_numpy_gpu(gpu_engine):
 
 
 @pytest.mark.gpu
-def test_batch_independence_gpu(gpu_engine):
+def test_traces_independent_of_batching_gpu(gpu_engine):
     ts.batch_independence(gpu_engine, es.TorchDevice())
 
 

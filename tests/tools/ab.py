@@ -1,7 +1,7 @@
 """A/B measurement of engine tuning options (zfb_set_option) in ONE process, so
 that a variant costs seconds of GPU time instead of a box:
 
-    python -m tests.tools.ab --workload cfg2 --set strips_async=1,0,2 --set late_mix=1,0
+    python -m tests.tools.ab --workload cfg2 --set strips_async=1,0 --set late_mix=1,0
     python -m tests.tools.ab --workload cfg1 --mode exact --set decim_threads=0,128,256
 
 Every combination of the listed values is configured on the same engine and

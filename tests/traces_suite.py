@@ -180,8 +180,8 @@ def exact_against_numpy(engine):
 
 
 def batch_independence(engine, dev, nframes=37):
-    """The same 37 frames in one batch, 5 + 32, one by one, through the host path, pipelined
-    batches and slabs: all four traces bit-identical, 37 rows counted each time."""
+    """The same 37 frames in one batch, 5 + 32, one by one, through the host path and pipelined
+    batches: all four traces bit-identical, 37 rows counted each time."""
     w = synth.CFG2
     frames = synth.make_frames(w, nframes, n=N7)
     p_in, keep = dev.put(frames)
@@ -208,7 +208,7 @@ def batch_independence(engine, dev, nframes=37):
         assert engine.trace_count == nframes, name
         results[name] = {k: engine.read_trace(k) for k in ("last", "max", "min", "avg")}
         for k in opts:
-            engine.set_option(k, {"slabs": 1, "slab_min": 64}.get(k, 0))
+            engine.set_option(k, 0)
 
     try:
         run("one batch", lambda: device_calls([nframes]))
@@ -219,8 +219,6 @@ def batch_independence(engine, dev, nframes=37):
         run("host path", lambda: engine.process(frames))
         run("pipelined", lambda: device_calls([5, 32]), pipeline=1)
         run("pipelined, no rows", lambda: device_calls([20, 17], rows_too=False), pipeline=1)
-        run("slabs", lambda: device_calls([nframes]), slabs=2, slab_min=2)
-        run("slabs, no rows", lambda: device_calls([nframes], rows_too=False), slabs=2, slab_min=2)
     finally:
         engine.set_group(0)
         engine.traces_enable(False)
