@@ -1,5 +1,5 @@
-// Welch PSD for FFT sizes that do not fit one CTA (N = 2^14 .. 2^18): a
-// four-step FFT, N = N1 * N2, as two kernels per group of frames.
+// Welch PSD for FFT sizes that do not fit one CTA: a four-step FFT, N = N1 * N2,
+// for N = 2^14, 2^15 and 2^18 (the radix-16 path further down takes 2^16 and 2^17).
 //
 // Same reference lines as zfb_welch.cuh (scipy.signal.welch called from
 // pypanadapter_spectrum.py:2111 / pypanadapter_thread.py:1536,1538); this is
@@ -16,8 +16,9 @@
 //
 // detrend='constant' needs the segment mean before windowing, but a column
 // tile only sees 1/16..1/64 of a segment.  FFT(w*(x-m)) = FFT(w*x) - m*FFT(w),
-// so the col pass also emits per-tile sums of the raw samples and the row pass
-// subtracts m * Wf[k] (Wf = FFT of the window, fp64 on the host) per segment.
+// so the col pass removes the frame's DC estimate (big_dc_kernel) before the
+// window, emits per-tile sums of what is left, and the row pass subtracts
+// (m - estimate) * Wf[k] (Wf = FFT of the window, fp64 on the host) per segment.
 #pragma once
 #include "zfb_welch.cuh"
 
@@ -38,8 +39,9 @@ struct BigParams {
     const float2 *twiddle;     // N entries exp(-2 pi i k / N)
     const float2 *winfft;      // N entries FFT(window)
     float2       *scratch;     // [frames][nseg][N]  (k1-major)
-    float2       *partial;     // [frames][nseg][ntiles_col] raw sums
-    float2       *means;       // [frames][nseg] segment means
+    float2       *partial;     // [frames][nseg][ntiles_col] sums of the samples less the DC estimate
+    float2       *means;       // [frames][nseg] segment means less the frame's DC estimate
+    float2       *dc;          // [frames] DC estimate of the frame (big_dc_kernel)
     int           W;
     float        *pow_out;     // [frames][nsplit][W]
 };
@@ -70,6 +72,36 @@ __device__ __forceinline__ void sub_fft(float2 (&v)[8], int j, float2 *sub, cons
     }
 }
 
+// A frame's DC estimate from 8192 samples spread over it (32 KB of an 8 MB row).  It is removed
+// BEFORE the window, the rest of each segment's mean after the FFT: exact in exact arithmetic
+// whatever the estimate is, and in fp32 the post-FFT correction then cancels a term proportional
+// to |segment mean - estimate| instead of |segment mean| (a chunk with a DC offset of 0.4 and
+// noise at 2e-3 read 0.015 dB20 off next to the DC bin with the plain post-FFT removal, DESIGN 3.3).
+constexpr int BIG_DC_SAMPLES = 8192;
+// P: BigParams (four-step path) or BigR16Params (radix-16 path).
+template <int KIND, class P>
+__global__ void __launch_bounds__(1024) big_dc_kernel(const P p) {
+    __shared__ float2 red[33];
+    const int frame = blockIdx.x, t = threadIdx.x;
+    const size_t esz = (KIND == KIND_U8_RAW) ? 2 : 8;
+    const char *frame_in = (const char *)p.in + (size_t)frame * (size_t)p.in_stride * esz;
+    const int used = (p.nseg + 1) * p.hop;                   // samples the segments cover
+    const int stride = used / BIG_DC_SAMPLES > 0 ? used / BIG_DC_SAMPLES : 1;
+    // 8 independent loads per thread (a serial loop of 32 took 20 us per launch: 32 DRAM round trips)
+    float2 x[BIG_DC_SAMPLES / 1024];
+#pragma unroll
+    for (int j = 0; j < BIG_DC_SAMPLES / 1024; ++j) {
+        const long long idx = (long long)(t + 1024 * j) * stride;
+        x[j] = idx < used ? welch_fetch<KIND>(frame_in, (int)idx, p.len, p.flip) : make_float2(0.f, 0.f);
+    }
+    float2 sum = make_float2(0.f, 0.f);
+#pragma unroll
+    for (int j = 0; j < BIG_DC_SAMPLES / 1024; ++j) sum = cadd(sum, x[j]);
+    sum = block_sum<1024>(sum, t, red);
+    const int cnt = (used + stride - 1) / stride < BIG_DC_SAMPLES ? (used + stride - 1) / stride : BIG_DC_SAMPLES;
+    if (t == 0) p.dc[frame] = make_float2(sum.x / (float)cnt, sum.y / (float)cnt);
+}
+
 template <int LM, int KIND>
 __global__ void __launch_bounds__(BIG_THREADS) bigfft_col_kernel(const BigParams p) {
     constexpr int M = 1 << LM;            // N1
@@ -91,11 +123,13 @@ __global__ void __launch_bounds__(BIG_THREADS) bigfft_col_kernel(const BigParams
 
     float2 v[8];
     float2 sum = make_float2(0.f, 0.f);
+    const float2 dc = __ldg(p.dc + frame);
 #pragma unroll
     for (int q = 0; q < 8; ++q) {
         const int idx = ((j + q * (M / 8)) << log2N2) + n2;
-        const float2 x = welch_fetch<KIND>(frame_in, base + idx, p.len, p.flip);
+        float2 x = welch_fetch<KIND>(frame_in, base + idx, p.len, p.flip);
         const float w = __ldg(p.window + idx);
+        x = make_float2(x.x - dc.x, x.y - dc.y);
         sum = cadd(sum, x);
         v[q] = make_float2(x.x * w, x.y * w);
     }
@@ -114,7 +148,7 @@ __global__ void __launch_bounds__(BIG_THREADS) bigfft_col_kernel(const BigParams
     }
 }
 
-// segment means from the column pass's per-tile raw sums (fixed summation order)
+// segment means (less the DC estimate) from the column pass's per-tile sums (fixed summation order)
 __global__ void bigfft_mean_kernel(const BigParams p, int nsegs_total) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nsegs_total) return;
@@ -181,7 +215,7 @@ __global__ void __launch_bounds__(BIG_THREADS, 2) bigfft_row_kernel(const BigPar
 }
 
 // ===========================================================================
-// N = 2^14 .. 2^17: decimation in frequency by 16 in front of the one-CTA FFT.
+// N = 2^16 and 2^17: decimation in frequency by 16 in front of the one-CTA FFT.
 //   X[16k + r] = FFT_S( Z_r )[k],  S = N/16,
 //   Z_r[n] = W_N^(r n) * sum_q x[n + S q] W_16^(q r),   x = window * (segment - mean)
 // big_r16_kernel     : window + 16-point DFT across the 16 blocks + twiddle, coalesced in and
@@ -207,35 +241,6 @@ struct BigR16Params {
     float2       *dc;          // [frames] DC estimate of the frame (big_dc_kernel)
     float2       *scratch;     // [frames][16][nseg][S]
 };
-
-// A frame's DC estimate from 8192 samples spread over it (32 KB of an 8 MB row).  It is removed
-// BEFORE the window, the rest of each segment's mean after the FFT: exact in exact arithmetic
-// whatever the estimate is, and in fp32 the post-FFT correction then cancels a term proportional
-// to |segment mean - estimate| instead of |segment mean| (a chunk with a DC offset of 0.4 and
-// noise at 2e-3 read 0.015 dB20 off next to the DC bin with the plain post-FFT removal).
-constexpr int BIG_DC_SAMPLES = 8192;
-template <int KIND>
-__global__ void __launch_bounds__(1024) big_dc_kernel(const BigR16Params p) {
-    __shared__ float2 red[33];
-    const int frame = blockIdx.x, t = threadIdx.x;
-    const size_t esz = (KIND == KIND_U8_RAW) ? 2 : 8;
-    const char *frame_in = (const char *)p.in + (size_t)frame * (size_t)p.in_stride * esz;
-    const int used = (p.nseg + 1) * p.hop;                   // samples the segments cover
-    const int stride = used / BIG_DC_SAMPLES > 0 ? used / BIG_DC_SAMPLES : 1;
-    // 8 independent loads per thread (a serial loop of 32 took 20 us per launch: 32 DRAM round trips)
-    float2 x[BIG_DC_SAMPLES / 1024];
-#pragma unroll
-    for (int j = 0; j < BIG_DC_SAMPLES / 1024; ++j) {
-        const long long idx = (long long)(t + 1024 * j) * stride;
-        x[j] = idx < used ? welch_fetch<KIND>(frame_in, (int)idx, p.len, p.flip) : make_float2(0.f, 0.f);
-    }
-    float2 sum = make_float2(0.f, 0.f);
-#pragma unroll
-    for (int j = 0; j < BIG_DC_SAMPLES / 1024; ++j) sum = cadd(sum, x[j]);
-    sum = block_sum<1024>(sum, t, red);
-    const int cnt = (used + stride - 1) / stride < BIG_DC_SAMPLES ? (used + stride - 1) / stride : BIG_DC_SAMPLES;
-    if (t == 0) p.dc[frame] = make_float2(sum.x / (float)cnt, sum.y / (float)cnt);
-}
 
 // segment means (less the DC estimate) from the front pass's per-CTA sums (fixed summation order)
 __global__ void big_mean16_kernel(const BigR16Params p, int nsegs_total) {
@@ -325,6 +330,8 @@ inline int big_ntiles_col(int log2N) {
     return (1 << lm2) / (BIG_TILE >> lm1);
 }
 
+// scratch [frames][nseg][N], then per frames x nseg: the tile sums (ntiles_col = N/4096 on both
+// paths), the segment means, and room for one more float2 -- dc[frames] lives there (nseg >= 1)
 inline size_t big_scratch_bytes(int log2N, int nseg, int frames) {
     return (size_t)frames * (size_t)nseg * (((size_t)1 << log2N) + (size_t)big_ntiles_col(log2N) + 2) * sizeof(float2);
 }
@@ -341,8 +348,15 @@ inline void big_launch_col(const BigParams &p, int kind, dim3 grid, cudaStream_t
     }
 }
 
-// enqueue the column pass for `frames` frames
+// enqueue the frames' DC estimates and the column pass for `frames` frames
 inline void big_run_col(const BigParams &p, int kind, int frames, cudaStream_t st) {
+    if (kind == KIND_C64_RAW) {
+        ZFB_LAUNCH((big_dc_kernel<KIND_C64_RAW, BigParams>), dim3((unsigned)frames), dim3(1024), 0, st, p);
+    } else if (kind == KIND_U8_RAW) {
+        ZFB_LAUNCH((big_dc_kernel<KIND_U8_RAW, BigParams>), dim3((unsigned)frames), dim3(1024), 0, st, p);
+    } else {
+        ZFB_LAUNCH((big_dc_kernel<KIND_C64_MID, BigParams>), dim3((unsigned)frames), dim3(1024), 0, st, p);
+    }
     int lm1, lm2;
     big_split(p.log2N, lm1, lm2);
     dim3 gcol((unsigned)p.ntiles_col, (unsigned)p.nseg, (unsigned)frames);

@@ -1516,13 +1516,13 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
         const int pr = prof_begin(e, 16);
         const dim3 gr((unsigned)(S / 256), (unsigned)e->nseg, (unsigned)gf);
         if (kind == KIND_C64_RAW) {
-            ZFB_LAUNCH(big_dc_kernel<KIND_C64_RAW>, dim3((unsigned)gf), dim3(1024), 0, st, r);
+            ZFB_LAUNCH((big_dc_kernel<KIND_C64_RAW, BigR16Params>), dim3((unsigned)gf), dim3(1024), 0, st, r);
             ZFB_LAUNCH(big_r16_kernel<KIND_C64_RAW>, gr, dim3(256), 0, st, r);
         } else if (kind == KIND_U8_RAW) {
-            ZFB_LAUNCH(big_dc_kernel<KIND_U8_RAW>, dim3((unsigned)gf), dim3(1024), 0, st, r);
+            ZFB_LAUNCH((big_dc_kernel<KIND_U8_RAW, BigR16Params>), dim3((unsigned)gf), dim3(1024), 0, st, r);
             ZFB_LAUNCH(big_r16_kernel<KIND_U8_RAW>, gr, dim3(256), 0, st, r);
         } else {
-            ZFB_LAUNCH(big_dc_kernel<KIND_C64_MID>, dim3((unsigned)gf), dim3(1024), 0, st, r);
+            ZFB_LAUNCH((big_dc_kernel<KIND_C64_MID, BigR16Params>), dim3((unsigned)gf), dim3(1024), 0, st, r);
             ZFB_LAUNCH(big_r16_kernel<KIND_C64_MID>, gr, dim3(256), 0, st, r);
         }
         const int nsegs_total = gf * e->nseg;
@@ -1588,6 +1588,7 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
         b.scratch = (float2 *)e->big.p;
         b.partial = b.scratch + ((size_t)e->group * (size_t)e->nseg << e->log2N);
         b.means = b.partial + (size_t)e->group * (size_t)e->nseg * (size_t)b.ntiles_col;
+        b.dc = b.means + (size_t)e->group * (size_t)e->nseg;
         b.W = e->W;
         b.pow_out = (float *)e->pow.p;
         const int pr = prof_begin(e, 16);
@@ -1596,7 +1597,7 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
         const int pr2 = prof_begin(e, 17);
         big_run_row(b, gf, st);
         prof_end(e, pr2);
-        e->counters[2] += 3;
+        e->counters[2] += 4;
     }
 
     CK(e, cudaGetLastError());
