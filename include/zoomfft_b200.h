@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ZFB_ABI_VERSION 3
+#define ZFB_ABI_VERSION 4
 
 /* status codes */
 #define ZFB_OK            0
@@ -320,6 +320,52 @@ int  zfb_ring_quantiles(zfb_engine *e, int height, int scroll, int64_t rows_seen
                         const double *q, int nq, double *out_values,
                         int64_t *out_count);
 
+/* ---- decaying persistence spectrum (DESIGN 3.9) ----------------------------
+ * The reference plots each row as it arrives (spectrum_plot.setData(psd),
+ * S:2130) and keeps nothing across rows.  A persistence set extends that plot
+ * with a spectrum analyser's persistence (level-density) display: how the level
+ * at each frequency is distributed over time.  It is one float32 intensity per
+ * (level bin, column), P[256][row_width], kept on the device over the same rows
+ * as the trace set (every row of zfb_process_device, zfb_process_host and
+ * zfb_samples_process on every path, also rows that never reach the ring; not
+ * rows of zfb_ring_push_rows).  The level bin of a row value v is the
+ * waterfall's colour index of v for (minlev, maxlev):
+ * clip(trunc((double(v) - minlev) * 256 / (maxlev - minlev)), 0, 255), in the
+ * rows' own units (dB20, or linear power with ZFB_FLAG_LINEAR); values below
+ * the range and -inf land in bin 0, values above it in bin 255.  Bin k covers
+ * row values from minlev + k (maxlev - minlev) / 256 up.  Per row, strictly in
+ * frame order, every cell becomes
+ *     P[k][c] = fl(fl(P[k][c] * decay) + (k == bin(row[c]) ? 1 : 0))
+ * with both operations rounded separately (numpy's float32 P * decay + hit), so
+ * the state is bit-identical however the frames are split into calls, groups or
+ * pipelined batches.  decay = 1: exact hit counts, up to 2^24 per cell (a cell
+ * stops counting there: 2^24 + 1 rounds back to 2^24).  decay < 1: a fading
+ * persistence, bounded by 1 / (1 - decay).  Off by default: then nothing is
+ * allocated or launched.  On, it costs 1 KB of device memory per column.  It
+ * starts empty on zfb_persist_enable (which also sets minlev, maxlev and decay),
+ * zfb_persist_reset and a zfb_configure that changes fs, fft_size, fft_ratio,
+ * row_width, f_demod or flags; it keeps counting over a change of frame_len,
+ * window, ema_alpha, dtype, flip or mode.  While it is on,
+ * zfb_process_channels_* return ZFB_EINVAL (one set per engine).
+ * zfb_persist_enable: ZFB_EINVAL for a non-finite level, maxlev <= minlev or
+ * decay outside (0, 1] (only checked when on != 0); ZFB_ENOMEM when the state
+ * cannot be allocated (the set is then off). */
+#define ZFB_PERSIST_LEVELS 256
+int  zfb_persist_enable(zfb_engine *e, int on, double minlev, double maxlev, double decay);
+int  zfb_persist_reset(zfb_engine *e);
+/* rows since the set last started empty; 0 while off */
+int64_t zfb_persist_count(const zfb_engine *e);
+/* [256][row_width] image of the set, row 0 = level bin 255 (high levels at the
+ * top, as a spectrum plot is drawn).  kind ZFB_IMAGE_F32: the intensities;
+ * ZFB_IMAGE_U8: colour indices of the intensities for (imin, imax) by the same
+ * pyqtgraph mapping as zfb_ring_image; ZFB_IMAGE_RGBA: lut_rgba[index].  Host
+ * out blocks; device out is asynchronous on the engine's stream.  Joins pending
+ * pipelined work first.  ZFB_EINVAL for an unknown kind, imax <= imin (U8,
+ * RGBA), RGBA without a table or out == NULL; ZFB_ESTATE when the set is off or
+ * holds no row. */
+int  zfb_persist_image(zfb_engine *e, int kind, double imin, double imax,
+                       const uint8_t *lut_rgba, void *out, int out_on_device);
+
 /* ---- taper design and preview on the device (SURVEY 8f.4) ----------------
  * The taper dialog's live preview (FFTTaperingControl.ShowCurve, S:1354-1379):
  * zfb_taper_design replaces scipy.signal.get_window(AppState.fft_tapering, 51)
@@ -378,8 +424,9 @@ int  zfb_get_counters(const zfb_engine *e, uint64_t out5[5]);
 /* kernel classes: 0..15 = decimate-by-2 stage s (replaces scipy.signal.
  * decimate call s of the loop at S:2097-2098), 16 = Welch kernel / four-step
  * column pass, 17 = four-step row pass (both: scipy.signal.welch, S:2111),
- * 18 = row finalisation (S:2114-2119 + EMA, trace update), 19 = waterfall image
- * (S:1625-1664), 20 = autolevel selection sweep (S:1676). */
+ * 18 = row finalisation (S:2114-2119 + EMA, trace and persistence updates),
+ * 19 = waterfall image (S:1625-1664) and persistence image, 20 = autolevel
+ * selection sweep (S:1676). */
 #define ZFB_PROF_CLASSES 21
 /* on != 0: bracket every kernel launch with CUDA events on the engine's
  * stream (no host synchronisation is added). */

@@ -32,7 +32,7 @@ ZFB_FLAG_NO_LO = 1
 ZFB_FLAG_LINEAR = 2
 ZFB_FLAG_ONESIDED = 4
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 PROF_CLASSES = 21
 ZFB_IMAGE_F32 = 0
 ZFB_IMAGE_U8 = 1
@@ -41,6 +41,7 @@ ZFB_TRACE_LAST = 0
 ZFB_TRACE_MAX = 1
 ZFB_TRACE_MIN = 2
 ZFB_TRACE_AVG = 3
+ZFB_PERSIST_LEVELS = 256
 
 
 class ZfbConfig(C.Structure):
@@ -113,6 +114,10 @@ SYMBOLS = {
     "zfb_find_peaks_device": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_int32),
                                         C.POINTER(C.c_float), C.POINTER(C.c_double), C.POINTER(C.c_int)]),
     "zfb_ring_image": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_double, C.c_double, _P, _P, C.c_int]),
+    "zfb_persist_enable": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, C.c_double]),
+    "zfb_persist_reset": (C.c_int, [_P]),
+    "zfb_persist_count": (C.c_int64, [_P]),
+    "zfb_persist_image": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, _P, _P, C.c_int]),
     "zfb_ring_quantiles": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, C.POINTER(C.c_double), C.c_int,
                                      C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "zfb_taper_design": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(C.c_double)]),

@@ -30,6 +30,7 @@
 #include "zfb_taper.cuh"
 #include "zfb_precise.cuh"
 #include "zfb_trace.cuh"
+#include "zfb_persist.cuh"
 
 using namespace zfb;
 
@@ -154,8 +155,16 @@ struct zfb_engine {
     int64_t trace_count = 0;           // rows in the traces (host side; launch order = stream order)
     double trace_key[6] = {0, 0, 0, 0, 0, 0};   // fs, N, R, row_width, f_demod, flags of the last configure
     DevBuf trace;                      // [W] fp64 sums, then LAST, MAX, MIN, AVG read-out [4][W] float
-    DevBuf trace_rows;                 // [group][W] rows of a launch group the caller did not ask for
+    DevBuf trace_rows;                 // [group][W] rows of a launch group the caller did not ask for (traces
+                                       // or persistence on)
     DevBuf peaks;                      // PeakOut, then one flag byte per element
+    // persistence set (zfb_persist_enable; zfb_persist.cuh): nothing is allocated or launched while it is off
+    bool persist_on = false;
+    int64_t persist_count = 0;         // rows in the set (host side; launch order = stream order)
+    float persist_decay = 1.f;
+    LevelMap persist_lv{};             // row value -> level bin for the set's (minlev, maxlev)
+    DevBuf persist;                    // [256][W] intensities, level-major
+    DevBuf persist_thr;                // the 257 level thresholds of persist_lv, built at enable
 
     // ZFB_MODE_FAST
     struct FastPlan {
@@ -1226,9 +1235,10 @@ cudaError_t run_decimation_fast(zfb_engine *e, const void *d_in, int gf, int *ou
     return cudaSuccess;
 }
 
-// traces on: the rows of a launch group go to the caller's buffer or, without one, to this scratch
+// traces or persistence on: the rows of a launch group go to the caller's buffer or, without one,
+// to this scratch
 float *trace_rows_or(zfb_engine *e, float *d_rows) {
-    return (d_rows || !e->traces_on || e->cur_nch > 0) ? d_rows : (float *)e->trace_rows.p;
+    return (d_rows || !(e->traces_on || e->persist_on) || e->cur_nch > 0) ? d_rows : (float *)e->trace_rows.p;
 }
 
 // fold `nf` finished rows into the trace set, on the stream that finished them (after them)
@@ -1252,6 +1262,34 @@ int trace_update(zfb_engine *e, const float *rows, int nf, cudaStream_t st) {
     e->trace_count += nf;
     CK(e, cudaGetLastError());
     return ZFB_OK;
+}
+
+// fold `nf` finished rows into the persistence set, on the stream that finished them (after them)
+int persist_update(zfb_engine *e, const float *rows, int nf, cudaStream_t st) {
+    if (!e->persist_on || e->cur_nch > 0 || nf < 1) return ZFB_OK;
+    PersistParams pp{};
+    pp.rows = rows;
+    pp.nframes = nf;
+    pp.W = e->W;
+    pp.have = e->persist_count > 0 ? 1 : 0;
+    pp.decay = e->persist_decay;
+    pp.state = (float *)e->persist.p;
+    pp.lv = e->persist_lv;
+    const int pr = prof_begin(e, 18, st);
+    ZFB_LAUNCH(persist_update_kernel, dim3((unsigned)((e->W + PS_COLS - 1) / PS_COLS), (unsigned)PS_SLICES),
+               dim3(PS_NT), 0, st, pp);
+    prof_end(e, pr, st);
+    e->counters[2] += 1;
+    e->persist_count += nf;
+    CK(e, cudaGetLastError());
+    return ZFB_OK;
+}
+
+// every row the engine finishes (not the rows of channel-batched launches) feeds the trace and
+// persistence sets that are on
+int rows_finished(zfb_engine *e, const float *rows, int nf, cudaStream_t st) {
+    const int rc = trace_update(e, rows, nf, st);
+    return rc ? rc : persist_update(e, rows, nf, st);
 }
 
 // fp64 path (zfb_precise.cuh): rows of few Welch segments, `gf` frames resident on the device
@@ -1351,7 +1389,7 @@ int run_group_precise(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
         e->counters[2] += 2;
         if (rp.alpha >= 0.0) e->ema_have = true;
         if (to_ring) e->ring_written += nf;
-        const int rc = trace_update(e, rp.rows, nf, st);
+        const int rc = rows_finished(e, rp.rows, nf, st);
         if (rc) return rc;
     }
     CK(e, cudaGetLastError());
@@ -1643,7 +1681,7 @@ int finish_rows(zfb_engine *e, zfb_engine *from, int gf, int nsplit, float *d_ro
     e->counters[2] += 1;
     prof_end(e, prf, st);
     CK(e, cudaGetLastError());
-    const int rc = trace_update(e, f.rows, gf, st);
+    const int rc = rows_finished(e, f.rows, gf, st);
     if (rc) return rc;
     if (to_ring) e->ring_written += gf;
     e->last_group_frames = gf;
@@ -1963,7 +2001,7 @@ void zfb_destroy(zfb_engine *e) {
     if (e->aux_stream) cudaStreamSynchronize(e->aux_stream);
     DevBuf *bufs[] = {&e->window, &e->winfft, &e->winfft16, &e->wf_sparse, &e->twiddle, &e->twiddle_sub, &e->pow16, &e->mid[0], &e->mid[1], &e->pow, &e->rows_tmp, &e->ema,
                       &e->img_out, &e->img_lut, &e->img_thr, &e->sel_hist, &e->ring, &e->stage_in[0], &e->stage_in[1], &e->big,
-                      &e->trace, &e->trace_rows, &e->peaks};
+                      &e->trace, &e->trace_rows, &e->peaks, &e->persist, &e->persist_thr};
     for (DevBuf *b : bufs) release(*b);
     for (int i = 0; i < 2; ++i) {
         if (e->h_stage[i]) cudaFreeHost(e->h_stage[i]);
@@ -2017,10 +2055,14 @@ int zfb_plan_geometry(int frame_len, int fft_size, int fft_ratio, int out5[5]) {
 static int configure_impl(zfb_engine *e, const zfb_config *cfg);
 static void setup_lanes(zfb_engine *e);
 
-// trace state and the scratch for rows of launch groups without a caller's row buffer
-static int trace_buffers(zfb_engine *e) {
+// state of the trace and persistence sets that are on, and the scratch for rows of launch groups
+// without a caller's row buffer
+static int row_set_buffers(zfb_engine *e) {
     const size_t W = (size_t)e->W;
-    int rc = ensure(e, e->trace, W * (sizeof(double) + 4 * sizeof(float)));
+    int rc = ZFB_OK;
+    if (e->traces_on) rc = ensure(e, e->trace, W * (sizeof(double) + 4 * sizeof(float)));
+    if (rc) return rc;
+    if (e->persist_on) rc = ensure(e, e->persist, (size_t)PS_LEVELS * W * sizeof(float));
     if (rc) return rc;
     return ensure(e, e->trace_rows, (size_t)e->group * W * sizeof(float));     // fp64 passes: px_group <= group
 }
@@ -2291,14 +2333,17 @@ static int configure_impl(zfb_engine *e, const zfb_config *cfg) {
         CK(e, cudaMemcpyAsync(e->px_win.p, cfg->window, (size_t)g.nperseg * sizeof(double), cudaMemcpyHostToDevice, e->stream));
         CK(e, cudaStreamSynchronize(e->stream));       // the caller's window table may go away
     }
-    // the traces keep counting over a change of frame_len, window, EMA, wire format, flip or mode;
-    // anything that changes what a column means or its units starts them afresh
+    // the traces and the persistence set keep counting over a change of frame_len, window, EMA, wire
+    // format, flip or mode; anything that changes what a column means or its units starts them afresh
     const double key[6] = {cfg->fs, (double)N, (double)cfg->fft_ratio, (double)cfg->row_width, cfg->f_demod,
                            (double)cfg->flags};
-    if (memcmp(key, e->trace_key, sizeof key) != 0) e->trace_count = 0;
+    if (memcmp(key, e->trace_key, sizeof key) != 0) {
+        e->trace_count = 0;
+        e->persist_count = 0;
+    }
     memcpy(e->trace_key, key, sizeof key);
-    if (e->traces_on) {
-        rc = trace_buffers(e);
+    if (e->traces_on || e->persist_on) {
+        rc = row_set_buffers(e);
         if (rc) return rc;
     }
     memcpy(e->geom, geom_now, sizeof geom_now);
@@ -2601,12 +2646,13 @@ int zfb_traces_enable(zfb_engine *e, int on) {
         // rows still being folded in read these buffers
         CK(e, cudaStreamSynchronize(e->stream));
         e->traces_on = false;
-        for (DevBuf *b : {&e->trace, &e->trace_rows, &e->peaks}) release(*b);
+        for (DevBuf *b : {&e->trace, &e->peaks}) release(*b);
+        if (!e->persist_on) release(e->trace_rows);
         return ZFB_OK;
     }
     e->traces_on = true;
     if (e->configured) {
-        const int rc = trace_buffers(e);
+        const int rc = row_set_buffers(e);
         if (rc) {
             e->traces_on = false;
             return rc;
@@ -2813,6 +2859,8 @@ static int check_channels(zfb_engine *e, const double *f_demod, int nch) {
         return fail(e, ZFB_EINVAL, "channels: EMA state is per engine; configure with ema_alpha < 0");
     if (nch > 0 && e->traces_on)
         return fail(e, ZFB_EINVAL, "channels: the trace set is per engine; zfb_traces_enable(e, 0) first");
+    if (nch > 0 && e->persist_on)
+        return fail(e, ZFB_EINVAL, "channels: the persistence set is per engine; zfb_persist_enable(e, 0, ...) first");
     if (nch > 0 && e->nstages == 0)
         return fail(e, ZFB_EINVAL, "channels: fft_ratio 1 has no software LO");
     return ZFB_OK;
@@ -3158,11 +3206,7 @@ static int image_params(zfb_engine *e, int height, int scroll, int64_t rows_seen
     p.scroll = scroll;
     p.tick_step = e->ring_W / 10;
     p.newest_slot = (int)((e->ring_written + (int64_t)e->ring_rows - 1) % e->ring_rows);
-    p.thr = nullptr;
-    p.fscale = 1.f;
-    p.foff = 0.f;
-    p.wide_guess = 0;
-    p.lut = nullptr;
+    p.lv = LevelMap{nullptr, 1.f, 0.f, 0, nullptr};
     p.out = nullptr;
     return ZFB_OK;
 }
@@ -3202,6 +3246,53 @@ static void level_thresholds(double minlev, double maxlev, float thr[257]) {
     }
 }
 
+// wf_level's fp32 guess for (minlev, maxlev)
+static void level_guess(double minlev, double maxlev, LevelMap &m) {
+    const double scale = 256.0 / (maxlev - minlev);
+    m.fscale = (float)scale;
+    m.foff = (float)(-minlev * scale);
+    // fp32 guess error <= (256 + 2|foff|) * 2^-23: stays below 1/4 for |foff| < 1e6
+    m.wide_guess = (fabs(minlev * scale) < 1.0e6 && scale < 1.0e30) ? 0 : 1;
+}
+
+// the thresholds of (minlev, maxlev) into `buf` (blocks: the table is built on this stack frame)
+static int put_thresholds(zfb_engine *e, DevBuf &buf, double minlev, double maxlev) {
+    float thr[257];
+    level_thresholds(minlev, maxlev, thr);
+    const int rc = ensure(e, buf, sizeof thr);
+    if (rc) return rc;
+    CK(e, cudaMemcpyAsync(buf.p, thr, sizeof thr, cudaMemcpyHostToDevice, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->counters[3] += sizeof thr;
+    return ZFB_OK;
+}
+
+// level mapping and colour table of an image call (zfb_ring_image, zfb_persist_image): the
+// thresholds go to img_thr, rebuilt only when the level pair changed; the table is uploaded
+static int image_levels(zfb_engine *e, int kind, double minlev, double maxlev, const uint8_t *lut_rgba,
+                        LevelMap &m) {
+    if (kind != ZFB_IMAGE_F32) {
+        if (!e->thr_valid || e->thr_levels[0] != minlev || e->thr_levels[1] != maxlev) {
+            e->thr_valid = false;
+            const int rc = put_thresholds(e, e->img_thr, minlev, maxlev);
+            if (rc) return rc;
+            e->thr_levels[0] = minlev;
+            e->thr_levels[1] = maxlev;
+            e->thr_valid = true;
+        }
+        m.thr = (const float *)e->img_thr.p;
+        level_guess(minlev, maxlev, m);
+    }
+    if (kind == ZFB_IMAGE_RGBA) {
+        const int rc = ensure(e, e->img_lut, 256 * sizeof(unsigned int));
+        if (rc) return rc;
+        CK(e, cudaMemcpyAsync(e->img_lut.p, lut_rgba, 256 * sizeof(unsigned int), cudaMemcpyHostToDevice, e->stream));
+        e->counters[3] += 256 * sizeof(unsigned int);
+        m.lut = (const unsigned int *)e->img_lut.p;
+    }
+    return ZFB_OK;
+}
+
 int zfb_ring_image(zfb_engine *e, int height, int scroll, int64_t rows_seen, int kind, double minlev, double maxlev,
                    const uint8_t *lut_rgba, void *out, int out_on_device) {
     if (!e) return ZFB_EINVAL;
@@ -3219,33 +3310,8 @@ int zfb_ring_image(zfb_engine *e, int height, int scroll, int64_t rows_seen, int
     cudaStream_t st = e->stream;
     const size_t px = (size_t)height * (size_t)e->ring_W;
     const size_t bytes = px * (kind == ZFB_IMAGE_U8 ? 1 : 4);
-    if (kind != ZFB_IMAGE_F32) {
-        if (!e->thr_valid || e->thr_levels[0] != minlev || e->thr_levels[1] != maxlev) {
-            float thr[257];
-            level_thresholds(minlev, maxlev, thr);
-            rc = ensure(e, e->img_thr, sizeof thr);
-            if (rc) return rc;
-            CK(e, cudaMemcpyAsync(e->img_thr.p, thr, sizeof thr, cudaMemcpyHostToDevice, st));
-            CK(e, cudaStreamSynchronize(st));             // thr lives on this stack frame
-            e->counters[3] += sizeof thr;
-            e->thr_levels[0] = minlev;
-            e->thr_levels[1] = maxlev;
-            e->thr_valid = true;
-        }
-        p.thr = (const float *)e->img_thr.p;
-        const double scale = 256.0 / (maxlev - minlev);
-        p.fscale = (float)scale;
-        p.foff = (float)(-minlev * scale);
-        // fp32 guess error <= (256 + 2|foff|) * 2^-23: stays below 1/4 for |foff| < 1e6
-        p.wide_guess = (fabs(minlev * scale) < 1.0e6 && scale < 1.0e30) ? 0 : 1;
-    }
-    if (kind == ZFB_IMAGE_RGBA) {
-        rc = ensure(e, e->img_lut, 256 * sizeof(unsigned int));
-        if (rc) return rc;
-        CK(e, cudaMemcpyAsync(e->img_lut.p, lut_rgba, 256 * sizeof(unsigned int), cudaMemcpyHostToDevice, st));
-        e->counters[3] += 256 * sizeof(unsigned int);
-        p.lut = (const unsigned int *)e->img_lut.p;
-    }
+    rc = image_levels(e, kind, minlev, maxlev, lut_rgba, p.lv);
+    if (rc) return rc;
     if (out_on_device) {
         p.out = out;
     } else {
@@ -3260,6 +3326,99 @@ int zfb_ring_image(zfb_engine *e, int height, int scroll, int64_t rows_seen, int
     if (kind == ZFB_IMAGE_F32) ZFB_LAUNCH(wf_image_kernel<IMG_F32>, grid, dim3(256), 0, st, p);
     else if (kind == ZFB_IMAGE_U8) ZFB_LAUNCH(wf_image_kernel<IMG_U8>, grid, dim3(256), 0, st, p);
     else ZFB_LAUNCH(wf_image_kernel<IMG_RGBA>, grid, dim3(256), 0, st, p);
+    prof_end(e, pr);
+    CK(e, cudaGetLastError());
+    e->counters[2] += 1;
+    if (!out_on_device) {
+        CK(e, cudaMemcpyAsync(out, p.out, bytes, cudaMemcpyDeviceToHost, st));
+        CK(e, cudaStreamSynchronize(st));
+        e->counters[4] += bytes;
+    }
+    return ZFB_OK;
+}
+
+// ---- decaying persistence spectrum (zfb_persist.cuh) -----------------------------------------
+int zfb_persist_enable(zfb_engine *e, int on, double minlev, double maxlev, double decay) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (on) {
+        if (!isfinite(minlev) || !isfinite(maxlev) || !(maxlev > minlev))
+            return fail(e, ZFB_EINVAL, "persistence: levels (%g, %g) must be finite with maxlev > minlev", minlev, maxlev);
+        if (!(decay > 0.0 && decay <= 1.0)) return fail(e, ZFB_EINVAL, "persistence: decay %g outside (0, 1]", decay);
+    }
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    // rows still being folded in read these buffers
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->persist_count = 0;
+    e->persist_on = false;
+    if (!on) {
+        for (DevBuf *b : {&e->persist, &e->persist_thr}) release(*b);
+        if (!e->traces_on) release(e->trace_rows);
+        return ZFB_OK;
+    }
+    int rc = put_thresholds(e, e->persist_thr, minlev, maxlev);
+    if (rc == ZFB_OK) {
+        e->persist_lv = LevelMap{(const float *)e->persist_thr.p, 1.f, 0.f, 0, nullptr};
+        level_guess(minlev, maxlev, e->persist_lv);
+        e->persist_decay = (float)decay;
+        e->persist_on = true;
+        if (e->configured) rc = row_set_buffers(e);
+    }
+    if (rc) {
+        e->persist_on = false;
+        for (DevBuf *b : {&e->persist, &e->persist_thr}) release(*b);
+        if (!e->traces_on) release(e->trace_rows);
+    }
+    return rc;
+}
+
+int zfb_persist_reset(zfb_engine *e) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    e->persist_count = 0;    // launch order is stream order: the next update starts afresh
+    return ZFB_OK;
+}
+
+int64_t zfb_persist_count(const zfb_engine *e) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    return e->persist_on ? e->persist_count : 0;
+}
+
+int zfb_persist_image(zfb_engine *e, int kind, double imin, double imax, const uint8_t *lut_rgba, void *out,
+                      int out_on_device) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    join_pending_work(e);
+    if (!out) return fail(e, ZFB_EINVAL, "persistence image: out is NULL");
+    if (kind != ZFB_IMAGE_F32 && kind != ZFB_IMAGE_U8 && kind != ZFB_IMAGE_RGBA)
+        return fail(e, ZFB_EINVAL, "persistence image: unknown kind %d", kind);
+    if (kind != ZFB_IMAGE_F32 && !(imax > imin)) return fail(e, ZFB_EINVAL, "persistence image: imax must exceed imin");
+    if (kind == ZFB_IMAGE_RGBA && !lut_rgba) return fail(e, ZFB_EINVAL, "persistence image: RGBA needs a 256-entry table");
+    if (!e->persist_on) return fail(e, ZFB_ESTATE, "persistence set is off (zfb_persist_enable)");
+    if (!e->configured || e->persist_count < 1) return fail(e, ZFB_ESTATE, "the persistence set holds no row yet");
+    CK(e, cudaSetDevice(e->device));
+    cudaStream_t st = e->stream;
+    PersistImageParams p{};
+    p.state = (const float *)e->persist.p;
+    p.W = e->W;
+    int rc = image_levels(e, kind, imin, imax, lut_rgba, p.lv);
+    if (rc) return rc;
+    const size_t bytes = (size_t)PS_LEVELS * (size_t)e->W * (kind == ZFB_IMAGE_U8 ? 1 : 4);
+    if (out_on_device) {
+        p.out = out;
+    } else {
+        if (e->img_out.cap < bytes) CK(e, cudaStreamSynchronize(st));
+        rc = ensure(e, e->img_out, bytes);
+        if (rc) return rc;
+        p.out = e->img_out.p;
+    }
+    const dim3 grid((unsigned)((e->W + PI_NT * PI_U - 1) / (PI_NT * PI_U)), (unsigned)PS_LEVELS);
+    const int pr = prof_begin(e, 19);
+    if (kind == ZFB_IMAGE_F32) ZFB_LAUNCH(persist_image_kernel<IMG_F32>, grid, dim3(PI_NT), 0, st, p);
+    else if (kind == ZFB_IMAGE_U8) ZFB_LAUNCH(persist_image_kernel<IMG_U8>, grid, dim3(PI_NT), 0, st, p);
+    else ZFB_LAUNCH(persist_image_kernel<IMG_RGBA>, grid, dim3(PI_NT), 0, st, p);
     prof_end(e, pr);
     CK(e, cudaGetLastError());
     e->counters[2] += 1;

@@ -20,6 +20,18 @@ namespace zfb {
 
 constexpr int IMG_F32 = 0, IMG_U8 = 1, IMG_RGBA = 2;
 
+// level mapping: index = clip(trunc((double(v) - minlev) * 256 / (maxlev - minlev)), 0, 255).
+// thr[k], k = 1..255 = the smallest float whose index is >= k (found on the host with
+// exactly that double arithmetic): the device makes an fp32 guess v * fscale + foff
+// (within 1 of the index for any sane level pair) and settles it by comparing with the
+// neighbouring thresholds, bit-exact with the double formula, no FP64 or F2I instructions.
+struct LevelMap {
+    const float *thr;         // [257]
+    float  fscale, foff;
+    int    wide_guess;        // the fp32 guess may be off by more than 1 (degenerate level pair)
+    const unsigned int *lut;  // 256 packed RGBA entries (IMG_RGBA)
+};
+
 struct ImageParams {
     const float *ring;        // [ring_rows][W] finished rows
     int    ring_rows;
@@ -30,15 +42,7 @@ struct ImageParams {
     int    scroll;            // AppState.scroll: > 0 newest row near the bottom, else at the top
     int    tick_step;         // W // 10
     int    newest_slot;       // ring slot of the newest row: (written - 1) mod ring_rows
-    // level mapping: index = clip(trunc((double(v) - minlev) * 256 / (maxlev - minlev)), 0, 255).
-    // thr[k], k = 1..255 = the smallest float whose index is >= k (found on the host with
-    // exactly that double arithmetic): the device makes an fp32 guess v * fscale + foff
-    // (within 1 of the index for any sane level pair) and settles it by comparing with the
-    // neighbouring thresholds, bit-exact with the double formula, no FP64 or F2I instructions.
-    const float *thr;         // [257]
-    float  fscale, foff;
-    int    wide_guess;        // the fp32 guess may be off by more than 1 (degenerate level pair)
-    const unsigned int *lut;  // 256 packed RGBA entries (IMG_RGBA)
+    LevelMap lv;              // (minlev, maxlev) -> colour index, and the RGBA table
     void  *out;
 };
 
@@ -103,12 +107,19 @@ __device__ __forceinline__ void wf_fix4(const ImageParams &p, bool from_ring, bo
     }
 }
 
-// thr2[g] = (thr[g], thr[g + 1]) with thr[0] = -inf and thr[256] = NaN (never reached)
-__device__ __forceinline__ unsigned int wf_level(const ImageParams &p, const float2 *thr2, float v) {
-    float x = fmaf(v, p.fscale, p.foff);
+// the shared-memory table wf_level reads: thr2[g] = (thr[g], thr[g + 1]) with
+// thr[0] = -inf and thr[256] = NaN (never reached)
+__device__ __forceinline__ void wf_load_levels(float2 *thr2, const float *thr) {
+    for (int i = threadIdx.x; i < 256; i += blockDim.x)
+        thr2[i] = make_float2(thr[i], i < 255 ? thr[i + 1] : __uint_as_float(0x7FC00000u));
+}
+
+__device__ __forceinline__ unsigned int wf_level(const float2 *thr2, float fscale, float foff, int wide_guess,
+                                                 float v) {
+    float x = fmaf(v, fscale, foff);
     x = fminf(fmaxf(x, 0.f), 255.f);                 // NaN -> 0
     int g = (int)(__float_as_uint(x + 8388608.0f) - 0x4B000000u);    // round to nearest, 0..255
-    if (!p.wide_guess) {
+    if (!wide_guess) {
         // |guess - index| <= 1 (the host checked the level pair): one LDS.64, two compares
         const float2 t = thr2[g];
         g += (v >= t.y) ? 1 : 0;
@@ -128,12 +139,12 @@ __global__ void __launch_bounds__(IMG_NT) wf_image_kernel(const ImageParams p) {
     __shared__ float2 thr[256];
     __shared__ unsigned int lut[256];
     if (KIND != IMG_F32) {
-        for (int i = threadIdx.x; i < 256; i += IMG_NT)
-            thr[i] = make_float2(p.thr[i], i < 255 ? p.thr[i + 1] : __uint_as_float(0x7FC00000u));
+        wf_load_levels(thr, p.lv.thr);
         if (KIND == IMG_RGBA)
-            for (int i = threadIdx.x; i < 256; i += IMG_NT) lut[i] = p.lut[i];
+            for (int i = threadIdx.x; i < 256; i += IMG_NT) lut[i] = p.lv.lut[i];
         __syncthreads();
     }
+    const LevelMap &m = p.lv;
     const int y = blockIdx.y;
     const float *row = wf_row(p, y);
     const bool tick_row = wf_tick_row(p, y);
@@ -158,14 +169,14 @@ __global__ void __launch_bounds__(IMG_NT) wf_image_kernel(const ImageParams p) {
             } else if (KIND == IMG_U8) {
                 unsigned int pk = 0;
 #pragma unroll
-                for (int e = 0; e < 4; ++e) pk |= wf_level(p, thr, q[e]) << (8 * e);
+                for (int e = 0; e < 4; ++e) pk |= wf_level(thr, m.fscale, m.foff, m.wide_guess, q[e]) << (8 * e);
                 *(unsigned int *)((unsigned char *)p.out + at) = pk;
             } else {
                 uint4 c;
-                c.x = lut[wf_level(p, thr, q[0])];
-                c.y = lut[wf_level(p, thr, q[1])];
-                c.z = lut[wf_level(p, thr, q[2])];
-                c.w = lut[wf_level(p, thr, q[3])];
+                c.x = lut[wf_level(thr, m.fscale, m.foff, m.wide_guess, q[0])];
+                c.y = lut[wf_level(thr, m.fscale, m.foff, m.wide_guess, q[1])];
+                c.z = lut[wf_level(thr, m.fscale, m.foff, m.wide_guess, q[2])];
+                c.w = lut[wf_level(thr, m.fscale, m.foff, m.wide_guess, q[3])];
                 *(uint4 *)((unsigned int *)p.out + at) = c;
             }
         }
@@ -175,8 +186,8 @@ __global__ void __launch_bounds__(IMG_NT) wf_image_kernel(const ImageParams p) {
             const float v = wf_fix(p, row != nullptr, tick_row, x, row ? row[x] : 0.f);
             const size_t at = (size_t)y * p.W + x;
             if (KIND == IMG_F32) ((float *)p.out)[at] = v;
-            else if (KIND == IMG_U8) ((unsigned char *)p.out)[at] = (unsigned char)wf_level(p, thr, v);
-            else ((unsigned int *)p.out)[at] = lut[wf_level(p, thr, v)];
+            else if (KIND == IMG_U8) ((unsigned char *)p.out)[at] = (unsigned char)wf_level(thr, m.fscale, m.foff, m.wide_guess, v);
+            else ((unsigned int *)p.out)[at] = lut[wf_level(thr, m.fscale, m.foff, m.wide_guess, v)];
         }
     }
 }

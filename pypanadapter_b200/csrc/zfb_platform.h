@@ -9,6 +9,18 @@
     ::cuemu::launch(kernel, grid, block, smem, __VA_ARGS__)
 #define ZFB_DYN_SMEM(name) unsigned char *name = ::cuemu::dyn_smem()
 #define ZFB_BUILD_KIND "emulated"
+// The device's separately rounded fp32 multiply and add (zfb_persist.cuh relies on them to
+// match numpy's float32 P * decay + hit).  They must not be plain a * b and a + b: under
+// g++ -O2 -mfma those contract into one vfmadd, so each result goes through a volatile
+// (one vmulss, then one vaddss).
+static inline float __fmul_rn(float a, float b) {
+    volatile float p = a * b;
+    return p;
+}
+static inline float __fadd_rn(float a, float b) {
+    volatile float s = a + b;
+    return s;
+}
 #else
 #include <cuda_runtime.h>
 #define ZFB_LAUNCH(kernel, grid, block, smem, stream, ...) \

@@ -445,6 +445,54 @@ class ZoomPSD:
         self._check(self._lib.zfb_ring_push_rows(self._h, C.c_void_p(r.ctypes.data), r.shape[0]),
                     "zfb_ring_push_rows")
 
+    # -- decaying persistence spectrum (DESIGN 3.9) -----------------------------
+    def persistence_enable(self, on: bool = True, levels=(-220.0, -120.0), decay: float = 1.0):
+        """Keep a persistence set on the device over every row the engine computes from now
+        on (starts it empty): per column, 256 level bins of ``levels`` = (minlev, maxlev) in
+        the rows' units, binned as the waterfall colours a pixel; per row every bin decays
+        by ``decay`` (0 < decay <= 1; 1 = hit counts) and the row's own bin gains 1.
+        ``False`` drops it."""
+        lo, hi = (float(levels[0]), float(levels[1])) if on else (0.0, 1.0)
+        rc = self._lib.zfb_persist_enable(self._h, 1 if on else 0, lo, hi, float(decay) if on else 1.0)
+        if rc != _lib.ZFB_EINVAL:                  # EINVAL leaves the set as it was
+            self._persist_levels = (lo, hi) if on and rc == 0 else None
+        self._check(rc, "zfb_persist_enable")
+
+    def persistence_reset(self):
+        self._check(self._lib.zfb_persist_reset(self._h), "zfb_persist_reset")
+
+    @property
+    def persistence_count(self) -> int:
+        """rows in the persistence set since it last started empty"""
+        return int(self._lib.zfb_persist_count(self._h))
+
+    def persistence_levels(self) -> np.ndarray:
+        """The lower edge of each of the 256 level bins in row units (float64), image row
+        ``255 - k`` being bin ``k``: minlev + k (maxlev - minlev) / 256."""
+        lv = getattr(self, "_persist_levels", None)
+        if lv is None:
+            raise ZoomFFTError(_lib.ZFB_ESTATE, "persistence_levels: the persistence set is off")
+        return lv[0] + np.arange(_lib.ZFB_PERSIST_LEVELS, dtype=np.float64) * ((lv[1] - lv[0]) / 256.0)
+
+    def persistence_image(self, kind: str = "f32", levels=None, lut=None) -> np.ndarray:
+        """The (256, row_width) image of the set, high levels at the top: ``kind`` 'f32' =
+        the intensities, 'u8' = their colour indices for ``levels`` (imin, imax), 'rgba' =
+        ``lut[index]`` (lut: (256, 4) uint8), (256, row_width, 4)."""
+        code, lo, hi, lut = _image_args(kind, levels, lut)
+        lut_p = None if lut is None else C.c_void_p(lut.ctypes.data)
+        W = self.row_width
+        out = np.empty((256, W) if kind != "rgba" else (256, W, 4), dtype=np.float32 if kind == "f32" else np.uint8)
+        self._check(self._lib.zfb_persist_image(self._h, code, lo, hi, lut_p, C.c_void_p(out.ctypes.data), 0),
+                    "zfb_persist_image")
+        return out
+
+    def persistence_image_device(self, d_out_ptr: int, kind: str = "u8", *, levels, lut=None):
+        """Same, into a caller-owned device buffer (asynchronous on the engine's stream)."""
+        code, lo, hi, lut = _image_args(kind, levels, lut)
+        lut_p = None if lut is None else C.c_void_p(lut.ctypes.data)
+        self._check(self._lib.zfb_persist_image(self._h, code, lo, hi, lut_p, C.c_void_p(d_out_ptr), 1),
+                    "zfb_persist_image")
+
     # -- waterfall image / autolevel on the device (S:1625-1676) ---------------
     def ring_image(self, height: int, scroll: int, rows_seen: int, kind: str = "f32", *,
                    levels=None, lut=None) -> np.ndarray:
@@ -536,6 +584,22 @@ def _trace_kind(kind: str) -> int:
     if kind not in _TRACE_KINDS:
         raise ValueError("trace kind must be one of %s, got %r" % (", ".join(map(repr, _TRACE_KINDS)), kind))
     return _TRACE_KINDS[kind]
+
+
+def _image_args(kind: str, levels, lut):
+    """(ZFB_IMAGE_* code, lo, hi, contiguous (256, 4) uint8 table or None) of a persistence image call"""
+    codes = {"f32": _lib.ZFB_IMAGE_F32, "u8": _lib.ZFB_IMAGE_U8, "rgba": _lib.ZFB_IMAGE_RGBA}
+    if kind not in codes:
+        raise ValueError("kind must be one of %s, got %r" % (", ".join(map(repr, codes)), kind))
+    if kind != "f32" and levels is None:
+        raise ValueError("kind %r needs levels=(imin, imax)" % kind)
+    lo, hi = (0.0, 1.0) if levels is None else (float(levels[0]), float(levels[1]))
+    if kind != "rgba":
+        return codes[kind], lo, hi, None
+    lut = np.ascontiguousarray(lut, dtype=np.uint8)
+    if lut.shape != (256, 4):
+        raise ValueError("lut must be (256, 4) uint8")
+    return codes[kind], lo, hi, lut
 
 
 def _prof_name(c: int) -> str:
