@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ZFB_ABI_VERSION 4
+#define ZFB_ABI_VERSION 5
 
 /* status codes */
 #define ZFB_OK            0
@@ -366,6 +366,81 @@ int64_t zfb_persist_count(const zfb_engine *e);
 int  zfb_persist_image(zfb_engine *e, int kind, double imin, double imax,
                        const uint8_t *lut_rgba, void *out, int out_on_device);
 
+/* ---- frequency-mask trigger (DESIGN 3.10) -----------------------------------
+ * Max-hold shows THAT a burst crossed a line; a real-time spectrum analyser's
+ * frequency-mask trigger says which row did it, when, and keeps its samples.
+ * The mask is checked on the device against the same rows as the trace set:
+ * every row of zfb_process_device, zfb_process_host and zfb_samples_process on
+ * every path (fp32 and fp64 rows, pipelined batches, one-sided, four-step),
+ * with EMA applied as the caller gets the rows, also rows that never reach the
+ * ring (ring_append = 0); not rows of zfb_ring_push_rows.
+ *   Mask: two optional limit lines of row_width float32 values each, in the
+ *   rows' own units (dB20, or linear power with ZFB_FLAG_LINEAR).  Column c of
+ *   a row v violates when v[c] > upper[c] or v[c] < lower[c].  A NaN limit
+ *   turns that side off at that column; +-inf limits are allowed.  A NaN row
+ *   value never violates; a -inf row value (a DC-only frame) violates any
+ *   finite lower limit.  Where both sides fail (only possible with infinite
+ *   limits) the larger excess counts, the upper side on a tie.
+ *   Trigger: a row with at least min_cols (1..row_width) violating columns.
+ *   Event record: one zfb_mask_event per triggering row (below).  excess is the
+ *   fp32 difference (value - upper) or (lower - value) at worst_col: > 0, +inf
+ *   for -inf below a finite lower limit.  worst_col has the largest excess,
+ *   ties to the lower column.
+ *   Log: the first max_events (1..2^20) events, in frame order; later events
+ *   are counted but not stored.  The event counter lives on the device (the
+ *   host never waits to learn how many rows triggered); the row counter on the
+ *   host, like zfb_persist_count.
+ *   Capture: event k gets capture slot k while k < capture_slots (0..max_events),
+ *   later events capture = -1.  A slot holds the first min(frame_len,
+ *   capture_samples) samples of the triggering frame as the caller handed them
+ *   over: wire format before flip (uint8 or int16 I,Q pairs as they came; the
+ *   caller's int16 buffer even where the CS16 path widens it).  Slots are
+ *   capture_samples x 8 bytes, so a later change of dtype or frame_len still
+ *   fits.  The copy runs on the device, in stream order, behind the check.  On
+ *   pipelined batches it reads the caller's d_in, which the caller keeps alive
+ *   until zfb_join anyway.
+ * The log, both counters and every capture are bit-identical however the same
+ * frames are cut into calls, groups, host or device paths or pipelined batches.
+ * Off by default: then nothing is allocated or launched.  With the mask on a
+ * launch group costs 2 more kernels, 3 with capture slots.
+ * zfb_mask_enable(on = 1) needs a configured engine (ZFB_ESTATE otherwise);
+ * it validates, uploads the lines and starts the log empty.  ZFB_EINVAL when
+ * both lines are NULL, lower[c] > upper[c] at a column where both are finite,
+ * or min_cols, max_events, capture_slots or capture_samples (>= 1 when
+ * capture_slots > 0) is out of range; ZFB_ENOMEM leaves the mask off.  on = 0
+ * turns it off and frees it.  zfb_mask_reset empties the log and both counters
+ * and keeps the lines.  A zfb_configure that changes fs, fft_size, fft_ratio,
+ * row_width, f_demod or flags turns the mask off (its lines no longer mean the
+ * same columns); a change of frame_len, window, ema_alpha, dtype, flip or mode
+ * keeps it armed and counting.  While it is on, zfb_process_channels_* return
+ * ZFB_EINVAL.  Every read returns ZFB_ESTATE while the mask is off. */
+typedef struct zfb_mask_event {
+    int64_t row;              /* 0-based index of the row among the rows checked since the log last started empty */
+    int32_t ncols;            /* violating columns (>= min_cols) */
+    int32_t first_col, last_col;
+    int32_t worst_col;        /* largest excess; ties to the lower column */
+    float   value;            /* row value at worst_col */
+    float   excess;           /* fp32 (value - upper) or (lower - value) at worst_col; > 0, +inf for -inf below a finite lower */
+    int32_t above;            /* 1: worst_col passed its upper limit, 0: its lower one */
+    int32_t capture;          /* capture slot, or -1 */
+    int32_t capture_samples;  /* samples in that slot, 0 without one */
+    int32_t dtype;            /* ZFB_DTYPE_* of the captured samples */
+} zfb_mask_event;
+int  zfb_mask_enable(zfb_engine *e, int on, const float *upper, const float *lower, int min_cols,
+                     int max_events, int capture_slots, int capture_samples);
+int  zfb_mask_reset(zfb_engine *e);
+/* out[0] = rows checked, out[1] = events detected (stored or not); joins pending work, blocks */
+int  zfb_mask_counts(zfb_engine *e, int64_t out2[2]);
+/* stored events [first, first + max) to out; *n = how many; joins, blocks.
+ * ZFB_EINVAL for first < 0, max < 0 or a NULL pointer. */
+int  zfb_mask_events(zfb_engine *e, int first, int max, zfb_mask_event *out, int *n);
+/* the samples of capture slot `slot` (event.capture_samples x sample size bytes:
+ * 8 complex64, 2 uint8, 4 int16); host out blocks, device out is asynchronous
+ * on the engine's stream (the slot's event is read first, which blocks).
+ * ZFB_EINVAL for a slot outside [0, capture_slots) or out == NULL; ZFB_ESTATE
+ * for a slot not filled yet. */
+int  zfb_mask_capture(zfb_engine *e, int slot, void *out, int out_on_device);
+
 /* ---- taper design and preview on the device (SURVEY 8f.4) ----------------
  * The taper dialog's live preview (FFTTaperingControl.ShowCurve, S:1354-1379):
  * zfb_taper_design replaces scipy.signal.get_window(AppState.fft_tapering, 51)
@@ -424,7 +499,8 @@ int  zfb_get_counters(const zfb_engine *e, uint64_t out5[5]);
 /* kernel classes: 0..15 = decimate-by-2 stage s (replaces scipy.signal.
  * decimate call s of the loop at S:2097-2098), 16 = Welch kernel / four-step
  * column pass, 17 = four-step row pass (both: scipy.signal.welch, S:2111),
- * 18 = row finalisation (S:2114-2119 + EMA, trace and persistence updates),
+ * 18 = row finalisation (S:2114-2119 + EMA, trace and persistence updates,
+ * frequency-mask check, log and capture),
  * 19 = waterfall image (S:1625-1664) and persistence image, 20 = autolevel
  * selection sweep (S:1676). */
 #define ZFB_PROF_CLASSES 21

@@ -32,7 +32,7 @@ ZFB_FLAG_NO_LO = 1
 ZFB_FLAG_LINEAR = 2
 ZFB_FLAG_ONESIDED = 4
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 PROF_CLASSES = 21
 ZFB_IMAGE_F32 = 0
 ZFB_IMAGE_U8 = 1
@@ -72,6 +72,23 @@ class ZfbFastPlan(C.Structure):
         ("comp_half", C.c_int32),
         ("comp_taps", C.POINTER(C.c_double)),
         ("strip", C.c_int32),
+    ]
+
+
+class ZfbMaskEvent(C.Structure):
+    """struct zfb_mask_event (include/zoomfft_b200.h), 48 bytes."""
+    _fields_ = [
+        ("row", C.c_int64),
+        ("ncols", C.c_int32),
+        ("first_col", C.c_int32),
+        ("last_col", C.c_int32),
+        ("worst_col", C.c_int32),
+        ("value", C.c_float),
+        ("excess", C.c_float),
+        ("above", C.c_int32),
+        ("capture", C.c_int32),
+        ("capture_samples", C.c_int32),
+        ("dtype", C.c_int32),
     ]
 
 
@@ -118,6 +135,11 @@ SYMBOLS = {
     "zfb_persist_reset": (C.c_int, [_P]),
     "zfb_persist_count": (C.c_int64, [_P]),
     "zfb_persist_image": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, _P, _P, C.c_int]),
+    "zfb_mask_enable": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "zfb_mask_reset": (C.c_int, [_P]),
+    "zfb_mask_counts": (C.c_int, [_P, C.POINTER(C.c_int64)]),
+    "zfb_mask_events": (C.c_int, [_P, C.c_int, C.c_int, _P, C.POINTER(C.c_int)]),
+    "zfb_mask_capture": (C.c_int, [_P, C.c_int, _P, C.c_int]),
     "zfb_ring_quantiles": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, C.POINTER(C.c_double), C.c_int,
                                      C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "zfb_taper_design": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(C.c_double)]),

@@ -31,6 +31,7 @@
 #include "zfb_precise.cuh"
 #include "zfb_trace.cuh"
 #include "zfb_persist.cuh"
+#include "zfb_mask.cuh"
 
 using namespace zfb;
 
@@ -165,6 +166,15 @@ struct zfb_engine {
     LevelMap persist_lv{};             // row value -> level bin for the set's (minlev, maxlev)
     DevBuf persist;                    // [256][W] intensities, level-major
     DevBuf persist_thr;                // the 257 level thresholds of persist_lv, built at enable
+    // frequency-mask trigger (zfb_mask_enable; zfb_mask.cuh): nothing is allocated or launched while it is off
+    bool mask_on = false;
+    int64_t mask_rows = 0;             // rows checked (host side; launch order = stream order)
+    int mask_min_cols = 1, mask_max_events = 0, mask_slots = 0, mask_cap_samples = 0;
+    DevBuf mask_lines;                 // [2][W]: upper, lower (NaN: that side off)
+    DevBuf mask_state;                 // event counter (u64), then the group's capture count (int)
+    DevBuf mask_log;                   // [max_events] zfb_mask_event
+    DevBuf mask_caps;                  // [capture_slots][capture_samples * 8] bytes
+    DevBuf mask_work;                  // [group][chunks] MaskPart, then [group] MaskCap
 
     // ZFB_MODE_FAST
     struct FastPlan {
@@ -1235,10 +1245,13 @@ cudaError_t run_decimation_fast(zfb_engine *e, const void *d_in, int gf, int *ou
     return cudaSuccess;
 }
 
-// traces or persistence on: the rows of a launch group go to the caller's buffer or, without one,
-// to this scratch
+// a set that reads every row (traces, persistence, frequency mask) is on
+bool row_sets_on(const zfb_engine *e) { return e->traces_on || e->persist_on || e->mask_on; }
+
+// traces, persistence or mask on: the rows of a launch group go to the caller's buffer or, without
+// one, to this scratch
 float *trace_rows_or(zfb_engine *e, float *d_rows) {
-    return (d_rows || !(e->traces_on || e->persist_on) || e->cur_nch > 0) ? d_rows : (float *)e->trace_rows.p;
+    return (d_rows || !row_sets_on(e) || e->cur_nch > 0) ? d_rows : (float *)e->trace_rows.p;
 }
 
 // fold `nf` finished rows into the trace set, on the stream that finished them (after them)
@@ -1285,15 +1298,80 @@ int persist_update(zfb_engine *e, const float *rows, int nf, cudaStream_t st) {
     return ZFB_OK;
 }
 
+// check `nf` finished rows against the frequency mask, log their events and capture the frames
+// that get a slot (`in`: the group's input as the caller handed it over, frames `fbytes` apart), on
+// the stream that finished them (after them)
+int mask_update(zfb_engine *e, const float *rows, const void *in, size_t fbytes, int nf, cudaStream_t st) {
+    if (!e->mask_on || e->cur_nch > 0 || nf < 1) return ZFB_OK;
+    const int W = e->W;
+    const int nchunks = (W + MK_CHUNK - 1) / MK_CHUNK;
+    MaskPart *part = (MaskPart *)e->mask_work.p;
+    MaskCap *caps = (MaskCap *)(part + (size_t)e->group * nchunks);
+    unsigned long long *counter = (unsigned long long *)e->mask_state.p;
+    int *ncap = (int *)(counter + 1);
+    MaskCheckParams cp{};
+    cp.rows = rows;
+    cp.lines = (const float *)e->mask_lines.p;
+    cp.nframes = nf;
+    cp.W = W;
+    cp.nchunks = nchunks;
+    cp.part = part;
+    // about 8 CTAs per SM: wide rows split into chunks, narrow rows one CTA each
+    const int gy = std::max(1, std::min(nf, 8 * e->sm_count / nchunks));
+    MaskLogParams lp{};
+    lp.part = part;
+    lp.rows = rows;
+    lp.nframes = nf;
+    lp.nchunks = nchunks;
+    lp.W = W;
+    lp.row0 = (long long)e->mask_rows;
+    lp.min_cols = e->mask_min_cols;
+    lp.max_events = e->mask_max_events;
+    lp.capture_slots = e->mask_slots;
+    lp.capture_samples = e->mask_cap_samples;
+    lp.frame_len = e->cfg.frame_len;
+    lp.dtype = e->cfg.dtype;
+    lp.counter = counter;
+    lp.events = (zfb_mask_event *)e->mask_log.p;
+    lp.cap_list = caps;
+    lp.ncap = ncap;
+    const int pr = prof_begin(e, 18, st);
+    ZFB_LAUNCH(mask_check_kernel, dim3((unsigned)nchunks, (unsigned)gy), dim3(MK_NT), 0, st, cp);
+    ZFB_LAUNCH(mask_log_kernel, dim3(1), dim3(ML_NT), 0, st, lp);
+    e->counters[2] += 2;
+    if (e->mask_slots > 0) {
+        MaskCopyParams mp{};
+        mp.src = (const unsigned char *)in;
+        mp.src_stride = fbytes;
+        mp.dst = (unsigned char *)e->mask_caps.p;
+        mp.dst_stride = (size_t)e->mask_cap_samples * 8;
+        mp.nbytes = (long long)std::min(e->cfg.frame_len, e->mask_cap_samples) * (long long)sample_bytes(e->cfg);
+        mp.list = caps;
+        mp.nlist = ncap;
+        const long long tiles = (mp.nbytes + MC_TILE - 1) / MC_TILE + 1;     // + 1: a destination word may straddle
+        const unsigned gx = (unsigned)std::min<long long>(tiles, 16);
+        const unsigned ny = (unsigned)std::min(nf, e->mask_slots);       // the group's captures fit here
+        ZFB_LAUNCH(mask_capture_kernel, dim3(gx, ny), dim3(MC_NT), 0, st, mp);
+        e->counters[2] += 1;
+    }
+    prof_end(e, pr, st);
+    e->mask_rows += nf;
+    CK(e, cudaGetLastError());
+    return ZFB_OK;
+}
+
 // every row the engine finishes (not the rows of channel-batched launches) feeds the trace and
-// persistence sets that are on
-int rows_finished(zfb_engine *e, const float *rows, int nf, cudaStream_t st) {
-    const int rc = trace_update(e, rows, nf, st);
-    return rc ? rc : persist_update(e, rows, nf, st);
+// persistence sets and the frequency mask that are on; `in` is the group's input
+int rows_finished(zfb_engine *e, const float *rows, const void *in, int nf, cudaStream_t st) {
+    int rc = trace_update(e, rows, nf, st);
+    if (rc == ZFB_OK) rc = persist_update(e, rows, nf, st);
+    if (rc == ZFB_OK) rc = mask_update(e, rows, in, (size_t)e->cfg.frame_len * sample_bytes(e->cfg), nf, st);
+    return rc;
 }
 
 // fp64 path (zfb_precise.cuh): rows of few Welch segments, `gf` frames resident on the device
-int run_group_precise(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
+// (`raw_in`: the same frames as the caller handed them over, before any widening of int16 IQ)
+int run_group_precise(zfb_engine *e, const void *d_in, const void *raw_in, int gf, float *d_rows) {
     const zfb_config &c = e->cfg;
     cudaStream_t st = e->stream;
     const int k = e->nstages;
@@ -1389,7 +1467,8 @@ int run_group_precise(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
         e->counters[2] += 2;
         if (rp.alpha >= 0.0) e->ema_have = true;
         if (to_ring) e->ring_written += nf;
-        const int rc = rows_finished(e, rp.rows, nf, st);
+        const int rc = rows_finished(e, rp.rows, (const char *)raw_in + (size_t)g0 * c.frame_len * sample_bytes(c),
+                                     nf, st);
         if (rc) return rc;
     }
     CK(e, cudaGetLastError());
@@ -1407,7 +1486,7 @@ bool fir_cs16_fused(const zfb_engine *e) {
 }
 
 // one group of frames, all resident on the device, through the whole chain
-int finish_rows(zfb_engine *e, zfb_engine *from, int gf, int nsplit, float *d_rows, cudaStream_t st);
+int finish_rows(zfb_engine *e, zfb_engine *from, const void *d_in, int gf, int nsplit, float *d_rows, cudaStream_t st);
 
 // a launch group up to the Welch power sums (e->pow, nsplit partial sums per row); finish_rows makes
 // rows of them.  *done: the fp64 path (run_group_precise) has written the rows itself
@@ -1415,6 +1494,7 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
     const zfb_config &c = e->cfg;
     cudaStream_t st = e->stream;
     *done = false;
+    const void *raw_in = d_in;
     const void *d_in_cs16 = nullptr;
     if (c.dtype == ZFB_DTYPE_CS16 && fir_cs16_fused(e)) {
         // the FIR interior converts on load (zfb_firchain.cuh, KIND_CS16_RAW); only the chunk ends the
@@ -1449,7 +1529,7 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
     }
     if (e->precise_active) {
         *done = true;
-        return run_group_precise(e, d_in, gf, d_rows);
+        return run_group_precise(e, d_in, raw_in, gf, d_rows);
     }
     const void *src = d_in;
     long long src_stride = c.frame_len;
@@ -1644,8 +1724,9 @@ int run_group_front(zfb_engine *e, const void *d_in, int gf, float *d_rows, int 
 }
 
 // rows of one launch group from the power sums in from->pow (this engine's, or a lane's): scale,
-// EMA in frame order, dB20, ring -- on stream st (e->stream, or fin_stream for pipelined batches)
-int finish_rows(zfb_engine *e, zfb_engine *from, int gf, int nsplit, float *d_rows, cudaStream_t st) {
+// EMA in frame order, dB20, ring -- on stream st (e->stream, or fin_stream for pipelined batches);
+// d_in: the group's input, for the frequency mask's captures
+int finish_rows(zfb_engine *e, zfb_engine *from, const void *d_in, int gf, int nsplit, float *d_rows, cudaStream_t st) {
     const zfb_config &c = e->cfg;
     FinalizeParams f{};
     f.pow_io = (float *)from->pow.p;
@@ -1681,7 +1762,7 @@ int finish_rows(zfb_engine *e, zfb_engine *from, int gf, int nsplit, float *d_ro
     e->counters[2] += 1;
     prof_end(e, prf, st);
     CK(e, cudaGetLastError());
-    const int rc = rows_finished(e, f.rows, gf, st);
+    const int rc = rows_finished(e, f.rows, d_in, gf, st);
     if (rc) return rc;
     if (to_ring) e->ring_written += gf;
     e->last_group_frames = gf;
@@ -1696,7 +1777,7 @@ int run_group(zfb_engine *e, const void *d_in, int gf, float *d_rows) {
     bool done = false;
     const int rc = run_group_front(e, d_in, gf, d_rows, &nsplit, &done);
     if (rc != ZFB_OK || done) return rc;
-    return finish_rows(e, e, gf, nsplit, d_rows, e->stream);
+    return finish_rows(e, e, d_in, gf, nsplit, d_rows, e->stream);
 }
 
 // late mix of the first register-blocked chain (zfb_firchain.cuh): allowed when the LO
@@ -2001,7 +2082,8 @@ void zfb_destroy(zfb_engine *e) {
     if (e->aux_stream) cudaStreamSynchronize(e->aux_stream);
     DevBuf *bufs[] = {&e->window, &e->winfft, &e->winfft16, &e->wf_sparse, &e->twiddle, &e->twiddle_sub, &e->pow16, &e->mid[0], &e->mid[1], &e->pow, &e->rows_tmp, &e->ema,
                       &e->img_out, &e->img_lut, &e->img_thr, &e->sel_hist, &e->ring, &e->stage_in[0], &e->stage_in[1], &e->big,
-                      &e->trace, &e->trace_rows, &e->peaks, &e->persist, &e->persist_thr};
+                      &e->trace, &e->trace_rows, &e->peaks, &e->persist, &e->persist_thr,
+                      &e->mask_lines, &e->mask_state, &e->mask_log, &e->mask_caps, &e->mask_work};
     for (DevBuf *b : bufs) release(*b);
     for (int i = 0; i < 2; ++i) {
         if (e->h_stage[i]) cudaFreeHost(e->h_stage[i]);
@@ -2055,14 +2137,25 @@ int zfb_plan_geometry(int frame_len, int fft_size, int fft_ratio, int out5[5]) {
 static int configure_impl(zfb_engine *e, const zfb_config *cfg);
 static void setup_lanes(zfb_engine *e);
 
-// state of the trace and persistence sets that are on, and the scratch for rows of launch groups
-// without a caller's row buffer
+// the frequency mask off and freed (no work that reads its buffers may be pending)
+static void mask_off(zfb_engine *e) {
+    e->mask_on = false;
+    e->mask_rows = 0;
+    for (DevBuf *b : {&e->mask_lines, &e->mask_state, &e->mask_log, &e->mask_caps, &e->mask_work}) release(*b);
+    if (!row_sets_on(e)) release(e->trace_rows);
+}
+
+// state of the trace and persistence sets that are on, the frequency mask's per-group scratch, and
+// the scratch for rows of launch groups without a caller's row buffer
 static int row_set_buffers(zfb_engine *e) {
     const size_t W = (size_t)e->W;
     int rc = ZFB_OK;
     if (e->traces_on) rc = ensure(e, e->trace, W * (sizeof(double) + 4 * sizeof(float)));
     if (rc) return rc;
     if (e->persist_on) rc = ensure(e, e->persist, (size_t)PS_LEVELS * W * sizeof(float));
+    if (rc) return rc;
+    const size_t nchunks = (W + MK_CHUNK - 1) / MK_CHUNK;
+    if (e->mask_on) rc = ensure(e, e->mask_work, (size_t)e->group * (nchunks * sizeof(MaskPart) + sizeof(MaskCap)));
     if (rc) return rc;
     return ensure(e, e->trace_rows, (size_t)e->group * W * sizeof(float));     // fp64 passes: px_group <= group
 }
@@ -2340,9 +2433,11 @@ static int configure_impl(zfb_engine *e, const zfb_config *cfg) {
     if (memcmp(key, e->trace_key, sizeof key) != 0) {
         e->trace_count = 0;
         e->persist_count = 0;
+        // the mask's lines no longer mean the same columns (the stream is idle: synchronised above)
+        if (e->mask_on) mask_off(e);
     }
     memcpy(e->trace_key, key, sizeof key);
-    if (e->traces_on || e->persist_on) {
+    if (row_sets_on(e)) {
         rc = row_set_buffers(e);
         if (rc) return rc;
     }
@@ -2422,7 +2517,8 @@ static int process_pipelined(zfb_engine *e, const void *d_in, int nframes, float
         }
         CK(e, cudaEventRecord(e->ev_lane[i], l->stream));
         CK(e, cudaStreamWaitEvent(e->fin_stream, e->ev_lane[i], 0));
-        rc = finish_rows(e, l, gf, nsplit, d_rows ? d_rows + (size_t)g0 * e->W : nullptr, e->fin_stream);
+        rc = finish_rows(e, l, (const char *)d_in + (size_t)g0 * fbytes, gf, nsplit,
+                         d_rows ? d_rows + (size_t)g0 * e->W : nullptr, e->fin_stream);
         if (rc != ZFB_OK) break;
         CK(e, cudaEventRecord(e->ev_fin[i], e->fin_stream));
         e->ev_fin_used[i] = true;
@@ -2647,7 +2743,7 @@ int zfb_traces_enable(zfb_engine *e, int on) {
         CK(e, cudaStreamSynchronize(e->stream));
         e->traces_on = false;
         for (DevBuf *b : {&e->trace, &e->peaks}) release(*b);
-        if (!e->persist_on) release(e->trace_rows);
+        if (!row_sets_on(e)) release(e->trace_rows);
         return ZFB_OK;
     }
     e->traces_on = true;
@@ -2861,6 +2957,8 @@ static int check_channels(zfb_engine *e, const double *f_demod, int nch) {
         return fail(e, ZFB_EINVAL, "channels: the trace set is per engine; zfb_traces_enable(e, 0) first");
     if (nch > 0 && e->persist_on)
         return fail(e, ZFB_EINVAL, "channels: the persistence set is per engine; zfb_persist_enable(e, 0, ...) first");
+    if (nch > 0 && e->mask_on)
+        return fail(e, ZFB_EINVAL, "channels: the frequency mask is per engine; zfb_mask_enable(e, 0, ...) first");
     if (nch > 0 && e->nstages == 0)
         return fail(e, ZFB_EINVAL, "channels: fft_ratio 1 has no software LO");
     return ZFB_OK;
@@ -3354,7 +3452,7 @@ int zfb_persist_enable(zfb_engine *e, int on, double minlev, double maxlev, doub
     e->persist_on = false;
     if (!on) {
         for (DevBuf *b : {&e->persist, &e->persist_thr}) release(*b);
-        if (!e->traces_on) release(e->trace_rows);
+        if (!row_sets_on(e)) release(e->trace_rows);
         return ZFB_OK;
     }
     int rc = put_thresholds(e, e->persist_thr, minlev, maxlev);
@@ -3368,7 +3466,7 @@ int zfb_persist_enable(zfb_engine *e, int on, double minlev, double maxlev, doub
     if (rc) {
         e->persist_on = false;
         for (DevBuf *b : {&e->persist, &e->persist_thr}) release(*b);
-        if (!e->traces_on) release(e->trace_rows);
+        if (!row_sets_on(e)) release(e->trace_rows);
     }
     return rc;
 }
@@ -3426,6 +3524,156 @@ int zfb_persist_image(zfb_engine *e, int kind, double imin, double imax, const u
         CK(e, cudaMemcpyAsync(out, p.out, bytes, cudaMemcpyDeviceToHost, st));
         CK(e, cudaStreamSynchronize(st));
         e->counters[4] += bytes;
+    }
+    return ZFB_OK;
+}
+
+// ---- frequency-mask trigger (zfb_mask.cuh) -----------------------------------------------------
+int zfb_mask_enable(zfb_engine *e, int on, const float *upper, const float *lower, int min_cols, int max_events,
+                    int capture_slots, int capture_samples) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    const int W = e->W;
+    if (on) {
+        if (!e->configured) return fail(e, ZFB_ESTATE, "mask: engine is not configured");
+        if (!upper && !lower) return fail(e, ZFB_EINVAL, "mask: neither an upper nor a lower line");
+        if (upper && lower)
+            for (int c = 0; c < W; ++c)
+                if (isfinite(upper[c]) && isfinite(lower[c]) && lower[c] > upper[c])
+                    return fail(e, ZFB_EINVAL, "mask: lower %g above upper %g at column %d", lower[c], upper[c], c);
+        if (min_cols < 1 || min_cols > W) return fail(e, ZFB_EINVAL, "mask: min_cols %d outside [1, %d]", min_cols, W);
+        if (max_events < 1 || max_events > (1 << 20))
+            return fail(e, ZFB_EINVAL, "mask: max_events %d outside [1, 2^20]", max_events);
+        if (capture_slots < 0 || capture_slots > max_events)
+            return fail(e, ZFB_EINVAL, "mask: capture_slots %d outside [0, max_events]", capture_slots);
+        if (capture_slots > 0 && (capture_samples < 1 || capture_samples > (1 << 28)))
+            return fail(e, ZFB_EINVAL, "mask: capture_samples %d outside [1, 2^28]", capture_samples);
+    }
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    // rows still being checked read these buffers
+    CK(e, cudaStreamSynchronize(e->stream));
+    mask_off(e);
+    if (!on) return ZFB_OK;
+    e->mask_min_cols = min_cols;
+    e->mask_max_events = max_events;
+    e->mask_slots = capture_slots;
+    e->mask_cap_samples = capture_slots > 0 ? capture_samples : 0;
+    std::vector<float> lines((size_t)2 * W, nanf(""));
+    for (int c = 0; c < W; ++c) {
+        if (upper) lines[(size_t)c] = upper[c];
+        if (lower) lines[(size_t)W + c] = lower[c];
+    }
+    e->mask_on = true;
+    int rc = ensure(e, e->mask_lines, lines.size() * sizeof(float));
+    if (rc == ZFB_OK) rc = ensure(e, e->mask_state, 16);
+    if (rc == ZFB_OK) rc = ensure(e, e->mask_log, (size_t)max_events * sizeof(zfb_mask_event));
+    if (rc == ZFB_OK && capture_slots > 0)
+        rc = ensure(e, e->mask_caps, (size_t)capture_slots * (size_t)capture_samples * 8);
+    if (rc == ZFB_OK) rc = row_set_buffers(e);
+    if (rc == ZFB_OK) {
+        cudaError_t st = cudaMemcpyAsync(e->mask_lines.p, lines.data(), lines.size() * sizeof(float),
+                                         cudaMemcpyHostToDevice, e->stream);
+        if (st == cudaSuccess) st = cudaMemsetAsync(e->mask_state.p, 0, 16, e->stream);
+        if (st == cudaSuccess) st = cudaStreamSynchronize(e->stream);      // `lines` lives on this stack frame
+        if (st != cudaSuccess) rc = fail(e, ZFB_ECUDA, "mask: upload failed: %s", cudaGetErrorString(st));
+        e->counters[3] += lines.size() * sizeof(float);
+    }
+    if (rc) mask_off(e);
+    return rc;
+}
+
+int zfb_mask_reset(zfb_engine *e) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (!e->mask_on) return fail(e, ZFB_ESTATE, "mask is off (zfb_mask_enable)");
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    // launch order is stream order: the next check starts at row 0, event 0
+    CK(e, cudaMemsetAsync(e->mask_state.p, 0, 16, e->stream));
+    e->mask_rows = 0;
+    return ZFB_OK;
+}
+
+// the device's event counter, after everything handed over so far (blocks)
+static int mask_events_detected(zfb_engine *e, int64_t *out) {
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    unsigned long long n = 0;
+    CK(e, cudaMemcpyAsync(&n, e->mask_state.p, sizeof n, cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->counters[4] += sizeof n;
+    *out = (int64_t)n;
+    return ZFB_OK;
+}
+
+int zfb_mask_counts(zfb_engine *e, int64_t out2[2]) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (!out2) return fail(e, ZFB_EINVAL, "mask counts: out is NULL");
+    if (!e->mask_on) return fail(e, ZFB_ESTATE, "mask is off (zfb_mask_enable)");
+    int64_t n = 0;
+    const int rc = mask_events_detected(e, &n);
+    if (rc) return rc;
+    out2[0] = e->mask_rows;
+    out2[1] = n;
+    return ZFB_OK;
+}
+
+int zfb_mask_events(zfb_engine *e, int first, int max, zfb_mask_event *out, int *n) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (first < 0 || max < 0 || !n || (max > 0 && !out))
+        return fail(e, ZFB_EINVAL, "mask events: bad arguments (first %d, max %d)", first, max);
+    if (!e->mask_on) return fail(e, ZFB_ESTATE, "mask is off (zfb_mask_enable)");
+    int64_t detected = 0;
+    const int rc = mask_events_detected(e, &detected);
+    if (rc) return rc;
+    const int64_t stored = std::min<int64_t>(detected, e->mask_max_events);
+    const int cnt = (int)std::max<int64_t>(0, std::min<int64_t>(stored - first, max));
+    if (cnt > 0) {
+        const size_t bytes = (size_t)cnt * sizeof(zfb_mask_event);
+        CK(e, cudaMemcpyAsync(out, (const zfb_mask_event *)e->mask_log.p + first, bytes, cudaMemcpyDeviceToHost,
+                              e->stream));
+        CK(e, cudaStreamSynchronize(e->stream));
+        e->counters[4] += bytes;
+    }
+    *n = cnt;
+    return ZFB_OK;
+}
+
+int zfb_mask_capture(zfb_engine *e, int slot, void *out, int out_on_device) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (!out) return fail(e, ZFB_EINVAL, "mask capture: out is NULL");
+    if (!e->mask_on) return fail(e, ZFB_ESTATE, "mask is off (zfb_mask_enable)");
+    if (slot < 0 || slot >= e->mask_slots)
+        return fail(e, ZFB_EINVAL, "mask capture: slot %d outside [0, %d)", slot, e->mask_slots);
+    int64_t detected = 0;
+    int rc = mask_events_detected(e, &detected);
+    if (rc) return rc;
+    if (detected <= slot) return fail(e, ZFB_ESTATE, "mask capture: slot %d is not filled yet", slot);
+    zfb_mask_event ev;       // event `slot` owns slot `slot` (capture_slots <= max_events: it is stored)
+    CK(e, cudaMemcpyAsync(&ev, (const zfb_mask_event *)e->mask_log.p + slot, sizeof ev, cudaMemcpyDeviceToHost,
+                          e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->counters[4] += sizeof ev;
+    const long long bytes = (long long)ev.capture_samples * (long long)dtype_bytes(ev.dtype);
+    const unsigned char *src = (const unsigned char *)e->mask_caps.p + (size_t)slot * (size_t)e->mask_cap_samples * 8;
+    if (out_on_device) {
+        MaskCopyParams mp{};
+        mp.src = src;
+        mp.dst = (unsigned char *)out;
+        mp.nbytes = bytes;
+        const long long tiles = (bytes + MC_TILE - 1) / MC_TILE + 1;
+        ZFB_LAUNCH(mask_capture_kernel, dim3((unsigned)std::min<long long>(tiles, 4 * (long long)e->sm_count)),
+                   dim3(MC_NT), 0, e->stream, mp);
+        CK(e, cudaGetLastError());
+        e->counters[2] += 1;
+    } else {
+        CK(e, cudaMemcpyAsync(out, src, (size_t)bytes, cudaMemcpyDeviceToHost, e->stream));
+        CK(e, cudaStreamSynchronize(e->stream));
+        e->counters[4] += (size_t)bytes;
     }
     return ZFB_OK;
 }

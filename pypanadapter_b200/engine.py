@@ -493,6 +493,85 @@ class ZoomPSD:
         self._check(self._lib.zfb_persist_image(self._h, code, lo, hi, lut_p, C.c_void_p(d_out_ptr), 1),
                     "zfb_persist_image")
 
+    # -- frequency-mask trigger (DESIGN 3.10) ----------------------------------
+    def mask_enable(self, upper=None, lower=None, *, min_cols: int = 1, max_events: int = 4096, capture: int = 0,
+                    capture_samples: int | None = None):
+        """Check every row the engine computes from now on against limit lines in the rows' units
+        (starts the log empty): a column violates above ``upper`` or below ``lower`` (each an
+        array of row_width, a scalar for every column, or None; NaN turns a side off at a
+        column), a row with at least ``min_cols`` violating columns is an event.  The first
+        ``max_events`` events are logged in frame order; the first ``capture`` of them keep the
+        first ``capture_samples`` (default: the configured frame_len) samples of their frame."""
+        W = self.row_width
+
+        def line(x):
+            return None if x is None else np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype=np.float32), (W,)))
+
+        up, lo = line(upper), line(lower)
+        ns = self.frame_len if capture_samples is None else int(capture_samples)
+        self._check(self._lib.zfb_mask_enable(self._h, 1, None if up is None else C.c_void_p(up.ctypes.data),
+                                              None if lo is None else C.c_void_p(lo.ctypes.data), int(min_cols),
+                                              int(max_events), int(capture), ns), "zfb_mask_enable")
+        self._mask_slots = int(capture)
+
+    def mask_disable(self):
+        self._check(self._lib.zfb_mask_enable(self._h, 0, None, None, 0, 0, 0, 0), "zfb_mask_enable")
+
+    def mask_reset(self):
+        """Empty the log and both counters; the lines stay (the caller's re-arm)."""
+        self._check(self._lib.zfb_mask_reset(self._h), "zfb_mask_reset")
+
+    @property
+    def mask_counts(self) -> tuple[int, int]:
+        """(rows checked, events detected) since the log last started empty"""
+        out = (C.c_int64 * 2)()
+        self._check(self._lib.zfb_mask_counts(self._h, out), "zfb_mask_counts")
+        return int(out[0]), int(out[1])
+
+    def mask_events(self, first: int = 0, max: int | None = None) -> np.ndarray:
+        """Stored events ``[first, first + max)`` as a structured array of the zfb_mask_event
+        fields plus ``freq_hz`` of ``worst_col``."""
+        if max is None:
+            max = self.mask_counts[1]
+        m = int(max)
+        buf = (_lib.ZfbMaskEvent * (m if m > 0 else 1))()
+        n = C.c_int(0)
+        self._check(self._lib.zfb_mask_events(self._h, int(first), m, C.cast(buf, C.c_void_p), C.byref(n)),
+                    "zfb_mask_events")
+        raw = np.frombuffer(buf, dtype=MASK_EVENT_DTYPE, count=n.value) if n.value else \
+            np.zeros(0, dtype=MASK_EVENT_DTYPE)
+        out = np.zeros(n.value, dtype=MASK_EVENT_RECORD)
+        for name in MASK_EVENT_DTYPE.names:
+            out[name] = raw[name]
+        out["freq_hz"] = self.row_frequencies()[raw["worst_col"]] if n.value else []
+        return out
+
+    def mask_capture(self, slot: int) -> np.ndarray:
+        """The samples of capture slot ``slot`` in wire form: complex64 ``(n,)``, or the
+        interleaved uint8 / int16 stream ``(2n,)``."""
+        ev = self._mask_slot_event(slot)
+        n, code = int(ev["capture_samples"]), int(ev["dtype"])
+        if code == _lib.ZFB_DTYPE_C64:
+            out = np.empty(n, dtype=np.complex64)
+        else:
+            out = np.empty(2 * n, dtype=np.uint8 if code == _lib.ZFB_DTYPE_U8 else np.int16)
+        self._check(self._lib.zfb_mask_capture(self._h, int(slot), C.c_void_p(out.ctypes.data), 0),
+                    "zfb_mask_capture")
+        return out
+
+    def mask_capture_device(self, slot: int, d_out_ptr: int):
+        """The same bytes into a caller-owned device buffer (asynchronous on the engine's stream)."""
+        self._check(self._lib.zfb_mask_capture(self._h, int(slot), C.c_void_p(d_out_ptr), 1), "zfb_mask_capture")
+
+    def _mask_slot_event(self, slot: int):
+        slot = int(slot)
+        ev = self.mask_events(max(slot, 0), 1)          # ESTATE while the mask is off
+        if not 0 <= slot < self._mask_slots:
+            raise ZoomFFTError(_lib.ZFB_EINVAL, "mask_capture: slot %d outside [0, %d)" % (slot, self._mask_slots))
+        if len(ev) != 1:
+            raise ZoomFFTError(_lib.ZFB_ESTATE, "mask_capture: slot %d is not filled yet" % slot)
+        return ev[0]
+
     # -- waterfall image / autolevel on the device (S:1625-1676) ---------------
     def ring_image(self, height: int, scroll: int, rows_seen: int, kind: str = "f32", *,
                    levels=None, lut=None) -> np.ndarray:
@@ -575,6 +654,12 @@ class ZoomPSD:
 
 PEAK_DTYPE = np.dtype([("column", np.int32), ("value", np.float32), ("offset", np.float64),
                        ("freq_hz", np.float64)])
+
+MASK_EVENT_DTYPE = np.dtype([("row", np.int64), ("ncols", np.int32), ("first_col", np.int32),
+                             ("last_col", np.int32), ("worst_col", np.int32), ("value", np.float32),
+                             ("excess", np.float32), ("above", np.int32), ("capture", np.int32),
+                             ("capture_samples", np.int32), ("dtype", np.int32)])
+MASK_EVENT_RECORD = np.dtype(MASK_EVENT_DTYPE.descr + [("freq_hz", np.float64)])
 
 _TRACE_KINDS = {"last": _lib.ZFB_TRACE_LAST, "max": _lib.ZFB_TRACE_MAX, "min": _lib.ZFB_TRACE_MIN,
                 "avg": _lib.ZFB_TRACE_AVG}
