@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ZFB_ABI_VERSION 5
+#define ZFB_ABI_VERSION 6
 
 /* status codes */
 #define ZFB_OK            0
@@ -441,6 +441,56 @@ int  zfb_mask_events(zfb_engine *e, int first, int max, zfb_mask_event *out, int
  * for a slot not filled yet. */
 int  zfb_mask_capture(zfb_engine *e, int slot, void *out, int out_on_device);
 
+/* ---- channel power and occupied bandwidth (DESIGN 3.11) ---------------------
+ * A spectrum analyser's measurement menu -- channel power, adjacent-channel
+ * leakage, occupied bandwidth and how each moved over time -- measured on the
+ * device over the same rows as the trace set (every row of zfb_process_device,
+ * zfb_process_host and zfb_samples_process on every path, EMA applied, also
+ * rows that never reach the ring; not rows of zfb_ring_push_rows), for nbands
+ * column ranges [first_col, end_col) of the row.  Per row and band:
+ *   power  = (fs / fft_size) * sum over the band of p[c], in fp64, where p[c] is
+ *            the row value with ZFB_FLAG_LINEAR, else 10^(v/20); a -inf value
+ *            (a DC-only frame) adds 0.  The rows are a density over the
+ *            undecimated fs, so this is the band's power, not sum * spacing.
+ *   obw_lo, obw_hi = the occupied-bandwidth edges for the fraction q, as
+ *            fractional row columns (column c's bin spans [c, c + 1)): with
+ *            C(j) = sum of p[c] for first_col <= c < j and T = C(end_col), the
+ *            edge for a target t is j + (t - C(j)) / p[j], j the first column
+ *            with C(j + 1) >= t; t = (1 - q)/2 * T for obw_lo, (1 + q)/2 * T for
+ *            obw_hi.  The power and both targets come from the same total T.
+ *            Both edges are NaN when the band's power is 0.
+ *   Log: a device ring of the newest log_rows rows; row k (counted from when
+ *   the set started empty) lives at slot k mod log_rows.
+ *   Summary: per band the max, min and fp64 sum of power over every row since
+ *   the set started empty, accumulated in frame order (a NaN power, from a NaN
+ *   row value, makes max, min and mean NaN, as numpy's do).
+ * The order of every sum depends only on a band's width: the log, the summary
+ * and the count are bit-identical however the same frames are cut into calls,
+ * groups, host or device paths or pipelined batches.  Off by default: then
+ * nothing is allocated or launched; on, a launch group costs 1 more kernel.
+ * zfb_power_enable(on = 1) needs a configured engine (ZFB_ESTATE otherwise);
+ * it validates, uploads the bands and starts the set empty.  ZFB_EINVAL for
+ * bands == NULL or bands, obw_fraction or log_rows out of range; ZFB_ENOMEM
+ * leaves the set off.  on = 0 turns it off and frees it.  A zfb_configure that
+ * changes fs, fft_size, fft_ratio, row_width, f_demod or flags turns the set off
+ * (its columns no longer mean the same frequencies); a change of frame_len,
+ * window, ema_alpha, dtype, flip or mode keeps it counting.  While it is on,
+ * zfb_process_channels_* return ZFB_EINVAL.  Every read returns ZFB_ESTATE
+ * while the set is off. */
+/* bands: nbands pairs [first_col, end_col), 0 <= first < end <= row_width; 1 <= nbands <= 64;
+ * 0 < obw_fraction < 1; log_rows >= 1 and log_rows * nbands <= 2^26 */
+int  zfb_power_enable(zfb_engine *e, int on, const int32_t *bands, int nbands,
+                      double obw_fraction, int64_t log_rows);
+int  zfb_power_reset(zfb_engine *e);              /* empty log, summary and count; keep the bands */
+int64_t zfb_power_count(const zfb_engine *e);     /* rows measured since the set started empty; 0 while off */
+/* rows [first_row, first_row + nrows) to [nrows][nbands] arrays (any may be NULL); joins, blocks.
+ * ZFB_EINVAL when a row is not in the log any more (< count - log_rows) or not yet measured (>= count). */
+int  zfb_power_read(zfb_engine *e, int64_t first_row, int nrows,
+                    double *power, double *obw_lo, double *obw_hi);
+/* out[nbands][3] = max, min, mean power over every row since the set started empty (NaN while
+ * no row has been measured); joins, blocks.  ZFB_EINVAL for out == NULL. */
+int  zfb_power_summary(zfb_engine *e, double *out);
+
 /* ---- taper design and preview on the device (SURVEY 8f.4) ----------------
  * The taper dialog's live preview (FFTTaperingControl.ShowCurve, S:1354-1379):
  * zfb_taper_design replaces scipy.signal.get_window(AppState.fft_tapering, 51)
@@ -500,7 +550,7 @@ int  zfb_get_counters(const zfb_engine *e, uint64_t out5[5]);
  * decimate call s of the loop at S:2097-2098), 16 = Welch kernel / four-step
  * column pass, 17 = four-step row pass (both: scipy.signal.welch, S:2111),
  * 18 = row finalisation (S:2114-2119 + EMA, trace and persistence updates,
- * frequency-mask check, log and capture),
+ * frequency-mask check, log and capture, channel power and OBW),
  * 19 = waterfall image (S:1625-1664) and persistence image, 20 = autolevel
  * selection sweep (S:1676). */
 #define ZFB_PROF_CLASSES 21

@@ -32,7 +32,7 @@ ZFB_FLAG_NO_LO = 1
 ZFB_FLAG_LINEAR = 2
 ZFB_FLAG_ONESIDED = 4
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 PROF_CLASSES = 21
 ZFB_IMAGE_F32 = 0
 ZFB_IMAGE_U8 = 1
@@ -140,6 +140,11 @@ SYMBOLS = {
     "zfb_mask_counts": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "zfb_mask_events": (C.c_int, [_P, C.c_int, C.c_int, _P, C.POINTER(C.c_int)]),
     "zfb_mask_capture": (C.c_int, [_P, C.c_int, _P, C.c_int]),
+    "zfb_power_enable": (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_double, C.c_int64]),
+    "zfb_power_reset": (C.c_int, [_P]),
+    "zfb_power_count": (C.c_int64, [_P]),
+    "zfb_power_read": (C.c_int, [_P, C.c_int64, C.c_int, _P, _P, _P]),
+    "zfb_power_summary": (C.c_int, [_P, _P]),
     "zfb_ring_quantiles": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, C.POINTER(C.c_double), C.c_int,
                                      C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "zfb_taper_design": (C.c_int, [_P, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(C.c_double)]),

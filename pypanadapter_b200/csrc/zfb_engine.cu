@@ -32,6 +32,7 @@
 #include "zfb_trace.cuh"
 #include "zfb_persist.cuh"
 #include "zfb_mask.cuh"
+#include "zfb_power.cuh"
 
 using namespace zfb;
 
@@ -175,6 +176,18 @@ struct zfb_engine {
     DevBuf mask_log;                   // [max_events] zfb_mask_event
     DevBuf mask_caps;                  // [capture_slots][capture_samples * 8] bytes
     DevBuf mask_work;                  // [group][chunks] MaskPart, then [group] MaskCap
+    // channel power and occupied bandwidth (zfb_power_enable; zfb_power.cuh): nothing is allocated or
+    // launched while it is off
+    bool power_on = false;
+    int64_t power_rows = 0;            // rows measured (host side; launch order = stream order)
+    int power_nbands = 0;
+    int power_nnarrow = 0, power_nwide = 0;    // bands of <= PW_NARROW columns (one warp each), the others
+    int64_t power_log_rows = 0;
+    double power_q = 0.99;
+    DevBuf power_bands;                // [nbands][2] int: first, end column; the narrow, then the wide band indices
+    DevBuf power_state;                // [nbands][3] double: max, min, sum; then the CTA completion counter
+    DevBuf power_log;                  // [log_rows][nbands][3] double: power, obw_lo, obw_hi
+    DevBuf power_work;                 // [group][nbands][3] double: the group's measurements
 
     // ZFB_MODE_FAST
     struct FastPlan {
@@ -1245,10 +1258,10 @@ cudaError_t run_decimation_fast(zfb_engine *e, const void *d_in, int gf, int *ou
     return cudaSuccess;
 }
 
-// a set that reads every row (traces, persistence, frequency mask) is on
-bool row_sets_on(const zfb_engine *e) { return e->traces_on || e->persist_on || e->mask_on; }
+// a set that reads every row (traces, persistence, frequency mask, power set) is on
+bool row_sets_on(const zfb_engine *e) { return e->traces_on || e->persist_on || e->mask_on || e->power_on; }
 
-// traces, persistence or mask on: the rows of a launch group go to the caller's buffer or, without
+// a row set on: the rows of a launch group go to the caller's buffer or, without
 // one, to this scratch
 float *trace_rows_or(zfb_engine *e, float *d_rows) {
     return (d_rows || !row_sets_on(e) || e->cur_nch > 0) ? d_rows : (float *)e->trace_rows.p;
@@ -1360,12 +1373,49 @@ int mask_update(zfb_engine *e, const float *rows, const void *in, size_t fbytes,
     return ZFB_OK;
 }
 
+// measure the bands of the power set on `nf` finished rows, log them and fold them into the
+// summary, on the stream that finished them (after them)
+int power_update(zfb_engine *e, const float *rows, int nf, cudaStream_t st) {
+    if (!e->power_on || e->cur_nch > 0 || nf < 1) return ZFB_OK;
+    const int nb = e->power_nbands;
+    PowerParams pp{};
+    pp.rows = rows;
+    pp.bands = (const int *)e->power_bands.p;
+    pp.narrow = pp.bands + 2 * nb;
+    pp.wide = pp.narrow + e->power_nnarrow;
+    pp.nnarrow = e->power_nnarrow;
+    pp.nwide = e->power_nwide;
+    pp.nframes = nf;
+    pp.W = e->W;
+    pp.nbands = nb;
+    pp.linear = (e->cfg.flags & ZFB_FLAG_LINEAR) ? 1 : 0;
+    pp.delta = e->cfg.fs / (double)e->cfg.fft_size;
+    pp.q_lo = (1.0 - e->power_q) / 2.0;
+    pp.q_hi = (1.0 + e->power_q) / 2.0;
+    pp.meas = (double *)e->power_work.p;
+    pp.log = (double *)e->power_log.p;
+    pp.log_rows = (int)e->power_log_rows;
+    pp.slot0 = (int)(e->power_rows % e->power_log_rows);
+    pp.summary = (double *)e->power_state.p;
+    pp.have = e->power_rows > 0 ? 1 : 0;
+    pp.done = (unsigned *)(pp.summary + 3 * (size_t)nb);
+    const int pr = prof_begin(e, 18, st);
+    const int ctas = nf * e->power_nwide + (nf * e->power_nnarrow + PW_NW - 1) / PW_NW;
+    ZFB_LAUNCH(power_measure_kernel, dim3((unsigned)ctas), dim3(PW_NT), 0, st, pp);
+    prof_end(e, pr, st);
+    e->counters[2] += 1;
+    e->power_rows += nf;
+    CK(e, cudaGetLastError());
+    return ZFB_OK;
+}
+
 // every row the engine finishes (not the rows of channel-batched launches) feeds the trace and
-// persistence sets and the frequency mask that are on; `in` is the group's input
+// persistence sets, the frequency mask and the power set that are on; `in` is the group's input
 int rows_finished(zfb_engine *e, const float *rows, const void *in, int nf, cudaStream_t st) {
     int rc = trace_update(e, rows, nf, st);
     if (rc == ZFB_OK) rc = persist_update(e, rows, nf, st);
     if (rc == ZFB_OK) rc = mask_update(e, rows, in, (size_t)e->cfg.frame_len * sample_bytes(e->cfg), nf, st);
+    if (rc == ZFB_OK) rc = power_update(e, rows, nf, st);
     return rc;
 }
 
@@ -2083,7 +2133,8 @@ void zfb_destroy(zfb_engine *e) {
     DevBuf *bufs[] = {&e->window, &e->winfft, &e->winfft16, &e->wf_sparse, &e->twiddle, &e->twiddle_sub, &e->pow16, &e->mid[0], &e->mid[1], &e->pow, &e->rows_tmp, &e->ema,
                       &e->img_out, &e->img_lut, &e->img_thr, &e->sel_hist, &e->ring, &e->stage_in[0], &e->stage_in[1], &e->big,
                       &e->trace, &e->trace_rows, &e->peaks, &e->persist, &e->persist_thr,
-                      &e->mask_lines, &e->mask_state, &e->mask_log, &e->mask_caps, &e->mask_work};
+                      &e->mask_lines, &e->mask_state, &e->mask_log, &e->mask_caps, &e->mask_work,
+                      &e->power_bands, &e->power_state, &e->power_log, &e->power_work};
     for (DevBuf *b : bufs) release(*b);
     for (int i = 0; i < 2; ++i) {
         if (e->h_stage[i]) cudaFreeHost(e->h_stage[i]);
@@ -2145,8 +2196,16 @@ static void mask_off(zfb_engine *e) {
     if (!row_sets_on(e)) release(e->trace_rows);
 }
 
-// state of the trace and persistence sets that are on, the frequency mask's per-group scratch, and
-// the scratch for rows of launch groups without a caller's row buffer
+// the power set off and freed (no work that reads its buffers may be pending)
+static void power_off(zfb_engine *e) {
+    e->power_on = false;
+    e->power_rows = 0;
+    for (DevBuf *b : {&e->power_bands, &e->power_state, &e->power_log, &e->power_work}) release(*b);
+    if (!row_sets_on(e)) release(e->trace_rows);
+}
+
+// state of the trace and persistence sets that are on, the per-group scratch of the frequency mask
+// and the power set, and the scratch for rows of launch groups without a caller's row buffer
 static int row_set_buffers(zfb_engine *e) {
     const size_t W = (size_t)e->W;
     int rc = ZFB_OK;
@@ -2156,6 +2215,8 @@ static int row_set_buffers(zfb_engine *e) {
     if (rc) return rc;
     const size_t nchunks = (W + MK_CHUNK - 1) / MK_CHUNK;
     if (e->mask_on) rc = ensure(e, e->mask_work, (size_t)e->group * (nchunks * sizeof(MaskPart) + sizeof(MaskCap)));
+    if (rc) return rc;
+    if (e->power_on) rc = ensure(e, e->power_work, (size_t)e->group * (size_t)e->power_nbands * 3 * sizeof(double));
     if (rc) return rc;
     return ensure(e, e->trace_rows, (size_t)e->group * W * sizeof(float));     // fp64 passes: px_group <= group
 }
@@ -2433,8 +2494,10 @@ static int configure_impl(zfb_engine *e, const zfb_config *cfg) {
     if (memcmp(key, e->trace_key, sizeof key) != 0) {
         e->trace_count = 0;
         e->persist_count = 0;
-        // the mask's lines no longer mean the same columns (the stream is idle: synchronised above)
+        // the mask's lines and the power set's bands no longer mean the same columns (the stream is
+        // idle: synchronised above)
         if (e->mask_on) mask_off(e);
+        if (e->power_on) power_off(e);
     }
     memcpy(e->trace_key, key, sizeof key);
     if (row_sets_on(e)) {
@@ -2959,6 +3022,8 @@ static int check_channels(zfb_engine *e, const double *f_demod, int nch) {
         return fail(e, ZFB_EINVAL, "channels: the persistence set is per engine; zfb_persist_enable(e, 0, ...) first");
     if (nch > 0 && e->mask_on)
         return fail(e, ZFB_EINVAL, "channels: the frequency mask is per engine; zfb_mask_enable(e, 0, ...) first");
+    if (nch > 0 && e->power_on)
+        return fail(e, ZFB_EINVAL, "channels: the power set is per engine; zfb_power_enable(e, 0, ...) first");
     if (nch > 0 && e->nstages == 0)
         return fail(e, ZFB_EINVAL, "channels: fft_ratio 1 has no software LO");
     return ZFB_OK;
@@ -3675,6 +3740,124 @@ int zfb_mask_capture(zfb_engine *e, int slot, void *out, int out_on_device) {
         CK(e, cudaStreamSynchronize(e->stream));
         e->counters[4] += (size_t)bytes;
     }
+    return ZFB_OK;
+}
+
+// ---- channel power and occupied bandwidth (zfb_power.cuh) -------------------------------------
+int zfb_power_enable(zfb_engine *e, int on, const int32_t *bands, int nbands, double obw_fraction, int64_t log_rows) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (on) {
+        if (!e->configured) return fail(e, ZFB_ESTATE, "power: engine is not configured");
+        if (!bands || nbands < 1 || nbands > PW_MAX_BANDS)
+            return fail(e, ZFB_EINVAL, "power: %d bands outside [1, %d] (or bands is NULL)", nbands, PW_MAX_BANDS);
+        for (int b = 0; b < nbands; ++b)
+            if (bands[2 * b] < 0 || bands[2 * b] >= bands[2 * b + 1] || bands[2 * b + 1] > e->W)
+                return fail(e, ZFB_EINVAL, "power: band %d [%d, %d) is not a column range of a %d-wide row", b,
+                            bands[2 * b], bands[2 * b + 1], e->W);
+        if (!(obw_fraction > 0.0 && obw_fraction < 1.0))
+            return fail(e, ZFB_EINVAL, "power: obw_fraction %g outside (0, 1)", obw_fraction);
+        if (log_rows < 1 || log_rows > (1 << 26) || log_rows * nbands > (1 << 26))
+            return fail(e, ZFB_EINVAL, "power: log_rows %lld x %d bands outside [1, 2^26]", (long long)log_rows,
+                        nbands);
+    }
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    // rows still being measured read these buffers
+    CK(e, cudaStreamSynchronize(e->stream));
+    power_off(e);
+    if (!on) return ZFB_OK;
+    // the bands, then the indices of the narrow bands (one warp per row) and of the wide ones
+    std::vector<int32_t> table(bands, bands + 2 * (size_t)nbands);
+    for (int pass = 0; pass < 2; ++pass)
+        for (int b = 0; b < nbands; ++b)
+            if ((bands[2 * b + 1] - bands[2 * b] <= PW_NARROW) == (pass == 0)) table.push_back(b);
+    e->power_nbands = nbands;
+    e->power_nnarrow = 0;
+    for (int b = 0; b < nbands; ++b) e->power_nnarrow += bands[2 * b + 1] - bands[2 * b] <= PW_NARROW ? 1 : 0;
+    e->power_nwide = nbands - e->power_nnarrow;
+    e->power_log_rows = log_rows;
+    e->power_q = obw_fraction;
+    e->power_on = true;
+    const size_t state_bytes = (size_t)nbands * 3 * sizeof(double) + sizeof(unsigned);
+    int rc = ensure(e, e->power_bands, table.size() * sizeof(int32_t));
+    if (rc == ZFB_OK) rc = ensure(e, e->power_state, state_bytes);
+    if (rc == ZFB_OK) rc = ensure(e, e->power_log, (size_t)log_rows * (size_t)nbands * 3 * sizeof(double));
+    if (rc == ZFB_OK) rc = row_set_buffers(e);
+    if (rc == ZFB_OK) {
+        cudaError_t st = cudaMemcpyAsync(e->power_bands.p, table.data(), table.size() * sizeof(int32_t),
+                                         cudaMemcpyHostToDevice, e->stream);
+        if (st == cudaSuccess) st = cudaMemsetAsync(e->power_state.p, 0, state_bytes, e->stream);
+        if (st == cudaSuccess) st = cudaStreamSynchronize(e->stream);      // `table` lives on this stack frame
+        if (st != cudaSuccess) rc = fail(e, ZFB_ECUDA, "power: upload failed: %s", cudaGetErrorString(st));
+        e->counters[3] += table.size() * sizeof(int32_t);
+    }
+    if (rc) power_off(e);
+    return rc;
+}
+
+int zfb_power_reset(zfb_engine *e) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (!e->power_on) return fail(e, ZFB_ESTATE, "power set is off (zfb_power_enable)");
+    e->power_rows = 0;       // launch order is stream order: the next group starts the log and summary afresh
+    return ZFB_OK;
+}
+
+int64_t zfb_power_count(const zfb_engine *e) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    return e->power_on ? e->power_rows : 0;
+}
+
+int zfb_power_read(zfb_engine *e, int64_t first_row, int nrows, double *power, double *obw_lo, double *obw_hi) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (!e->power_on) return fail(e, ZFB_ESTATE, "power set is off (zfb_power_enable)");
+    const int64_t count = e->power_rows, L = e->power_log_rows;
+    if (first_row < 0 || nrows < 0 || (nrows > 0 && (first_row < count - L || first_row + nrows > count)))
+        return fail(e, ZFB_EINVAL, "power read: rows [%lld, %lld) are not all in the log, which holds rows [%lld, %lld)",
+                    (long long)first_row, (long long)(first_row + nrows), (long long)std::max<int64_t>(0, count - L),
+                    (long long)count);
+    if (nrows == 0) return ZFB_OK;
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    const size_t rec = (size_t)e->power_nbands * 3;           // doubles per row
+    std::vector<double> buf((size_t)nrows * rec);
+    const int64_t s0 = first_row % L;
+    const int64_t n1 = std::min<int64_t>(nrows, L - s0);       // up to the end of the ring, then from its start
+    const double *log = (const double *)e->power_log.p;
+    CK(e, cudaMemcpyAsync(buf.data(), log + (size_t)s0 * rec, (size_t)n1 * rec * sizeof(double),
+                          cudaMemcpyDeviceToHost, e->stream));
+    if (n1 < nrows)
+        CK(e, cudaMemcpyAsync(buf.data() + (size_t)n1 * rec, log, (size_t)(nrows - n1) * rec * sizeof(double),
+                              cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->counters[4] += buf.size() * sizeof(double);
+    double *outs[3] = {power, obw_lo, obw_hi};
+    const size_t nv = (size_t)nrows * e->power_nbands;
+    for (int k = 0; k < 3; ++k)
+        if (outs[k])
+            for (size_t i = 0; i < nv; ++i) outs[k][i] = buf[3 * i + k];
+    return ZFB_OK;
+}
+
+int zfb_power_summary(zfb_engine *e, double *out) {
+    if (!e) return ZFB_EINVAL;
+    std::lock_guard<std::mutex> lk(e->mu);
+    if (!out) return fail(e, ZFB_EINVAL, "power summary: out is NULL");
+    if (!e->power_on) return fail(e, ZFB_ESTATE, "power set is off (zfb_power_enable)");
+    const int nb = e->power_nbands;
+    if (e->power_rows == 0) {
+        for (int i = 0; i < 3 * nb; ++i) out[i] = nan("");
+        return ZFB_OK;
+    }
+    join_pending_work(e);
+    CK(e, cudaSetDevice(e->device));
+    CK(e, cudaMemcpyAsync(out, e->power_state.p, (size_t)nb * 3 * sizeof(double), cudaMemcpyDeviceToHost, e->stream));
+    CK(e, cudaStreamSynchronize(e->stream));
+    e->counters[4] += (size_t)nb * 3 * sizeof(double);
+    for (int b = 0; b < nb; ++b) out[3 * b + 2] /= (double)e->power_rows;     // sum -> mean
     return ZFB_OK;
 }
 

@@ -21,6 +21,15 @@ static inline float __fadd_rn(float a, float b) {
     volatile float s = a + b;
     return s;
 }
+static inline double __dadd_rn(double a, double b) {
+    volatile double s = a + b;
+    return s;
+}
+// zfb_power.cuh's last-CTA hand-off: CTAs run on several OS threads, so the fence is a real one;
+// an L2-only load is a plain load here
+static inline void __threadfence() { std::atomic_thread_fence(std::memory_order_seq_cst); }
+template <typename T>
+static inline T __ldcg(const T *p) { return *p; }
 #else
 #include <cuda_runtime.h>
 #define ZFB_LAUNCH(kernel, grid, block, smem, stream, ...) \

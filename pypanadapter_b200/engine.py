@@ -572,6 +572,102 @@ class ZoomPSD:
             raise ZoomFFTError(_lib.ZFB_ESTATE, "mask_capture: slot %d is not filled yet" % slot)
         return ev[0]
 
+    # -- channel power and occupied bandwidth (DESIGN 3.11) -----------------------
+    def power_enable(self, bands, *, obw: float = 0.99, log_rows: int = 4096, units: str = "hz"):
+        """Measure every row the engine computes from now on (starts the set empty): per band the
+        power (fs/N times the sum of the band's linear density, fp64) and the edges of the band's
+        ``obw`` occupied bandwidth; the newest ``log_rows`` rows are logged.  ``bands``: a list of
+        ``(f_lo, f_hi)`` in Hz, a band being the columns whose ``row_frequencies()`` lie in
+        ``[f_lo, f_hi]``; with ``units="cols"``, ``[first, end)`` column pairs."""
+        if units == "hz":
+            f = self.row_frequencies()
+            cols = []
+            for lo, hi in bands:
+                idx = np.flatnonzero((f >= float(lo)) & (f <= float(hi)))
+                if idx.size == 0:
+                    raise ValueError("band (%g, %g) Hz holds no column of the row" % (lo, hi))
+                if idx[-1] - idx[0] + 1 != idx.size:
+                    raise ValueError("band (%g, %g) Hz is not one run of columns (the row wraps in frequency)"
+                                     % (lo, hi))
+                cols.append((idx[0], idx[-1] + 1))
+        elif units == "cols":
+            cols = [(int(a), int(b)) for a, b in bands]
+        else:
+            raise ValueError("units must be 'hz' or 'cols', got %r" % (units,))
+        arr = np.ascontiguousarray(np.array(cols, dtype=np.int32).reshape(-1, 2))
+        self._check(self._lib.zfb_power_enable(self._h, 1, C.c_void_p(arr.ctypes.data), len(arr), float(obw),
+                                               int(log_rows)), "zfb_power_enable")
+        self._power = (arr.copy(), int(log_rows))
+
+    def power_disable(self):
+        self._check(self._lib.zfb_power_enable(self._h, 0, None, 0, 0.0, 0), "zfb_power_enable")
+        self._power = None
+
+    def power_reset(self):
+        """Empty the log, the summary and the count; the bands stay."""
+        self._check(self._lib.zfb_power_reset(self._h), "zfb_power_reset")
+
+    @property
+    def power_count(self) -> int:
+        """rows measured since the power set last started empty (0 while it is off)"""
+        return int(self._lib.zfb_power_count(self._h))
+
+    def _power_bands(self) -> np.ndarray:
+        # the bands of the last successful power_enable (the C side answers ESTATE when a
+        # configure has turned the set off since)
+        if getattr(self, "_power", None) is None:
+            raise ZoomFFTError(_lib.ZFB_ESTATE, "the power set is off (power_enable)")
+        return self._power[0]
+
+    def power_log(self, first: int | None = None, n: int | None = None) -> np.ndarray:
+        """Logged rows ``[first, first + n)`` (default: every row the log still holds) as a
+        structured array: ``row``, and per band (fields of shape (nbands,)) ``power`` (linear,
+        float64), ``level`` (in the rows' units: 20 log10(power), or power for linear rows), the
+        OBW edges ``obw_lo`` / ``obw_hi`` in fractional row columns and ``obw_lo_hz``,
+        ``obw_hi_hz``, ``obw_hz`` (their distance)."""
+        count = self.power_count
+        bands = self._power_bands()
+        if first is None:
+            first = max(0, count - self._power[1])
+        if n is None:
+            n = max(0, count - int(first))
+        nb, n = len(bands), int(n)
+        raw = np.empty((3, max(n, 1), nb), dtype=np.float64)
+        self._check(self._lib.zfb_power_read(self._h, int(first), n, *(C.c_void_p(raw[k].ctypes.data) for k in range(3))),
+                    "zfb_power_read")
+        raw = raw[:, :n]
+        out = np.zeros(n, dtype=power_log_dtype(nb))
+        out["row"] = int(first) + np.arange(n)
+        out["power"], out["obw_lo"], out["obw_hi"] = raw
+        with np.errstate(divide="ignore"):
+            out["level"] = raw[0] if self._key[11] else 20.0 * np.log10(raw[0])
+        out["obw_lo_hz"] = self._column_hz(raw[1], bands)
+        out["obw_hi_hz"] = self._column_hz(raw[2], bands)
+        out["obw_hz"] = out["obw_hi_hz"] - out["obw_lo_hz"]
+        return out
+
+    def _column_hz(self, x, bands) -> np.ndarray:
+        """Fractional row columns ``x`` (shape (..., nbands)) of each band in Hz: f(k) + (x - k -
+        0.5) spacing with k = floor(x) kept inside the band, f = row_frequencies() and the
+        spacing fs/(R N), or fs/N for one-sided rows."""
+        fs, N, R, _W, onesided, _f = self._axis
+        spacing = fs / N if onesided else fs / (R * N)
+        x = np.asarray(x, dtype=np.float64)
+        bands = np.asarray(bands)
+        with np.errstate(invalid="ignore"):
+            k = np.clip(np.floor(np.nan_to_num(x)), bands[:, 0], bands[:, 1] - 1).astype(np.int64)
+        return self.row_frequencies()[k] + (x - k - 0.5) * spacing
+
+    def power_summary(self) -> np.ndarray:
+        """Per band ``max``, ``min`` and ``mean`` power (linear) over every row since the set
+        started empty (NaN before the first row)."""
+        nb = len(self._power_bands())
+        out = np.empty((nb, 3), dtype=np.float64)
+        self._check(self._lib.zfb_power_summary(self._h, C.c_void_p(out.ctypes.data)), "zfb_power_summary")
+        rec = np.zeros(nb, dtype=POWER_SUMMARY_DTYPE)
+        rec["max"], rec["min"], rec["mean"] = out.T
+        return rec
+
     # -- waterfall image / autolevel on the device (S:1625-1676) ---------------
     def ring_image(self, height: int, scroll: int, rows_seen: int, kind: str = "f32", *,
                    levels=None, lut=None) -> np.ndarray:
@@ -660,6 +756,14 @@ MASK_EVENT_DTYPE = np.dtype([("row", np.int64), ("ncols", np.int32), ("first_col
                              ("excess", np.float32), ("above", np.int32), ("capture", np.int32),
                              ("capture_samples", np.int32), ("dtype", np.int32)])
 MASK_EVENT_RECORD = np.dtype(MASK_EVENT_DTYPE.descr + [("freq_hz", np.float64)])
+
+POWER_SUMMARY_DTYPE = np.dtype([("max", np.float64), ("min", np.float64), ("mean", np.float64)])
+
+
+def power_log_dtype(nbands: int) -> np.dtype:
+    """The records of ZoomPSD.power_log: the row, then one float64 per band of each quantity"""
+    per_band = ("power", "level", "obw_lo", "obw_hi", "obw_lo_hz", "obw_hi_hz", "obw_hz")
+    return np.dtype([("row", np.int64)] + [(k, np.float64, (int(nbands),)) for k in per_band])
 
 _TRACE_KINDS = {"last": _lib.ZFB_TRACE_LAST, "max": _lib.ZFB_TRACE_MAX, "min": _lib.ZFB_TRACE_MIN,
                 "avg": _lib.ZFB_TRACE_AVG}
